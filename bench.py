@@ -5,7 +5,7 @@ Workload (BASELINE.json configs[1]): Face-DeId Camera forward + backward into th
 batch 64 of synthetic 256x256 RGB images per GPU, loss = sum(sensor*w) + loss_rad + centering_loss.
 A "step" is one such forward+backward over one batch.  Prints ONE JSON line (rank 0).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--size N] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--size N] [--impl reference] [--dump-outputs DIR]
 
 * value      : images/s over all ranks, inputs resident in HBM, CUDA-graph replay of the step,
                CUDA events, barrier + synchronize on both sides, max over ranks.
@@ -17,6 +17,9 @@ A "step" is one such forward+backward over one batch.  Prints ONE JSON line (ran
                sample of the same workload - reported, not the target.
 * --impl reference : times only that CPU implementation (the reference itself is PyTorch code that is
                not present on the GPU box; the oracle is its bit-exact restatement).
+* --dump-outputs DIR : after the timed steps, writes what the last timed step returned to its caller (sensor
+               images, PSF, regularisers, gradient) as DIR/<name>.npy, so that two builds can be compared output
+               for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -42,7 +45,7 @@ FALLBACK_HBM_GBS = 6650.0   # /opt/skills/guides/B200_PROFILING.md fallback
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2000)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 2000; --impl reference: 20)")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--batch", type=int, default=64, help="images per GPU")
     ap.add_argument("--size", type=int, default=256, help="image side N")
@@ -51,6 +54,8 @@ def parse():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of the cpu_baseline leg")
     ap.add_argument("--quick", action="store_true", help="timed loop only (for ncu): no breakdown / e2e / cpu legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB in all)")
     ap.add_argument("--config", default="2", choices=["1", "2", "3cam", "4cam", "5"],
                     help="BASELINE.json config: 1 = forward only, batch 8 (CPU-reference shape); 2 = fwd+bwd batch 64 (headline, "
                          "default); 3cam = the Image_Caption camera of config 3 (896/256/T=350, batch 128) without the caption "
@@ -58,6 +63,12 @@ def parse():
                          "FAN heat-map regressor is the reference's own model and is not on the GPU box: \"downstream\": \"absent\"); "
                          "5 = hi-res sweep (use --size 512|1024; the batch defaults to what fits the bench comfortably)")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 20 if args.impl == "reference" else 2000      # a CPU step of the oracle port takes ~70 ms
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA implementation, not to --impl reference")
     if args.config == "1":
         args.batch = 8 if args.batch == 64 else args.batch
     if args.config == "5":
@@ -71,6 +82,32 @@ def parse():
         world = int(os.environ.get("WORLD_SIZE", str(max(1, args.gpus))))
         args.batch = max(1, 512 // max(1, world))
     return args
+
+
+DUMP_BYTES = 64_000_000         # --dump-outputs: bytes written in all, at most
+
+
+def dump_outputs(out_dir: str, outs: dict) -> None:
+    """Write each output as <out_dir>/<name>.npy (float32).  When together they exceed DUMP_BYTES, the largest is cut to
+    a fixed seeded sample of its leading (batch) dimension and the kept indices go to <name>_index.npy (float64): runs
+    with the same arguments write the same sample."""
+    import numpy as np
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in outs.items()}
+    budget = DUMP_BYTES - 1024 * (len(arrays) + 1)             # room for the .npy headers
+    total = sum(a.nbytes for a in arrays.values())
+    if total > budget:
+        big = max(arrays, key=lambda k: arrays[k].nbytes)
+        a = arrays[big]
+        keep_n = (budget - (total - a.nbytes)) // (a[0].nbytes + 8)
+        if keep_n < 1:
+            raise RuntimeError(f"--dump-outputs: one row of {big} {tuple(a.shape)} does not fit in {DUMP_BYTES} bytes")
+        keep = np.sort(np.random.default_rng(0).choice(a.shape[0], size=keep_n, replace=False))
+        arrays[big] = np.ascontiguousarray(a[keep])
+        arrays[big + "_index"] = keep.astype(np.float64)
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out / f"{name}.npy", a)
 
 
 # --------------------------------------------------------------------------------------------
@@ -113,8 +150,6 @@ def cpu_port_rate(N: int, B: int, budget_s: float, steps: int | None = None, war
         step()
         sync()
         times.append(time.perf_counter() - t0)
-        if steps is not None and time.perf_counter() > t_end + 120:
-            break
     times.sort()
     med = times[len(times) // 2]
     return B / med, med, len(times), torch.get_num_threads()
@@ -188,7 +223,7 @@ def run_reference(args) -> None:
     if rank != 0:
         return
     N, B = args.size, args.batch
-    steps = min(args.steps, 20)
+    steps = args.steps
     warm = max(1, min(args.warmup, 10))            # the warm-up the caller asked for (a CPU step is ~70 ms: cheap)
     rate, med, n, cores = cpu_port_rate(N, B, budget_s=120.0, steps=steps, warmup=warm, forward_only=args.config == "1")
     line = {
@@ -307,19 +342,23 @@ def run_b200(args) -> None:
 
     one = torch.ones((), device=dev)
     fwd_only = args.config == "1"
-    last_y = [None]
 
-    def step(i: int):
+    def step(i: int) -> dict:
         """forward + backward into h; upstream gradients: w for the sensor image, 1 for the two regularisers
         (i.e. L = sum(sensor*w) + loss_rad + centering_loss without materialising the product).
-        Config 1: the forward alone (no autograd graph)."""
+        Config 1: the forward alone (no autograd graph).  Returns what the caller receives (detached)."""
         if fwd_only:
             with torch.no_grad():
-                last_y[0] = cam(imgs[i % R])
-            return
-        h.grad = None
-        y = cam(imgs[i % R])
-        torch.autograd.backward([y, cam.loss_rad, cam.centering_loss], [ws[i % R], one, one])
+                y = cam(imgs[i % R])
+        else:
+            h.grad = None
+            y = cam(imgs[i % R])
+            torch.autograd.backward([y, cam.loss_rad, cam.centering_loss], [ws[i % R], one, one])
+        outs = {"sensor": y.detach(), "psf": cam.psfs.detach(), "loss_rad": cam.loss_rad.detach(),
+                "centering_loss": cam.centering_loss.detach()}
+        if not fwd_only:
+            outs["grad_h"] = h.grad
+        return outs
 
     def drop_graph_refs():
         # the module keeps psfs / loss tensors (like the reference); they pin the previous autograd graph and
@@ -347,12 +386,12 @@ def run_b200(args) -> None:
                     step(r)
             torch.cuda.current_stream().wait_stream(side)
             torch.cuda.synchronize()
-            graphs = []
+            graphs, graph_outs = [], []          # graph_outs[r]: the static output tensors that replays of graphs[r] rewrite
             for r in range(R):
                 g = torch.cuda.CUDAGraph()
                 drop_graph_refs()
                 with torch.cuda.graph(g):
-                    step(r)
+                    graph_outs.append(step(r))
                 graphs.append(g)
         except Exception as exc:   # e.g. NCCL capture unsupported: fall back to eager launches of the same kernels
             if rank == 0:
@@ -360,11 +399,11 @@ def run_b200(args) -> None:
             graphs = None
             torch.cuda.synchronize()
 
-    def run_step(i: int):
+    def run_step(i: int) -> dict:
         if graphs is not None:
             graphs[i % R].replay()
-        else:
-            step(i)
+            return graph_outs[i % R]
+        return step(i)
 
     # rough step time (same code path on every rank) to size the load phase before the timed region
     torch.cuda.synchronize()
@@ -399,7 +438,7 @@ def run_b200(args) -> None:
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(args.steps):
-        run_step(i)
+        last = run_step(i)
     e1.record()
     sync_all()
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
@@ -409,6 +448,8 @@ def run_b200(args) -> None:
     clocks = sampler.stop() if rank == 0 else None
     ms_per_step = total_ms / args.steps
     value = world * B * args.steps / (total_ms * 1e-3)
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(args.dump_outputs, last)          # before the passes below replay the graphs again
 
     if args.quick:
         if rank == 0:
@@ -725,10 +766,11 @@ def run_caption_camera(args) -> None:
     imgs = [t.to(dev) for t in imgs_host]
     ws = [torch.rand(B, 3, P, P, generator=g).to(dev) for _ in range(R)]
 
-    def step(i):
+    def step(i) -> dict:
         cam.zero_grad(set_to_none=True)
         sensor, psf, coeffs, loss = cam(imgs[i % R])
         torch.autograd.backward([sensor], [ws[i % R]])
+        return {"sensor": sensor.detach(), "psf": psf.detach(), "grad_defocus": cam.zernike_coeffs_train.grad}
 
     for i in range(3):
         step(i)
@@ -748,23 +790,23 @@ def run_caption_camera(args) -> None:
                     step(i)
             torch.cuda.current_stream(dev).wait_stream(side)
             torch.cuda.synchronize()
-            graphs = []
+            graphs, graph_outs = [], []
             for r in range(R):
                 cam.zero_grad(set_to_none=True)
                 g = torch.cuda.CUDAGraph()
                 with torch.cuda.graph(g):
-                    step(r)
+                    graph_outs.append(step(r))
                 graphs.append(g)
         except Exception as exc:
             print(f"[bench] CUDA graph capture of the caption camera failed ({exc}); timing eager launches", file=sys.stderr)
             graphs = None
             torch.cuda.synchronize()
 
-    def run_step(i):
+    def run_step(i) -> dict:
         if graphs is not None:
             graphs[i % R].replay()
-        else:
-            step(i)
+            return graph_outs[i % R]
+        return step(i)
 
     sampler = ClockSampler(dev.index)
     sampler.start()
@@ -775,15 +817,20 @@ def run_caption_camera(args) -> None:
     for i in range(max(3, args.warmup)):
         run_step(i)
     torch.cuda.synchronize()
-    steps = min(args.steps, 200)
+    steps = args.steps
+    # every step draws the lens tolerance noise from torch's generator (a graph replay reads its state when it runs), and
+    # the spin above runs for a wall-clock time: seed here, so that the timed steps see the same noise on every run
+    torch.manual_seed(0)
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(steps):
-        run_step(i)
+        last = run_step(i)
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / steps
     clocks = sampler.stop()
+    if args.dump_outputs is not None:
+        dump_outputs(args.dump_outputs, last)
     # end to end: pinned host images in, sensor checksum + coefficient gradient out; the host-to-device copy of step i+1 runs on
     # a copy stream beside the compute of step i (two device buffers), as the config-2 e2e leg does.  The module call
     # (cam(img) + backward) is captured once per device buffer in a CUDA graph and replayed; `e2e_eager` = eager calls.

@@ -18,8 +18,8 @@ known-answer artefacts for this path (SURVEY.md section 4 / 8c).  The oracle is
 pinned instead against outputs of the reference module itself, run in the build
 container through ``oracle/ref_shim.py``: ``oracle/make_golden.py`` writes those
 outputs to ``tests/golden/facedeid_*.npz`` and ``tests/test_oracle_vs_golden.py``
-checks this file against them (and, when ``/root/reference`` is mounted, against
-the live reference module).
+checks this file against them (and, when ``B200CAM_REFERENCE_ROOT`` names a
+reference checkout, against the live reference module).
 """
 from __future__ import annotations
 

@@ -1,8 +1,8 @@
 """TEST INFRASTRUCTURE ONLY - generate tests/golden/facedeid_*.npz from the live reference.
 
-Run in the build container (``/root/reference`` mounted):
+Run with a checkout of the reference named by ``B200CAM_REFERENCE_ROOT``:
 
-    python oracle/make_golden.py
+    B200CAM_REFERENCE_ROOT=<reference checkout> python oracle/make_golden.py
 
 Each fixture holds the outputs of the UNMODIFIED reference ``Camera``
 (``Face-DeId/Camera/Optics.py:9``, imported through ``oracle/ref_shim.py``) on the
@@ -82,6 +82,29 @@ def main() -> None:
         print(name, "gap", r["min_top2_gap"].item(), "loss_rad", r["loss_rad"].item(),
               "centering", r["centering_loss"].item(), "bytes", (out_dir / f"{name}.npz").stat().st_size)
     make_caption_fixture(out_dir)
+    make_camera_init_fixture(out_dir, ref_shim.load_face_deid_camera(), "reference")
+
+
+CAMERA_INIT_ATTRS = ("XY", "FF", "XY2", "rho", "rad", "k", "flmb", "lamb", "u", "x2", "fx1", "r", "r2")
+
+
+def make_camera_init_fixture(out_dir: Path, Camera, source: str) -> None:
+    """tests/golden/camera_init_n64_t10.npz: what ``Camera(N=64, zernike_terms=10)`` holds right after construction
+    under torch seed 3 - its state_dict, the buffers the forward reads, the initial lens's height map and phase shift
+    and the names of the trainable parameters.  ``source`` records which ``Camera`` class wrote the file."""
+    torch.manual_seed(3)
+    cam = Camera(N=64, zernike_terms=10)
+    sd = cam.state_dict()
+    payload = {"source": np.array([source]), "torch_version": np.array([torch.__version__]),
+               "state_keys": np.array(list(sd)),
+               "trainable": np.array([n for n, p in cam.named_parameters() if p.requires_grad])}
+    payload.update({f"sd.{k}": v.detach().numpy() for k, v in sd.items()})
+    payload.update({f"attr.{n}": getattr(cam, n).detach().numpy() for n in CAMERA_INIT_ATTRS})
+    with torch.no_grad():
+        payload["heith_map"] = cam.get_Heith_Map().numpy()
+        payload["phase_shift"] = cam.get_phase_shift().numpy()
+    np.savez_compressed(out_dir / "camera_init_n64_t10.npz", **payload)
+    print("wrote camera_init_n64_t10 from", source)
 
 
 def make_caption_fixture(out_dir: Path) -> None:

@@ -1,10 +1,12 @@
 """TEST INFRASTRUCTURE ONLY - import the *unmodified* reference camera modules.
 
-Only usable in the build container, where ``/root/reference`` is mounted
-(read-only).  It does not exist on the GPU box, so nothing under ``-m gpu``,
-``smoke()`` or ``bench.py`` may call into this file.  Its two users are
-``oracle/make_golden.py`` (writes ``tests/golden/*.npz``) and the CPU tests that
-pin ``oracle/camera_oracle.py`` / ``oracle/lens_oracle.py`` to the reference.
+The reference sources are not part of this repository.  They are used only when
+the environment variable ``B200CAM_REFERENCE_ROOT`` names a checkout of
+carlosh93/privacy-preserving-vision; without it ``reference_available()`` is
+False and the tests that need the live reference skip.  Nothing under
+``-m gpu``, ``smoke()`` or ``bench.py`` may call into this file.  Its two users
+are ``oracle/make_golden.py`` (writes ``tests/golden/*.npz``) and the CPU tests
+that pin ``oracle/camera_oracle.py`` / ``oracle/lens_oracle.py`` to the reference.
 
 The reference imports ``matplotlib`` and ``poppy`` at module import time
 (``Face-DeId/Camera/Optics.py:4``, ``Face-DeId/Camera/Utils.py:2-3``,
@@ -24,12 +26,17 @@ import sys
 import types
 from pathlib import Path
 
-REFERENCE_ROOT = Path(os.environ.get("B200CAM_REFERENCE_ROOT", "/root/reference"))
+REFERENCE_ROOT = Path(os.environ["B200CAM_REFERENCE_ROOT"]) if os.environ.get("B200CAM_REFERENCE_ROOT") else None
 _REPO = Path(__file__).resolve().parent.parent
 
 
 def reference_available() -> bool:
-    return (REFERENCE_ROOT / "Face-DeId" / "Camera" / "Optics.py").is_file()
+    if REFERENCE_ROOT is None:
+        return False
+    try:
+        return (REFERENCE_ROOT / "Face-DeId" / "Camera" / "Optics.py").is_file()
+    except OSError:                      # e.g. a path this user may not read
+        return False
 
 
 def _load_zernike():
@@ -79,7 +86,7 @@ def _import_package(alias: str, pkg_dir: Path):
 def load_face_deid_camera():
     """Returns the reference ``Camera`` class (Face-DeId/Camera/Optics.py:9)."""
     if not reference_available():
-        raise RuntimeError(f"reference not mounted at {REFERENCE_ROOT}")
+        raise RuntimeError(f"reference sources not found (B200CAM_REFERENCE_ROOT={REFERENCE_ROOT})")
     _install_stubs()
     _import_package("_ref_facedeid_camera", REFERENCE_ROOT / "Face-DeId" / "Camera")
     return importlib.import_module("_ref_facedeid_camera.Optics").Camera
@@ -87,7 +94,7 @@ def load_face_deid_camera():
 
 def load_face_deid_utils():
     if not reference_available():
-        raise RuntimeError(f"reference not mounted at {REFERENCE_ROOT}")
+        raise RuntimeError(f"reference sources not found (B200CAM_REFERENCE_ROOT={REFERENCE_ROOT})")
     _install_stubs()
     _import_package("_ref_facedeid_camera", REFERENCE_ROOT / "Face-DeId" / "Camera")
     return importlib.import_module("_ref_facedeid_camera.Utils")
@@ -96,7 +103,7 @@ def load_face_deid_utils():
 def load_image_caption_lens():
     """Returns the reference module ``Image_Caption/Camera/Lens.py`` (class OpticsZernike :11)."""
     if not reference_available():
-        raise RuntimeError(f"reference not mounted at {REFERENCE_ROOT}")
+        raise RuntimeError(f"reference sources not found (B200CAM_REFERENCE_ROOT={REFERENCE_ROOT})")
     _install_stubs()
     _import_package("_ref_caption_camera", REFERENCE_ROOT / "Image_Caption" / "Camera")
     return importlib.import_module("_ref_caption_camera.Lens")

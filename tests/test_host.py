@@ -139,7 +139,7 @@ def test_noll_indices_and_orthonormality():
     assert zernike.zernike_volume(64, 5).max() <= 4e-6
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason="/root/reference not mounted")
+@pytest.mark.skipif(not ref_shim.reference_available(), reason="reference sources not present (B200CAM_REFERENCE_ROOT)")
 def test_module_constructs_like_the_reference():
     torch.manual_seed(3)
     ours = Camera(N=64, zernike_terms=10)
@@ -154,6 +154,27 @@ def test_module_constructs_like_the_reference():
     assert torch.equal(ours.get_Heith_Map(), ref.get_Heith_Map())
     assert torch.equal(ours.get_phase_shift(), ref.get_phase_shift())
     ours.load_state_dict(ref.state_dict(), strict=True)
+
+
+def test_module_constructs_like_the_stored_state():
+    """The checks of test_module_constructs_like_the_reference against tests/golden/camera_init_n64_t10.npz, without the
+    live reference.  The file's ``source`` names the Camera class that wrote it (oracle/make_golden.py writes it from the
+    reference); written from this package, it guards the constructor against change rather than pinning it to the
+    reference."""
+    z = np.load(REPO / "tests" / "golden" / "camera_init_n64_t10.npz")
+    torch.manual_seed(3)
+    ours = Camera(N=64, zernike_terms=10)
+    so = ours.state_dict()
+    assert list(so) == z["state_keys"].tolist()
+    assert all(torch.equal(so[k], torch.from_numpy(z[f"sd.{k}"])) for k in so)
+    assert [n for n, p in ours.named_parameters() if p.requires_grad] == z["trainable"].tolist()
+    attrs = [k for k in z.files if k.startswith("attr.")]
+    assert len(attrs) == 13
+    for key in attrs:
+        assert torch.equal(getattr(ours, key[len("attr."):]), torch.from_numpy(z[key])), key
+    with torch.no_grad():
+        assert torch.equal(ours.get_Heith_Map(), torch.from_numpy(z["heith_map"]))
+        assert torch.equal(ours.get_phase_shift(), torch.from_numpy(z["phase_shift"]))
 
 
 def test_state_dict_roundtrip(tmp_path):
@@ -183,14 +204,16 @@ def test_caption_camera_loads_both_reference_checkpoint_layouts():
     assert torch.equal(cam.zernike_coeffs_no_train2.detach(), full[4:] + 1.0)
 
 
-@pytest.mark.skipif(not Path("/root/reference/Image_Caption/Camera/Model.pth").exists(), reason="/root/reference not mounted")
+@pytest.mark.skipif(not (ref_shim.reference_available()
+                         and (ref_shim.REFERENCE_ROOT / "Image_Caption" / "Camera" / "Model.pth").is_file()),
+                    reason="reference sources not present (B200CAM_REFERENCE_ROOT)")
 def test_caption_camera_loads_the_real_reference_checkpoint():
     """SURVEY 8 f3 with the checkpoint the reference ships: Image_Caption/Camera/Model.pth holds {'model': {optics.
     zernike_coeffs_no_train (3,1,1), optics.zernike_coeffs_train (347,1,1)}} - the 3 + (T-3) layout of train.py:71-78 at
     T = 350, which the shipped module's own load_state_dict rejects.  Loaded here into a T = 350 camera (small wave grid:
     the coefficient vector, not the basis, is what the checkpoint defines)."""
     from b200cam.lens import OpticsZernike
-    ck = torch.load("/root/reference/Image_Caption/Camera/Model.pth", map_location="cpu", weights_only=False)
+    ck = torch.load(ref_shim.REFERENCE_ROOT / "Image_Caption" / "Camera" / "Model.pth", map_location="cpu", weights_only=False)
     ref = ck["model"]
     cam = OpticsZernike(input_shape=[None, 16, 16, 3], device="cpu", zernike_terms=350, patch_size=16,
                         wave_resolution=[32, 32], sample_interval=3e-6, height_tolerance=None)
@@ -199,3 +222,24 @@ def test_caption_camera_loads_the_real_reference_checkpoint():
     want = torch.cat((ref["optics.zernike_coeffs_no_train"], ref["optics.zernike_coeffs_train"]), 0)
     assert got.shape == (350, 1, 1) and torch.equal(got.detach(), want)
     assert float(cam.zernike_coeffs_train) == float(ref["optics.zernike_coeffs_train"][0])
+
+
+def test_bench_dump_outputs_stays_in_budget_and_samples_reproducibly(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 .npy files, at most DUMP_BYTES in all; an output too large for that is cut to the
+    same seeded sample of its batch dimension on every run."""
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 100_000)
+    g = torch.Generator().manual_seed(0)
+    outs = {"sensor": torch.rand(40, 3, 16, 16, generator=g), "grad_h": torch.rand(1, 16, 16, generator=g),
+            "loss_rad": torch.tensor(0.5)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), outs)
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["grad_h.npy", "loss_rad.npy", "sensor.npy", "sensor_index.npy"]
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= 100_000
+    idx = np.load(tmp_path / "a" / "sensor_index.npy")
+    sensor = np.load(tmp_path / "a" / "sensor.npy")
+    assert sensor.dtype == np.float32 and 1 <= len(idx) < 40 and np.all(np.diff(idx) > 0)
+    assert np.array_equal(sensor, outs["sensor"].numpy()[idx.astype(int)])
+    assert np.array_equal(idx, np.load(tmp_path / "b" / "sensor_index.npy"))
+    assert np.array_equal(np.load(tmp_path / "a" / "grad_h.npy"), outs["grad_h"].numpy())

@@ -1,5 +1,5 @@
 """CPU: pins ``oracle/lens_oracle.py`` (Image_Caption camera restatement) to the UNMODIFIED reference module
-``Image_Caption/Camera/Lens.py`` (imported through ``oracle/ref_shim.py`` when /root/reference is mounted) and to
+``Image_Caption/Camera/Lens.py`` (imported through ``oracle/ref_shim.py`` when B200CAM_REFERENCE_ROOT is set) and to
 the committed golden vectors written from it by ``oracle/make_golden.py``."""
 import numpy as np
 import pytest
@@ -48,7 +48,7 @@ def test_oracle_matches_golden(case):
     assert abs(float(g[3]) - float(gold["grad_defocus"].reshape(-1)[0])) <= 1e-4 * abs(float(gold["grad_defocus"].reshape(-1)[0]))
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason="/root/reference not mounted")
+@pytest.mark.skipif(not ref_shim.reference_available(), reason="reference sources not present (B200CAM_REFERENCE_ROOT)")
 @pytest.mark.parametrize("case", list(CASES))
 def test_oracle_matches_live_reference(case, tmp_path, monkeypatch):
     monkeypatch.chdir(tmp_path)                                  # the reference caches its Zernike volume in cwd

@@ -2,7 +2,7 @@
 
 1. against the committed golden vectors (outputs of the unmodified reference Camera,
    written by oracle/make_golden.py) - runs anywhere;
-2. against the live reference module when /root/reference is mounted (build container only).
+2. against the live reference module when B200CAM_REFERENCE_ROOT names a reference checkout.
 """
 import pytest
 import torch
@@ -83,7 +83,7 @@ def test_amax_tie_splitting_matches_torch():
     assert rel_l2(gpsf, psf.grad) <= 1e-12
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason="/root/reference not mounted")
+@pytest.mark.skipif(not ref_shim.reference_available(), reason="reference sources not present (B200CAM_REFERENCE_ROOT)")
 @pytest.mark.parametrize("N,B", [(128, 2), (256, 1)])
 def test_oracle_matches_live_reference(N, B):
     Camera = ref_shim.load_face_deid_camera()

@@ -1,5 +1,6 @@
 import sys, time
-sys.path.insert(0, '/root/repo')
+from pathlib import Path
+sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
 import torch
 from b200cam.lens import OpticsZernike
 dev = torch.device("cuda", 0)
