@@ -185,7 +185,8 @@ int b200cam_sensor_finish(const float* psf, float* sensor, float* img_max, int* 
  *     y = conv / max;   NOISE: y += noise_scale * noise[b][c][y][x];   QUANT: y = round(clamp(y, 0, 1) * L) / L,  L = 2^quant_bits - 1
  * `noise` is a caller-supplied standard-normal tensor shaped like the images (draw it with the framework's seeded generator;
  * a fused Philox could not reproduce torch's stream).  b200cam_sensor_bwd treats the epilogue as the identity (straight
- * through).  Same arguments / reference lines as the calls without _ex. */
+ * through).  Same arguments / reference lines as the calls without _ex.  The Image_Caption camera applies the same epilogue
+ * through b200cam_lens_normalise_ex (below). */
 #define B200CAM_SENSOR_NOISE 1
 #define B200CAM_SENSOR_QUANT 2
 int b200cam_sensor_fwd_ex(const float* img, const float* psf, float* sensor, float* img_max, int* tie_count, int* tie_pos,
@@ -263,11 +264,23 @@ int b200cam_lens_psf_bwd(const double* grad_psf_out, const double* grad_loss, co
  *   b200cam_lens_sensor_bwd   adjoint: dL/dconv = sign(raw) (grad_y / gmax - [|raw| == gmax] coef), coef = s / (gmax n) a device
  *                             scalar from the (all-reduced) dot_ties; grad_kernel [3][n][n] summed over the batch (crop it to
  *                             the PSF window), grad_img [B][3][P][P] or NULL
- * workspace: b200cam_lens_sensor_workspace_bytes(P, B), shared by the four calls of a step. */
+ * workspace: b200cam_lens_sensor_workspace_bytes(P, B), shared by the four calls of a step.
+ * Read-out variants (same reference lines, same checks):
+ *   b200cam_lens_sensor_fwd_u8  the forward from uint8 images img [B][3][P][P] (what a decoder or the caption HDF5 store
+ *                               yields, a quarter of the bytes): each value is read as x * fp32(1/255), bit-identical to
+ *                               torch's img.float() / 255.0 on the GPU; the padded image still never exists.  The backward is
+ *                               the same (it reads the saved spectrum and raw, never the image).
+ *   b200cam_lens_normalise_ex   y = |raw| / gmax followed by the opt-in read-out epilogue of b200cam_sensor_fwd_ex
+ *                               (flags B200CAM_SENSOR_NOISE / _QUANT, noise [B][3][P][P] indexed like y; flags = 0 is
+ *                               b200cam_lens_normalise).  b200cam_lens_sensor_dot / _bwd read raw, not y: straight through. */
 size_t b200cam_lens_sensor_workspace_bytes(int P, int B);
 int b200cam_lens_sensor_fwd(const float* img, const float* kernel, float* raw, float* gmax, float* otf, float* spectrum, void* workspace,
                             size_t workspace_bytes, int B, int P, void* stream);
+int b200cam_lens_sensor_fwd_u8(const unsigned char* img, const float* kernel, float* raw, float* gmax, float* otf, float* spectrum,
+                               void* workspace, size_t workspace_bytes, int B, int P, void* stream);
 int b200cam_lens_normalise(const float* raw, const float* gmax, float* y, long long count, void* stream);
+int b200cam_lens_normalise_ex(const float* raw, const float* gmax, float* y, long long count, void* stream, int flags, const float* noise,
+                              float noise_scale, int quant_bits);
 int b200cam_lens_sensor_dot(const float* grad_y, const float* raw, const float* gmax, float* dot_ties, void* workspace, size_t workspace_bytes,
                             int B, int P, void* stream);
 int b200cam_lens_sensor_bwd(const float* grad_y, const float* raw, const float* gmax, const float* coef, const float* otf, const float* spectrum,

@@ -88,7 +88,10 @@ _SIGNATURES = {
                                             ctypes.c_void_p]),
     "b200cam_lens_sensor_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int, ctypes.c_int]),
     "b200cam_lens_sensor_fwd": (ctypes.c_int, [_f, _f, _f, _f, _f, _f, _f, ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_void_p]),
+    "b200cam_lens_sensor_fwd_u8": (ctypes.c_int, [_f, _f, _f, _f, _f, _f, _f, ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_void_p]),
     "b200cam_lens_normalise": (ctypes.c_int, [_f, _f, _f, ctypes.c_longlong, ctypes.c_void_p]),
+    "b200cam_lens_normalise_ex": (ctypes.c_int, [_f, _f, _f, ctypes.c_longlong, ctypes.c_void_p, ctypes.c_int, _f, ctypes.c_float,
+                                                 ctypes.c_int]),
     "b200cam_lens_sensor_dot": (ctypes.c_int, [_f, _f, _f, _f, _f, ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_void_p]),
     "b200cam_lens_sensor_bwd": (ctypes.c_int, [_f, _f, _f, _f, _f, _f, _f, _f, _f, ctypes.c_size_t, ctypes.c_int, ctypes.c_int,
                                                ctypes.c_void_p]),

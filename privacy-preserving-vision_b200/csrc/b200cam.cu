@@ -1789,21 +1789,6 @@ size_t b200cam_spectrum_bytes(int N, int B) {
     return static_cast<size_t>(3) * B * (N / 2 + 1) * N * sizeof(float2);
 }
 
-static int make_epilogue(int flags, const float* noise, float noise_scale, int quant_bits, SensorEpilogue* epi) {
-    *epi = SensorEpilogue{nullptr, 0.f, 0.f};
-    if (flags & ~(B200CAM_SENSOR_NOISE | B200CAM_SENSOR_QUANT)) return B200CAM_E_BAD_SIZE;
-    if (flags & B200CAM_SENSOR_NOISE) {
-        if (noise == nullptr) return B200CAM_E_NULL;
-        epi->noise = noise;
-        epi->noise_scale = noise_scale;
-    }
-    if (flags & B200CAM_SENSOR_QUANT) {
-        if (quant_bits < 1 || quant_bits > 16) return B200CAM_E_BAD_SIZE;
-        epi->levels = static_cast<float>((1 << quant_bits) - 1);
-    }
-    return 0;
-}
-
 int b200cam_sensor_fwd(const float* img, const float* psf, float* sensor, float* img_max, int* tie_count,
                        int* tie_pos, float* otf, float* spectrum, void* workspace, size_t workspace_bytes, int B,
                        int N, void* stream) {

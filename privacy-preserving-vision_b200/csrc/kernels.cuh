@@ -11,6 +11,7 @@
 // Reference lines each body replaces are cited at the body.
 #pragma once
 
+#include "../../include/b200cam.h"
 #include "compat.cuh"
 #include "exec.cuh"
 #include "fft_plan.cuh"
@@ -442,9 +443,12 @@ B200_HD void cols_fwd_body(Exec& ex, const ColsFwdParams& p, float2* smem) {
 // ---------------------------------------------------------------------------------------------
 constexpr int C2R_MAX_TIES = 8;     // = MAX_TIES (declared with the normalise kernel below)
 
-// Opt-in sensor read-out epilogue (north_star step 5; SURVEY trap T6: the reference has NO live sensor noise and no
-// quantisation - its gaussian_noise call is commented out, Image_Caption/Camera/Lens.py:295-301, Utils.py:300-302 - so
-// both are OFF unless asked for):   y <- conv / max ;  y += noise_scale * noise[idx] ;  y <- round(clamp(y,0,1) * L) / L
+// Opt-in sensor read-out epilogue of both cameras (north_star step 5; SURVEY trap T6: the reference has NO live sensor
+// noise and no quantisation - its gaussian_noise call is commented out, Image_Caption/Camera/Lens.py:295-301,
+// Utils.py:300-302 - so both are OFF unless asked for):
+//     y <- conv / max ;  y += noise_scale * noise[idx] ;  y <- round(clamp(y,0,1) * L) / L
+// Face-DeId `Camera`: applied where the sensor kernels write y (one-pass inverse rows, normalise kernel; b200cam.cu);
+// Image_Caption `OpticsZernike`: in the normalise kernel of lens_conv.cu, after the batch-global maximum.
 // `noise` is a caller-supplied N(0,1) tensor shaped like the image batch (drawn with torch's generator, so a run is
 // reproducible against the oracle); L = 2^bits - 1.  The backward is straight through (dL/dconv as if the epilogue
 // were the identity), the usual treatment of a quantiser.
@@ -460,6 +464,22 @@ B200_HD float apply_epilogue(const SensorEpilogue& e, float y, size_t idx) {
         y = rintf(y * e.levels) / e.levels;
     }
     return y;
+}
+// Validates the (flags, noise, noise_scale, quant_bits) arguments of the _ex entry points of both cameras (include/b200cam.h)
+// and builds the epilogue they select; host side, before anything is enqueued.
+inline int make_epilogue(int flags, const float* noise, float noise_scale, int quant_bits, SensorEpilogue* epi) {
+    *epi = SensorEpilogue{nullptr, 0.f, 0.f};
+    if (flags & ~(B200CAM_SENSOR_NOISE | B200CAM_SENSOR_QUANT)) return B200CAM_E_BAD_SIZE;
+    if (flags & B200CAM_SENSOR_NOISE) {
+        if (noise == nullptr) return B200CAM_E_NULL;
+        epi->noise = noise;
+        epi->noise_scale = noise_scale;
+    }
+    if (flags & B200CAM_SENSOR_QUANT) {
+        if (quant_bits < 1 || quant_bits > 16) return B200CAM_E_BAD_SIZE;
+        epi->levels = static_cast<float>((1 << quant_bits) - 1);
+    }
+    return 0;
 }
 
 struct RowsC2RParams {

@@ -7,7 +7,9 @@
 //   here:       the padded image is never written: the row pass transforms the P live rows only (zero columns filled in
 //               shared memory), the column pass reads / writes the P live rows of every spectral column, the inverse row pass
 //               transforms the P rows the crop keeps and writes  raw[i][j] = conv[pt + max(i,1)][pt + max(j,1)]  (signed) plus
-//               the batch maximum of |raw| (integer atomics); one element-wise pass then gives |raw| / max.
+//               the batch maximum of |raw| (integer atomics); one element-wise pass then gives |raw| / max, optionally followed by
+//               the read-out epilogue of kernels.cuh (sensor noise, quantisation).
+// The row pass reads fp32 images or uint8 images (converted in registers exactly as torch's u8.float() / 255.0 on the GPU).
 //   Spectrum traffic is half that of the padded transform, the 4x padded image and the 4x conv output never exist.
 // The backward reads (g, raw) in the loader of the gradient's row pass: dL/dconv = sign(raw) (g / m - tie s / (m n)).
 //
@@ -34,6 +36,13 @@ struct ImgLoad {        // the image itself (Utils.py:266-277)
     __device__ __forceinline__ void init() {}
     __device__ __forceinline__ float operator()(int plane, int r, int c, int P) const {
         return __ldg(x + (static_cast<size_t>(plane) * P + r) * P + c);
+    }
+};
+struct ImgLoadU8 {      // a uint8 image: a quarter of the bytes; = torch's u8.float() / 255.0 on the GPU, which multiplies by the
+    const unsigned char* x;   // [planes][P][P]                                   fp32 reciprocal of a CPU scalar divisor
+    __device__ __forceinline__ void init() {}
+    __device__ __forceinline__ float operator()(int plane, int r, int c, int P) const {
+        return __fmul_rn(static_cast<float>(__ldg(x + (static_cast<size_t>(plane) * P + r) * P + c)), 1.0f / 255.0f);
     }
 };
 struct GradLoad {       // dL/dconv from dL/dy: adjoint of / max, |.|, crop and nearest resize (Utils.py:289-295, Lens.py:312)
@@ -315,13 +324,21 @@ __global__ void __launch_bounds__(ColsSmem<N>::THREADS, N <= 512 ? 2 : 1) k_lcol
     }
 }
 
-// ---- element-wise: y = |raw| / m ; partial sums of g * y and the number of positions that attain m -------------------------
+// ---- element-wise: y = |raw| / m [-> read-out epilogue] ; partial sums of g * y and the number of positions that attain m -----
 constexpr int EWT = 256;
-__global__ void __launch_bounds__(EWT) k_lnormalise(const float4* __restrict__ raw, const float* __restrict__ gmax, float4* __restrict__ y, long long n4) {
+template <bool EPI>
+__global__ void __launch_bounds__(EWT) k_lnormalise(const float4* __restrict__ raw, const float* __restrict__ gmax, float4* __restrict__ y, long long n4,
+                                                    SensorEpilogue epi) {
     const float m = __ldg(gmax);
     for (long long i = blockIdx.x * static_cast<long long>(EWT) + threadIdx.x; i < n4; i += static_cast<long long>(gridDim.x) * EWT) {
         const float4 v = __ldg(raw + i);
-        y[i] = make_float4(fabsf(v.x) / m, fabsf(v.y) / m, fabsf(v.z) / m, fabsf(v.w) / m);
+        float4 o = make_float4(fabsf(v.x) / m, fabsf(v.y) / m, fabsf(v.z) / m, fabsf(v.w) / m);
+        if (EPI) {
+            const size_t e = static_cast<size_t>(i) * 4;
+            o = make_float4(apply_epilogue(epi, o.x, e), apply_epilogue(epi, o.y, e + 1), apply_epilogue(epi, o.z, e + 2),
+                            apply_epilogue(epi, o.w, e + 3));
+        }
+        y[i] = o;
     }
 }
 // part[block] = {sum g y, ties} in double / as a count; fixed order inside a block, blocks summed in order by k_ldot_final
@@ -434,8 +451,8 @@ static cudaError_t optin(K kernel, size_t bytes) {
     return bytes > 48 * 1024 ? cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(bytes)) : cudaSuccess;
 }
 
-template <int N>
-static int fwd_impl(const float* img, const float* kern, float* raw, float* gmax, float2* otf, float2* spectrum, void* wsp, int B, cudaStream_t s) {
+template <int N, class Load>
+static int fwd_impl(Load load, const float* kern, float* raw, float* gmax, float2* otf, float2* spectrum, void* wsp, int B, cudaStream_t s) {
     using T = Tile<N>;
     const float2* tw = lens_twiddle(N);
     if (tw == nullptr) return B200CAM_E_NOT_INIT;
@@ -444,10 +461,10 @@ static int fwd_impl(const float* img, const float* kern, float* raw, float* gmax
     if (rc) return rc;
     const int planes = 3 * B, tiles = (N / 2) / T::ROWS;
     const int colgroups = (3 * T::NC + T::COLS - 1) / T::COLS, nch = lchunks(N, B);
-    LCK(optin(k_lrows_r2c<N, ImgLoad>, RowsR2CSmem<N>::BYTES));
+    LCK(optin(k_lrows_r2c<N, Load>, RowsR2CSmem<N>::BYTES));
     LCK(optin(k_lcols_conv<N>, ColsSmem<N>::BYTES_CONV));
     LCK(optin(k_lrows_c2r<N, 0>, RowsR2CSmem<N>::BYTES));
-    k_lrows_r2c<N, ImgLoad><<<dim3(tiles, planes), RowsR2CSmem<N>::THREADS, RowsR2CSmem<N>::BYTES, s>>>(ImgLoad{img}, spectrum, tw);
+    k_lrows_r2c<N, Load><<<dim3(tiles, planes), RowsR2CSmem<N>::THREADS, RowsR2CSmem<N>::BYTES, s>>>(load, spectrum, tw);
     LLAUNCH();
     k_lcols_conv<N><<<dim3(colgroups, nch), ColsSmem<N>::THREADS, ColsSmem<N>::BYTES_CONV, s>>>(spectrum, ws.st2, otf, tw, B, nch, 0);
     LLAUNCH();
@@ -494,15 +511,10 @@ using namespace b200cam::lconv;
 static bool lens_n_ok(int P) { return P == 64 || P == 128 || P == 256 || P == 512; }
 static bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
-extern "C" {
-
-size_t b200cam_lens_sensor_workspace_bytes(int P, int B) {
-    if (!lens_n_ok(P) || B < 1) return 0;
-    return Ws(nullptr, 2 * P, B).bytes;
-}
-
-int b200cam_lens_sensor_fwd(const float* img, const float* kernel, float* raw, float* gmax, float* otf, float* spectrum, void* workspace,
-                            size_t workspace_bytes, int B, int P, void* stream) {
+// the checks and the dispatch of both forward entry points; `Load` reads the image (ImgLoad: fp32, ImgLoadU8: uint8)
+template <class Load>
+static int lens_fwd(Load load, const void* img, const float* kernel, float* raw, float* gmax, float* otf, float* spectrum, void* workspace,
+                    size_t workspace_bytes, int B, int P, void* stream) {
     if (!lens_n_ok(P) || B < 1) return B200CAM_E_BAD_SIZE;
     if (!img || !kernel || !raw || !gmax || !otf || !spectrum || !workspace) return B200CAM_E_NULL;
     if (!al16(img) || !al16(raw) || !al16(spectrum) || !al16(workspace)) return B200CAM_E_ALIGN;
@@ -512,20 +524,49 @@ int b200cam_lens_sensor_fwd(const float* img, const float* kernel, float* raw, f
     float2* o = reinterpret_cast<float2*>(otf);
     float2* sp = reinterpret_cast<float2*>(spectrum);
     switch (N) {
-        case 128: return fwd_impl<128>(img, kernel, raw, gmax, o, sp, workspace, B, s);
-        case 256: return fwd_impl<256>(img, kernel, raw, gmax, o, sp, workspace, B, s);
-        case 512: return fwd_impl<512>(img, kernel, raw, gmax, o, sp, workspace, B, s);
-        default: return fwd_impl<1024>(img, kernel, raw, gmax, o, sp, workspace, B, s);
+        case 128: return fwd_impl<128>(load, kernel, raw, gmax, o, sp, workspace, B, s);
+        case 256: return fwd_impl<256>(load, kernel, raw, gmax, o, sp, workspace, B, s);
+        case 512: return fwd_impl<512>(load, kernel, raw, gmax, o, sp, workspace, B, s);
+        default: return fwd_impl<1024>(load, kernel, raw, gmax, o, sp, workspace, B, s);
     }
 }
 
+extern "C" {
+
+size_t b200cam_lens_sensor_workspace_bytes(int P, int B) {
+    if (!lens_n_ok(P) || B < 1) return 0;
+    return Ws(nullptr, 2 * P, B).bytes;
+}
+
+int b200cam_lens_sensor_fwd(const float* img, const float* kernel, float* raw, float* gmax, float* otf, float* spectrum, void* workspace,
+                            size_t workspace_bytes, int B, int P, void* stream) {
+    return lens_fwd(ImgLoad{img}, img, kernel, raw, gmax, otf, spectrum, workspace, workspace_bytes, B, P, stream);
+}
+
+int b200cam_lens_sensor_fwd_u8(const unsigned char* img, const float* kernel, float* raw, float* gmax, float* otf, float* spectrum,
+                               void* workspace, size_t workspace_bytes, int B, int P, void* stream) {
+    return lens_fwd(ImgLoadU8{img}, img, kernel, raw, gmax, otf, spectrum, workspace, workspace_bytes, B, P, stream);
+}
+
 int b200cam_lens_normalise(const float* raw, const float* gmax, float* y, long long count, void* stream) {
+    return b200cam_lens_normalise_ex(raw, gmax, y, count, stream, 0, nullptr, 0.f, 0);
+}
+
+int b200cam_lens_normalise_ex(const float* raw, const float* gmax, float* y, long long count, void* stream, int flags, const float* noise,
+                              float noise_scale, int quant_bits) {
+    SensorEpilogue epi;
+    if (const int rc = make_epilogue(flags, noise, noise_scale, quant_bits, &epi)) return rc;
     if (!raw || !gmax || !y) return B200CAM_E_NULL;
     if (count < 0 || count % 4 != 0) return B200CAM_E_BAD_SIZE;
     if (!al16(raw) || !al16(y)) return B200CAM_E_ALIGN;
     if (count == 0) return 0;
-    k_lnormalise<<<ew_grid(count / 4), EWT, 0, static_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const float4*>(raw), gmax,
-                                                                                 reinterpret_cast<float4*>(y), count / 4);
+    const auto r4 = reinterpret_cast<const float4*>(raw);
+    const auto y4 = reinterpret_cast<float4*>(y);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (flags)
+        k_lnormalise<true><<<ew_grid(count / 4), EWT, 0, s>>>(r4, gmax, y4, count / 4, epi);
+    else
+        k_lnormalise<false><<<ew_grid(count / 4), EWT, 0, s>>>(r4, gmax, y4, count / 4, epi);
     LLAUNCH();
     return 0;
 }

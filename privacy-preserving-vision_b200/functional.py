@@ -273,6 +273,18 @@ def zernike_project(coef: torch.Tensor, volume: torch.Tensor, plan: DevicePlan) 
     return ZernikeProject.apply(coef, volume, plan)
 
 
+def read_out(img: torch.Tensor, sigma: float, bits: int, noise: torch.Tensor | None = None):
+    """The opt-in sensor read-out of both cameras (``sensor_noise_sigma`` / ``sensor_quant_bits``): (noise tensor, noise scale,
+    quantisation bits) for the kernels' epilogue, or None when it is off (the reference).  With ``sigma > 0`` and no ``noise``
+    given, the noise is drawn here with torch.randn shaped like ``img`` (torch's global generator: seed it to reproduce)."""
+    sigma, bits = float(sigma), int(bits)
+    if noise is None and sigma > 0.0:
+        noise = torch.randn(img.shape, dtype=torch.float32, device=img.device)
+    if noise is None and bits == 0:
+        return None
+    return (noise, sigma if noise is not None else 0.0, bits)
+
+
 def _check_img(img: torch.Tensor, N: int) -> None:
     if img.dim() != 4 or img.shape[1] != 3 or img.shape[2] != N or img.shape[3] != N:
         raise ValueError(f"expected img of shape (B,3,{N},{N}), got {tuple(img.shape)}")

@@ -19,6 +19,16 @@ What runs where (everything below the Zernike coefficients is b200cam kernels, `
   two, e.g. the constructor default 368) use the reference's own torch expression on the GPU (``_psf``, ``_sensor_torch``,
   ``CircConv`` / ``CropAbsResize`` / ``GlobalMaxNormalise``).
 
+Read-out (no reference counterpart, same meaning as on the Face-DeId ``Camera``)
+* uint8 images (B,3,P,P) are accepted as they are: the row kernel reads them (``b200cam_lens_sensor_fwd_u8``) as
+  ``img.float() / 255.0``, bit for bit, so the host-to-device copy is a quarter of the fp32 one; the other geometries convert
+  with that torch expression;
+* ``sensor_noise_sigma`` / ``sensor_quant_bits`` (default 0 / 0 = the reference): y += sigma * noise, then
+  y = round(clamp(y, 0, 1) * L) / L, L = 2^bits - 1, applied after the batch-global max by the normalise kernel
+  (``b200cam_lens_normalise_ex``; the torch expression elsewhere), straight through in backward.  ``forward(..., noise=)``
+  takes the standard-normal tensor; otherwise it is drawn with ``torch.randn`` after the lens tolerance field.  With
+  ``data_parallel`` each rank draws the noise of its own shard.
+
 Not reproduced: comet.ml summaries (``attach_summaries``), the ``psf_lab`` image file path, ``upsample=True``
 (1792^2 convolution, not a power of two) - they raise ``NotImplementedError`` - and the side effect of caching the
 Zernike volume as ``zernike_volumes/*.npy`` in the working directory (``Lens.py:66-75``).
@@ -172,30 +182,48 @@ class LensSensor(torch.autograd.Function):
     """sensor = |img_psf_conv(img, psf)| / max over the whole batch (Utils.py:251-297 + Lens.py:312) on the pruned kernels of
     ``csrc/lens_conv.cu``: the zero-padded image and the padded convolution output are never materialised.  With a process
     group the maximum is all-reduced (MAX) and, in the backward, sum(g*y) and the tie count (SUM): N ranks reproduce the
-    one-GPU result, the arg-max term landing on the rank(s) that hold the maximum."""
+    one-GPU result, the arg-max term landing on the rank(s) that hold the maximum.
+    ``img`` may be fp32 or uint8 (read by the row kernel as img / 255.0).  ``epilogue``: None or (noise, noise_scale,
+    quant_bits) of ``F.read_out``, applied by the normalise kernel after the maximum; straight through in backward."""
 
     @staticmethod
     @F.nvtx("b200cam.LensSensor.forward")
-    def forward(ctx, img: torch.Tensor, kpad: torch.Tensor, plan: F.DevicePlan, group):
+    def forward(ctx, img: torch.Tensor, kpad: torch.Tensor, plan: F.DevicePlan, group, epilogue=None):
         import torch.distributed as dist
         dev, n = plan.device, plan.N
         P = n // 2
-        x = F._as_f32(img.detach(), dev)
+        lib = plan.lib
+        if img.dtype == torch.uint8:
+            if img.device != dev:
+                raise RuntimeError(f"b200cam: tensor on {img.device}, camera tables on {dev}")
+            x, fwd = img.detach().contiguous(), lib.b200cam_lens_sensor_fwd_u8
+        else:
+            x, fwd = F._as_f32(img.detach(), dev), lib.b200cam_lens_sensor_fwd
         k = F._as_f32(kpad.detach(), dev).reshape(3, n, n)
         B = x.shape[0]
-        lib = plan.lib
-        raw = torch.empty_like(x)
-        y = torch.empty_like(x)
+        flags, noise, noise_scale, quant_bits = 0, None, 0.0, 0
+        if epilogue is not None:
+            noise, noise_scale, quant_bits = epilogue
+            if noise is not None:
+                noise = F._as_f32(noise.detach(), dev)
+                if noise.shape != x.shape:
+                    raise ValueError(f"sensor noise must have the shape of the images {tuple(x.shape)}, got {tuple(noise.shape)}")
+                flags |= 1
+            if quant_bits:
+                flags |= 2
+        raw = torch.empty(x.shape, dtype=torch.float32, device=dev)
+        y = torch.empty_like(raw)
         gmax = torch.zeros(1, dtype=torch.float32, device=dev)
         otf = torch.empty(plan.otf_floats, dtype=torch.float32, device=dev)
         spectrum = torch.empty(lib.b200cam_spectrum_bytes(n, B) // 4, dtype=torch.float32, device=dev)
         ws = torch.empty(lib.b200cam_lens_sensor_workspace_bytes(P, B), dtype=torch.uint8, device=dev)
         with torch.cuda.device(plan.index):
-            _lib.check(lib.b200cam_lens_sensor_fwd(_lib.ptr(x), _lib.ptr(k), _lib.ptr(raw), _lib.ptr(gmax), _lib.ptr(otf),
-                                                   _lib.ptr(spectrum), _lib.ptr(ws), ws.numel(), B, P, F._stream()))
+            _lib.check(fwd(_lib.ptr(x), _lib.ptr(k), _lib.ptr(raw), _lib.ptr(gmax), _lib.ptr(otf), _lib.ptr(spectrum), _lib.ptr(ws),
+                           ws.numel(), B, P, F._stream()))
             if group is not None and dist.is_initialized():
                 dist.all_reduce(gmax, op=dist.ReduceOp.MAX, group=group)
-            _lib.check(lib.b200cam_lens_normalise(_lib.ptr(raw), _lib.ptr(gmax), _lib.ptr(y), raw.numel(), F._stream()))
+            _lib.check(lib.b200cam_lens_normalise_ex(_lib.ptr(raw), _lib.ptr(gmax), _lib.ptr(y), raw.numel(), F._stream(), flags,
+                                                     _lib.ptr(noise), float(noise_scale), int(quant_bits)))
         ctx.plan, ctx.group, ctx.kshape = plan, group, kpad.shape
         ctx.spectrum = spectrum if any(ctx.needs_input_grad[:2]) else None
         ctx.save_for_backward(raw, gmax, otf)
@@ -224,7 +252,7 @@ class LensSensor(torch.autograd.Function):
             _lib.check(lib.b200cam_lens_sensor_bwd(_lib.ptr(gy), _lib.ptr(raw), _lib.ptr(gmax), _lib.ptr(coef), _lib.ptr(otf),
                                                    _lib.ptr(ctx.spectrum), _lib.ptr(grad_k), _lib.ptr(grad_img), _lib.ptr(ws),
                                                    ws.numel(), B, P, F._stream()))
-        return grad_img, grad_k.reshape(ctx.kshape), None, None
+        return grad_img, grad_k.reshape(ctx.kshape), None, None, None
 
 
 class LensPsf(torch.autograd.Function):
@@ -330,6 +358,11 @@ class OpticsZernike(nn.Module):
         self.mask_1 = m1.to(self.device)
         self.mask_2 = m2.to(self.device)
 
+        # opt-in sensor read-out, as on the Face-DeId Camera (the reference's gaussian_noise call is commented out, Lens.py:295-301):
+        # additive Gaussian noise of this standard deviation on the normalised sensor image, then quantisation to this many
+        # bits; 0 / 0 = the reference
+        self.sensor_noise_sigma = 0.0
+        self.sensor_quant_bits = 0
         self._const: dict = {}            # per-device constant tables (wavefront, aperture, transfer function)
         self._plans: dict = {}
         self._process_group = None
@@ -511,8 +544,9 @@ class OpticsZernike(nn.Module):
         x = TF.interpolate(x, size=2 * [up * target], mode="nearest")     # torchvision Resize(interpolation=0)
         return TF.avg_pool2d(x, up, stride=up).permute(0, 2, 3, 1)
 
-    def _sensor(self, img: torch.Tensor, psf: torch.Tensor) -> torch.Tensor:
-        """img_psf_conv (Utils.py:251-297): zero-pad to 2P, circular FFT convolution, abs, crop, nearest resize."""
+    def _sensor(self, img: torch.Tensor, psf: torch.Tensor, epilogue=None) -> torch.Tensor:
+        """img_psf_conv (Utils.py:251-297): zero-pad to 2P, circular FFT convolution, abs, crop, nearest resize; then the batch-global
+        max of Lens.py:312 and the opt-in read-out ``epilogue`` (``F.read_out``).  ``img``: fp32, or uint8 read as img / 255.0."""
         P = img.shape[2]
         if img.dim() != 4 or img.shape[1] != 3 or img.shape[3] != P or psf.shape[1] != P:
             raise ValueError(f"expected images (B,3,{psf.shape[1]},{psf.shape[1]}), got {tuple(img.shape)}")
@@ -522,10 +556,13 @@ class OpticsZernike(nn.Module):
         pad = (n - P) / 2
         pt, pb = int(np.ceil(pad)), int(np.floor(pad))
         fused = P in (64, 128, 256, 512)
+        if not fused and img.dtype == torch.uint8:       # the fused row kernel reads uint8 itself; elsewhere: torch's expression
+            img = img.to(torch.float32) / 255.0
         if not fused and not _lib.load_library().b200cam_supported(n):
             # patch sizes whose padded transform is not a power of two (the constructor default 368 -> 736): the reference's
             # own expression on the GPU (torch.fft), so that every constructor-valid geometry runs
-            return GlobalMaxNormalise.apply(self._sensor_torch(img.to(torch.float32), psf, n, pt, pb), self._process_group)
+            y = GlobalMaxNormalise.apply(self._sensor_torch(img.to(torch.float32), psf, n, pt, pb), self._process_group)
+            return self._read_out_torch(y, epilogue)
         x = None if fused else TF.pad(img.to(torch.float32), [pt, pb, pt, pb])
         # psf2otf (Utils.py:127-158): pad so that the PSF centre lands on n/2, the kernel's "centred frame"
         if (n - P) % 2 != 0:
@@ -534,11 +571,28 @@ class OpticsZernike(nn.Module):
             kt, kb = int(pad) + 1, int(pad) - 1
         k = TF.pad(psf[0].permute(2, 0, 1).to(torch.float32), [kt, kb, kt, kb])          # (3, n, n)
         plan = self._plan(img.device, n)
-        if fused:      # padding, |.|, crop, resize and the batch-global max inside the transform kernels (csrc/lens_conv.cu)
-            return LensSensor.apply(img, k, plan, self._process_group)
+        if fused:      # padding, |.|, crop, resize, the batch-global max and the read-out inside the kernels (csrc/lens_conv.cu)
+            return LensSensor.apply(img, k, plan, self._process_group, epilogue)
         # |.|, the [pt+1 : n-pb] crop to (P-1)^2 and the nearest resize back to P (out[i] = crop[max(i-1,0)]) in one pass
         out = CropAbsResize.apply(CircConv.apply(x, k, plan), P, pt + 1, plan)
-        return GlobalMaxNormalise.apply(out, self._process_group)
+        return self._read_out_torch(GlobalMaxNormalise.apply(out, self._process_group), epilogue)
+
+    @staticmethod
+    def _read_out_torch(y: torch.Tensor, epilogue) -> torch.Tensor:
+        """The read-out epilogue of the kernels (kernels.cuh apply_epilogue) as torch ops, straight through in backward - for
+        the geometries the fused kernels do not cover."""
+        if epilogue is None:
+            return y
+        noise, sigma, bits = epilogue
+        z = y
+        if noise is not None:
+            if noise.shape != y.shape:
+                raise ValueError(f"sensor noise must have the shape of the images {tuple(y.shape)}, got {tuple(noise.shape)}")
+            z = z + sigma * noise.to(y.dtype)
+        if bits:
+            L = float(2 ** bits - 1)
+            z = torch.round(torch.clamp(z, 0.0, 1.0) * L) / L
+        return y + (z - y).detach()
 
     @staticmethod
     def _sensor_torch(img: torch.Tensor, psf: torch.Tensor, n: int, pt: int, pb: int) -> torch.Tensor:
@@ -556,7 +610,11 @@ class OpticsZernike(nn.Module):
         return TF.interpolate(res, size=[P, P], mode="nearest")
 
     # ------------------------------------------------------------------ reference API
-    def forward(self, input_img, new_zernike=None, prueba=None, psf_lab=None, enfoco=None):
+    def forward(self, input_img, new_zernike=None, prueba=None, psf_lab=None, enfoco=None, noise=None):
+        """The reference's forward (Lens.py:157-316).  ``input_img``: (B,3,P,P) fp32, or uint8 (what a decoder or the caption
+        HDF5 store yields; read as input_img / 255.0 on the GPU, a quarter of the host-to-device bytes).  ``noise``: optional
+        standard-normal tensor shaped like the batch for the opt-in sensor noise (``sensor_noise_sigma``); with sigma > 0 and
+        none given it is drawn with torch.randn AFTER the lens tolerance field, so a seeded run draws both in the same order."""
         if psf_lab is True:
             raise NotImplementedError("psf_lab loads '../dataset_paula_real/psf_lab.jpg' in the reference (Lens.py:222-236)")
         if self.upsample:
@@ -582,7 +640,9 @@ class OpticsZernike(nn.Module):
             if prueba == "2" or prueba == "3":
                 psf = psf * self.mask_2
 
-        sensor = self._sensor(input_img, psf)
+        epilogue = (F.read_out(input_img, self.sensor_noise_sigma, self.sensor_quant_bits, noise)
+                    if torch.is_tensor(input_img) else None)
+        sensor = self._sensor(input_img, psf, epilogue)
         np.random.uniform(low=0.001, high=0.02)                     # noise_sigma is drawn and discarded (Lens.py:295)
         return sensor, psf, coeffs, loss                            # (the batch-global max of Lens.py:312 is inside _sensor)
 

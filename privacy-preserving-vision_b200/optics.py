@@ -154,15 +154,6 @@ class Camera(nn.Module):
         self._pending_centering = centering
         return self.psfs
 
-    def _epilogue(self, img, noise):
-        """(noise tensor, sigma, bits) for the kernels, or None when the read-out epilogue is off (the reference)."""
-        sigma, bits = float(self.sensor_noise_sigma), int(self.sensor_quant_bits)
-        if noise is None and sigma > 0.0:
-            noise = torch.randn(img.shape, dtype=torch.float32, device=img.device)     # torch's global generator: seed it to reproduce
-        if noise is None and bits == 0:
-            return None
-        return (noise, sigma if noise is not None else 0.0, bits)
-
     def forward(self, img, noise=None):
         """`noise`: optional standard-normal tensor shaped like `img` for the opt-in sensor noise (drawn here with
         torch.randn when `sensor_noise_sigma > 0` and none is given)."""
@@ -177,7 +168,7 @@ class Camera(nn.Module):
         h_dev = self.Zer_train.device
         overlap = (self.overlap_psf and torch.is_tensor(img) and img.is_cuda and img.dim() == 4 and img.shape[0] > 0
                    and h_dev.type == "cuda")
-        epi = self._epilogue(img, noise) if torch.is_tensor(img) else None
+        epi = F.read_out(img, self.sensor_noise_sigma, self.sensor_quant_bits, noise) if torch.is_tensor(img) else None
         if not overlap:
             psf = self.get_psf()
             self.centering_loss = self._pending_centering
