@@ -14,6 +14,8 @@
  *    (b200cam_init must have been called for that N on that device before capture).
  *  - return value: 0 on success, a positive cudaError_t value, or a negative B200CAM_E_* code.
  *  - N must be one of 64, 128, 256, 512, 1024.
+ *  - bf16 tensors (the _bf16 entry points: sensor image out, its gradient in) cross this ABI as `unsigned short*`: the
+ *    bfloat16 bit patterns (C has no bf16 type), i.e. a torch.bfloat16 tensor's data pointer as it is.
  */
 #ifndef B200CAM_H_
 #define B200CAM_H_
@@ -207,6 +209,29 @@ int b200cam_sensor_bwd(const float* grad_sensor, const float* img, const float* 
                        float* grad_psf, float* grad_img,
                        void* workspace, size_t workspace_bytes, int B, int N, void* stream);
 
+/* bf16 hand-over to a downstream network that runs in bf16 (torch.autocast): the same forward and backward, with the sensor
+ * image written and its gradient read in bf16.  Saves the cast kernels at the boundary: the fp32 image written and re-read
+ * by the cast, the bf16 gradient widened into an fp32 copy.
+ *   b200cam_sensor_fwd_bf16 / _finish_bf16   the arguments of the _ex calls, with the sensor output split in two:
+ *       conv    [B][3][N][N] fp32 scratch: the un-normalised image (caller-owned; dead once the call's kernels have run)
+ *       sensor  [B][3][N][N] bf16 out: the fp32 sensor image after the read-out epilogue, rounded to nearest-even - bit for bit
+ *               the fp32 call's output cast with torch's .to(torch.bfloat16)
+ *   b200cam_sensor_bwd_bf16   b200cam_sensor_bwd with grad_sensor [B][3][N][N] bf16, widened exactly in the row kernels; it
+ *       takes no sensor image (the backward never reads it).  dL/dpsf and dL/dimg are those of b200cam_sensor_bwd on the
+ *       widened gradient, bit for bit.
+ * These always run the default two-pass pipeline: the opt-in B200CAM_PLANE=1 and B200CAM_ONE_PASS=1 kernels are fp32 only
+ * and are not used.  With B200CAM_PLANE=1 at N = 256 b200cam_sensor_rows writes the plane layout, which
+ * b200cam_sensor_finish_bf16 cannot read: it returns B200CAM_E_BAD_SIZE there (use b200cam_sensor_fwd_bf16). */
+int b200cam_sensor_fwd_bf16(const float* img, const float* psf, float* conv, unsigned short* sensor, float* img_max, int* tie_count,
+                            int* tie_pos, float* otf, float* spectrum, void* workspace, size_t workspace_bytes, int B, int N,
+                            void* stream, int flags, const float* noise, float noise_scale, int quant_bits);
+int b200cam_sensor_finish_bf16(const float* psf, float* conv, unsigned short* sensor, float* img_max, int* tie_count, int* tie_pos,
+                               float* otf, const float* spectrum, int otf_ready, void* workspace, size_t workspace_bytes, int B,
+                               int N, void* stream, int flags, const float* noise, float noise_scale, int quant_bits);
+int b200cam_sensor_bwd_bf16(const unsigned short* grad_sensor, const float* img, const float* img_max, const int* tie_count,
+                            const int* tie_pos, const float* psf, const float* otf, const float* spectrum, float* grad_psf,
+                            float* grad_img, void* workspace, size_t workspace_bytes, int B, int N, void* stream);
+
 /* Plain circular convolution of a batch with one centred kernel per channel, and its adjoints.  Replaces the FFT
  * part of img_psf_conv (Image_Caption/Camera/Utils.py:251-297): the caller zero-pads image and PSF to N (a power of
  * two, Utils.py:266-277 and psf2otf :127-158), then
@@ -272,7 +297,11 @@ int b200cam_lens_psf_bwd(const double* grad_psf_out, const double* grad_loss, co
  *                               the same (it reads the saved spectrum and raw, never the image).
  *   b200cam_lens_normalise_ex   y = |raw| / gmax followed by the opt-in read-out epilogue of b200cam_sensor_fwd_ex
  *                               (flags B200CAM_SENSOR_NOISE / _QUANT, noise [B][3][P][P] indexed like y; flags = 0 is
- *                               b200cam_lens_normalise).  b200cam_lens_sensor_dot / _bwd read raw, not y: straight through. */
+ *                               b200cam_lens_normalise).  b200cam_lens_sensor_dot / _bwd read raw, not y: straight through.
+ * bf16 variants (a downstream network in bf16): same arguments and checks, y / grad_y as bf16 bit patterns.
+ *   b200cam_lens_normalise_bf16   b200cam_lens_normalise_ex rounded to nearest-even as the last step (= its output cast with
+ *                                 torch); b200cam_lens_sensor_dot_bf16 / _bwd_bf16 read grad_y in bf16, widened exactly, and
+ *                                 equal the fp32 calls on the widened gradient, bit for bit. */
 size_t b200cam_lens_sensor_workspace_bytes(int P, int B);
 int b200cam_lens_sensor_fwd(const float* img, const float* kernel, float* raw, float* gmax, float* otf, float* spectrum, void* workspace,
                             size_t workspace_bytes, int B, int P, void* stream);
@@ -285,6 +314,13 @@ int b200cam_lens_sensor_dot(const float* grad_y, const float* raw, const float* 
                             int B, int P, void* stream);
 int b200cam_lens_sensor_bwd(const float* grad_y, const float* raw, const float* gmax, const float* coef, const float* otf, const float* spectrum,
                             float* grad_kernel, float* grad_img, void* workspace, size_t workspace_bytes, int B, int P, void* stream);
+int b200cam_lens_normalise_bf16(const float* raw, const float* gmax, unsigned short* y, long long count, void* stream, int flags,
+                                const float* noise, float noise_scale, int quant_bits);
+int b200cam_lens_sensor_dot_bf16(const unsigned short* grad_y, const float* raw, const float* gmax, float* dot_ties, void* workspace,
+                                 size_t workspace_bytes, int B, int P, void* stream);
+int b200cam_lens_sensor_bwd_bf16(const unsigned short* grad_y, const float* raw, const float* gmax, const float* coef, const float* otf,
+                                 const float* spectrum, float* grad_kernel, float* grad_img, void* workspace, size_t workspace_bytes, int B,
+                                 int P, void* stream);
 
 #ifdef __cplusplus
 }

@@ -95,6 +95,20 @@ _SIGNATURES = {
     "b200cam_lens_sensor_dot": (ctypes.c_int, [_f, _f, _f, _f, _f, ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_void_p]),
     "b200cam_lens_sensor_bwd": (ctypes.c_int, [_f, _f, _f, _f, _f, _f, _f, _f, _f, ctypes.c_size_t, ctypes.c_int, ctypes.c_int,
                                                ctypes.c_void_p]),
+    # bf16 sensor image out / gradient in (unsigned short* bit patterns: passed as plain device pointers)
+    "b200cam_sensor_fwd_bf16": (ctypes.c_int, [_f, _f, _f, _f, _f, _f, _f, _f, _f,
+                                               _f, ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_void_p,
+                                               ctypes.c_int, _f, ctypes.c_float, ctypes.c_int]),
+    "b200cam_sensor_finish_bf16": (ctypes.c_int, [_f, _f, _f, _f, _f, _f, _f, _f, ctypes.c_int,
+                                                  _f, ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_void_p,
+                                                  ctypes.c_int, _f, ctypes.c_float, ctypes.c_int]),
+    "b200cam_sensor_bwd_bf16": (ctypes.c_int, [_f, _f, _f, _f, _f, _f, _f, _f, _f, _f,
+                                               _f, ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_void_p]),
+    "b200cam_lens_normalise_bf16": (ctypes.c_int, [_f, _f, _f, ctypes.c_longlong, ctypes.c_void_p, ctypes.c_int, _f, ctypes.c_float,
+                                                   ctypes.c_int]),
+    "b200cam_lens_sensor_dot_bf16": (ctypes.c_int, [_f, _f, _f, _f, _f, ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_void_p]),
+    "b200cam_lens_sensor_bwd_bf16": (ctypes.c_int, [_f, _f, _f, _f, _f, _f, _f, _f, _f, ctypes.c_size_t, ctypes.c_int, ctypes.c_int,
+                                                    ctypes.c_void_p]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 

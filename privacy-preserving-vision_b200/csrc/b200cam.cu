@@ -6,6 +6,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <mutex>
+#include <type_traits>
 #include <utility>
 
 #include "../../include/b200cam.h"
@@ -29,8 +30,8 @@ __device__ __forceinline__ void pdl_gate() {
 }
 #define SMEM2 reinterpret_cast<float2*>(smem_raw)
 
-template <int N>
-__global__ void __launch_bounds__(RowsR2CSmem<N>::THREADS) k_rows_r2c(RowsR2CParams p) {
+template <int N, class In = float>
+__global__ void __launch_bounds__(RowsR2CSmem<N>::THREADS) k_rows_r2c(RowsR2CParamsT<In> p) {
     pdl_gate();
     DeviceExec ex;
     rows_r2c_body<N>(ex, p, SMEM2);
@@ -38,8 +39,8 @@ __global__ void __launch_bounds__(RowsR2CSmem<N>::THREADS) k_rows_r2c(RowsR2CPar
 // the same row pass as a persistent grid of `gridDim.x` CTAs walking the tiles: the number of resident CTAs per SM is
 // then the launch's choice, not the occupancy limit - used for the image rows that run BESIDE the PSF chain, whose
 // small high-priority kernels need free registers / shared memory on every SM the moment they are launched
-template <int N>
-__global__ void __launch_bounds__(RowsStreamSmem<N>::THREADS) k_rows_r2c_persist(RowsR2CParams p, int tiles_total) {
+template <int N, class In = float>
+__global__ void __launch_bounds__(RowsStreamSmem<N, In>::THREADS) k_rows_r2c_persist(RowsR2CParamsT<In> p, int tiles_total) {
     pdl_gate();
     DeviceExec ex;
     rows_r2c_stream_body<N>(ex, p, SMEM2, tiles_total, static_cast<int>(gridDim.x));
@@ -74,6 +75,12 @@ __global__ void __launch_bounds__(EW_THREADS) k_normalise(NormaliseParams p) {
     pdl_gate();
     DeviceExec ex;
     normalise_body(ex, p, gridDim.x);
+}
+// bf16 sensor image: reads the fp32 conv (p.y), writes the rounded image to `out`
+__global__ void __launch_bounds__(EW_THREADS) k_normalise_bf16(NormaliseParams p, bf16* out) {
+    pdl_gate();
+    DeviceExec ex;
+    normalise_body<bf16>(ex, p, gridDim.x, out);
 }
 template <int N>
 __global__ void __launch_bounds__(ColsSmem<N>::THREADS, N <= 256 ? 3 : 1) k_cols_accum(ColsAccumParams p) {
@@ -566,6 +573,7 @@ struct DeviceState {
     int conv_slots[11] = {0}, accum_slots[11] = {0};     // resident CTAs of the persistent column kernels
     cudaEvent_t chain_ev = nullptr;                      // orders a caller stream behind the first PSF-chain kernel
     int r2c_fit[11] = {0}, c2r_fit[11] = {0};            // resident CTAs per SM of the persistent row kernels
+    int r2c16_fit[11] = {0};                             // ... and of the bf16-input forward row kernel (upstream gradient)
     float* scratch = nullptr;                            // SCRATCH_FLOATS floats: slice partials of the Zernike adjoint
     int prow_fit = 0, pconv_g3 = 0, pacc_g3 = 0;         // plane kernels (N = 256): resident CTAs per SM / co-resident cluster triples
     unsigned* err_host = nullptr; unsigned* err_dev = nullptr;   // device error word (mapped pinned host memory)
@@ -618,6 +626,8 @@ static cudaError_t init_kernels() {
     if ((e = optin(k_rows_r2c<N>, RowsR2CSmem<N>::BYTES))) return e;
     if ((e = optin(k_rows_c2r<N>, RowsR2CSmem<N>::BYTES))) return e;
     if ((e = optin(k_rows_r2c_persist<N>, RowsStreamSmem<N>::BYTES))) return e;
+    if ((e = optin(k_rows_r2c<N, bf16>, RowsR2CSmem<N>::BYTES))) return e;
+    if ((e = optin(k_rows_r2c_persist<N, bf16>, RowsStreamSmem<N, bf16>::BYTES))) return e;
     if ((e = optin(k_rows_c2r_persist<N, false>, RowsC2RStreamSmem<N>::BYTES))) return e;
     if ((e = optin(k_rows_c2r_persist<N, true>, RowsC2RStreamSmem<N>::BYTES))) return e;
     if ((e = optin(k_cols_conv<N>, ColsSmem<N>::BYTES_CONV))) return e;
@@ -653,9 +663,11 @@ static cudaError_t coop_grid_size(int dev, int sms, int* out) {
 
 // resident CTAs (one wave) of the persistent column kernels on this device
 template <int N>
-static cudaError_t row_fits(int* r2c, int* c2r) {
+static cudaError_t row_fits(int* r2c, int* r2c16, int* c2r) {
     cudaError_t e;
     if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(r2c, k_rows_r2c_persist<N>, RowsStreamSmem<N>::THREADS, RowsStreamSmem<N>::BYTES))) return e;
+    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(r2c16, k_rows_r2c_persist<N, bf16>, RowsStreamSmem<N, bf16>::THREADS,
+                                                           RowsStreamSmem<N, bf16>::BYTES))) return e;
     return cudaOccupancyMaxActiveBlocksPerMultiprocessor(c2r, k_rows_c2r_persist<N, false>, RowsC2RStreamSmem<N>::THREADS, RowsC2RStreamSmem<N>::BYTES);
 }
 template <int N>
@@ -728,9 +740,10 @@ static int persistent_grid(int fit, int want_per_sm, int total_tiles) {
     const long long cap = static_cast<long long>(sms) * per_sm;
     return static_cast<int>(total_tiles < cap ? total_tiles : cap);
 }
-static int rows_fit(int N, bool inverse) {
+static int rows_fit(int N, bool inverse, bool bf16_input = false) {
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= MAX_DEV) return 1;
+    if (bf16_input) return g_state[dev].r2c16_fit[log2i(N)];
     return inverse ? g_state[dev].c2r_fit[log2i(N)] : g_state[dev].r2c_fit[log2i(N)];
 }
 
@@ -1029,15 +1042,17 @@ static int otf_cols_impl(const float2* rows, float2* otf, const float2* tw, floa
 
 // first half of the generic forward: row transforms of the images (independent of the PSF, so a caller may run it on a
 // second stream while b200cam_psf_fwd is still busy); also resets the per-image max / tie counters
+// allow_plane = false: always the standard spectrum layout (the bf16 sensor path runs the default two-pass pipeline only)
 template <int N>
-static int sensor_rows_impl(const float* img, float2* srow, float* img_max, int* tie_count, int B, cudaStream_t s) {
+static int sensor_rows_impl(const float* img, float2* srow, float* img_max, int* tie_count, int B, cudaStream_t s,
+                            bool allow_plane = true) {
     using T = Tile<N>;
     const float2* tw = twiddle(N);
     if (tw == nullptr) return B200CAM_E_NOT_INIT;
     // B200CAM_ROWS_PER_SM resident CTAs per SM (default 3 of the 4 that fit): see k_rows_r2c_persist
     static const int per_sm = [] { const char* e = getenv("B200CAM_ROWS_PER_SM"); const int v = e ? atoi(e) : 3; return v > 0 ? v : 3; }();
     if constexpr (N == 256) {
-        if (plane_selected()) {
+        if (allow_plane && plane_selected()) {
             // plane layout "A"; the words behind it (the buffer is sized for 129 columns, A uses 128) hold the per-image
             // {max key, arrivals} pairs of k_pconv: reset here, early, beside the PSF chain
             const DeviceState* st = cur_state();
@@ -1061,10 +1076,12 @@ static int sensor_rows_impl(const float* img, float2* srow, float* img_max, int*
 }
 
 // second half: OTF of the PSF, column convolution, inverse rows + per-image max, normalise
+// out16 != nullptr: bf16 sensor image.  `sensor` is then the fp32 conv scratch, and the default two-pass pipeline runs
+// whatever B200CAM_PLANE / B200CAM_ONE_PASS say (those opt-in kernels write fp32 only).
 template <int N>
 static int sensor_finish_impl(const float* psf, float* sensor, float* img_max, int* tie_count, int* tie_pos, float2* otf,
                               const float2* srow, const SensorWs& ws, int B, int otf_ready, cudaStream_t s,
-                              SensorEpilogue epi = SensorEpilogue{nullptr, 0.f, 0.f}) {
+                              SensorEpilogue epi = SensorEpilogue{nullptr, 0.f, 0.f}, bf16* out16 = nullptr) {
     using T = Tile<N>;
     const float2* tw = twiddle(N);
     if (tw == nullptr) return B200CAM_E_NOT_INIT;
@@ -1074,7 +1091,7 @@ static int sensor_finish_impl(const float* psf, float* sensor, float* img_max, i
     }
     const int planes = 3 * B;
     if constexpr (N == 256) {
-        if (plane_selected() && epi.noise == nullptr && epi.levels <= 0.f) {      // (the opt-in plane kernels have no read-out epilogue)
+        if (out16 == nullptr && plane_selected() && epi.noise == nullptr && epi.levels <= 0.f) {   // (the opt-in plane kernels have no read-out epilogue)
             const DeviceState* st = cur_state();
             if (st == nullptr || st->pconv_g3 < 1) return B200CAM_E_NOT_INIT;
             const int G3 = B < st->pconv_g3 ? B : st->pconv_g3;
@@ -1096,7 +1113,7 @@ static int sensor_finish_impl(const float* psf, float* sensor, float* img_max, i
     // previous tile's outputs (128 registers / thread at 4 CTAs per SM) that costs the time, not the waiting.
     static const int one_pass = [] { const char* e = getenv("B200CAM_ONE_PASS"); return e ? atoi(e) : 0; }();
     constexpr bool FUSABLE = (Plan<N>::R1 <= 16) && (Plan<N>::LANES == Plan<N>::R2);
-    const bool fused = FUSABLE && one_pass && per_sm > 0;
+    const bool fused = FUSABLE && one_pass && per_sm > 0 && out16 == nullptr;
     launch_k(k_cols_conv<N>, dim3(colgroups, nchunks), ColsSmem<N>::THREADS, ColsSmem<N>::BYTES_CONV, s, 
         ColsConvParams{srow, ws.st2, otf, tw, nullptr, B, nchunks, 0, 1.0f, fused ? ws.arrive : nullptr, fused ? 64 * B : 0});
     LAUNCH_CHECK();
@@ -1124,7 +1141,10 @@ static int sensor_finish_impl(const float* psf, float* sensor, float* img_max, i
     LAUNCH_CHECK();
     const long long n4 = static_cast<long long>(planes) * N * N / 4;
     const int grid = static_cast<int>(n4 / EW_THREADS < 148 * 8 ? (n4 + EW_THREADS - 1) / EW_THREADS : 148 * 8);
-    launch_k(k_normalise, grid, EW_THREADS, 0, s, NormaliseParams{sensor, img_max, tie_count, tie_pos, n4, 3 * N * N / 4, epi});
+    if (out16 != nullptr)
+        launch_k(k_normalise_bf16, grid, EW_THREADS, 0, s, NormaliseParams{sensor, img_max, tie_count, tie_pos, n4, 3 * N * N / 4, epi}, out16);
+    else
+        launch_k(k_normalise, grid, EW_THREADS, 0, s, NormaliseParams{sensor, img_max, tie_count, tie_pos, n4, 3 * N * N / 4, epi});
     LAUNCH_CHECK();
     return 0;
 }
@@ -1253,16 +1273,18 @@ static int conv_bwd_impl(const float* g, const float* img, const float2* otf, co
 template <int N>
 static int sensor_fwd_impl(const float* img, const float* psf, float* sensor, float* img_max, int* tie_count,
                            int* tie_pos, float2* otf, float2* spectrum, void* ws_ptr, int B, cudaStream_t s,
-                           SensorEpilogue epi = SensorEpilogue{nullptr, 0.f, 0.f}) {
+                           SensorEpilogue epi = SensorEpilogue{nullptr, 0.f, 0.f}, bf16* out16 = nullptr) {
     SensorWs ws(ws_ptr, N, B, false);
     float2* srow = spectrum != nullptr ? spectrum : ws.stx;      // row spectra: kept for the backward when asked
-    int rc = sensor_rows_impl<N>(img, srow, img_max, tie_count, B, s);
+    int rc = sensor_rows_impl<N>(img, srow, img_max, tie_count, B, s, out16 == nullptr);
     if (rc) return rc;
-    return sensor_finish_impl<N>(psf, sensor, img_max, tie_count, tie_pos, otf, srow, ws, B, 0, s, epi);
+    return sensor_finish_impl<N>(psf, sensor, img_max, tie_count, tie_pos, otf, srow, ws, B, 0, s, epi, out16);
 }
 
-template <int N>
-static int sensor_bwd_impl(const float* g, const float* img, const float* sensor, const float* img_max,
+// In = bf16: the upstream gradient arrives in bf16 and is widened in the row kernels; everything after them is the fp32
+// pipeline (the plane kernels are fp32 only: the bf16 path always runs the generic one)
+template <int N, class In = float>
+static int sensor_bwd_impl(const In* g, const float* img, const float* sensor, const float* img_max,
                            const int* tie_count, const int* tie_pos, const float* psf, const float2* otf,
                            const float2* spectrum, float* grad_psf, float* grad_img, void* ws_ptr, int B,
                            cudaStream_t s) {
@@ -1272,7 +1294,7 @@ static int sensor_bwd_impl(const float* g, const float* img, const float* sensor
     SensorWs ws(ws_ptr, N, B, true);
     const int planes = 3 * B, tiles = N / T::ROWS;
     const dim3 rgrid(tiles, planes);
-    if constexpr (N == 256) {
+    if constexpr (N == 256 && std::is_same<In, float>::value) {
         if (plane_selected()) {
             const DeviceState* st = cur_state();
             if (st == nullptr || st->pacc_g3 < 1 || st->pconv_g3 < 1) return B200CAM_E_NOT_INIT;
@@ -1335,11 +1357,11 @@ static int sensor_bwd_impl(const float* g, const float* img, const float* sensor
         static const int per_sm = [] { const char* e = getenv("B200CAM_GROWS_PER_SM"); return e ? atoi(e) : 3; }();
         if (per_sm > 0) {
             const int total = tiles * planes;
-            const int grid = persistent_grid(rows_fit(N, false), per_sm, total);
-            launch_k(k_rows_r2c_persist<N>, grid, RowsStreamSmem<N>::THREADS, RowsStreamSmem<N>::BYTES, s, 
-                RowsR2CParams{g, ws.stg, tw, nullptr, nullptr}, total);
+            const int grid = persistent_grid(rows_fit(N, false, !std::is_same<In, float>::value), per_sm, total);
+            launch_k(k_rows_r2c_persist<N, In>, grid, RowsStreamSmem<N, In>::THREADS, RowsStreamSmem<N, In>::BYTES, s,
+                RowsR2CParamsT<In>{g, ws.stg, tw, nullptr, nullptr}, total);
         } else {
-            launch_k(k_rows_r2c<N>, rgrid, RowsR2CSmem<N>::THREADS, RowsR2CSmem<N>::BYTES, s, RowsR2CParams{g, ws.stg, tw, nullptr, nullptr});
+            launch_k(k_rows_r2c<N, In>, rgrid, RowsR2CSmem<N>::THREADS, RowsR2CSmem<N>::BYTES, s, RowsR2CParamsT<In>{g, ws.stg, tw, nullptr, nullptr});
         }
     }
     LAUNCH_CHECK();
@@ -1550,13 +1572,14 @@ int b200cam_init(int N) {
     }
     if (e == cudaSuccess) {
         int* rf = &g_state[dev].r2c_fit[l];
+        int* rf16 = &g_state[dev].r2c16_fit[l];
         int* cf = &g_state[dev].c2r_fit[l];
         switch (N) {
-            case 64: e = row_fits<64>(rf, cf); break;
-            case 128: e = row_fits<128>(rf, cf); break;
-            case 256: e = row_fits<256>(rf, cf); break;
-            case 512: e = row_fits<512>(rf, cf); break;
-            case 1024: e = row_fits<1024>(rf, cf); break;
+            case 64: e = row_fits<64>(rf, rf16, cf); break;
+            case 128: e = row_fits<128>(rf, rf16, cf); break;
+            case 256: e = row_fits<256>(rf, rf16, cf); break;
+            case 512: e = row_fits<512>(rf, rf16, cf); break;
+            case 1024: e = row_fits<1024>(rf, rf16, cf); break;
         }
     }
     if (e != cudaSuccess) {
@@ -1902,6 +1925,58 @@ int b200cam_sensor_bwd(const float* grad_sensor, const float* img, const float* 
     DISPATCH_N(N, (sensor_bwd_impl<NN_>(grad_sensor, img, sensor, img_max, tie_count, tie_pos, psf,
                                         reinterpret_cast<const float2*>(otf), spec, grad_psf, grad_img, workspace,
                                         B, s)));
+}
+
+// ---- bf16 sensor image / bf16 upstream gradient ------------------------------------------------------------
+// `conv` [B][3][N][N] fp32 scratch (the un-normalised image; free once the call's work has run), `sensor` bf16 bit patterns
+int b200cam_sensor_fwd_bf16(const float* img, const float* psf, float* conv, unsigned short* sensor, float* img_max, int* tie_count,
+                            int* tie_pos, float* otf, float* spectrum, void* workspace, size_t workspace_bytes, int B, int N,
+                            void* stream, int flags, const float* noise, float noise_scale, int quant_bits) {
+    SensorEpilogue epi;
+    if (const int rc = make_epilogue(flags, noise, noise_scale, quant_bits, &epi)) return rc;
+    if (!b200cam_supported(N) || B < 1) return B200CAM_E_BAD_SIZE;
+    if (!img || !psf || !conv || !sensor || !img_max || !tie_count || !tie_pos || !otf || !workspace) return B200CAM_E_NULL;
+    if (workspace_bytes < b200cam_sensor_workspace_bytes(N, B, 0)) return B200CAM_E_WORKSPACE;
+    if (!aligned16(img) || !aligned16(conv) || !aligned16(sensor) || !aligned16(otf) || !aligned16(workspace) || !aligned16(psf) ||
+        (spectrum != nullptr && !aligned16(spectrum)))
+        return B200CAM_E_ALIGN;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    bf16* out = reinterpret_cast<bf16*>(sensor);
+    DISPATCH_N(N, (sensor_fwd_impl<NN_>(img, psf, conv, img_max, tie_count, tie_pos, reinterpret_cast<float2*>(otf),
+                                        reinterpret_cast<float2*>(spectrum), workspace, B, s, epi, out)));
+}
+
+int b200cam_sensor_finish_bf16(const float* psf, float* conv, unsigned short* sensor, float* img_max, int* tie_count, int* tie_pos,
+                               float* otf, const float* spectrum, int otf_ready, void* workspace, size_t workspace_bytes, int B,
+                               int N, void* stream, int flags, const float* noise, float noise_scale, int quant_bits) {
+    SensorEpilogue epi;
+    if (const int rc = make_epilogue(flags, noise, noise_scale, quant_bits, &epi)) return rc;
+    if (!b200cam_supported(N) || B < 1) return B200CAM_E_BAD_SIZE;
+    if (N == 256 && plane_selected()) return B200CAM_E_BAD_SIZE;     // b200cam_sensor_rows wrote the plane layout
+    if (!psf || !conv || !sensor || !img_max || !tie_count || !tie_pos || !otf || !spectrum || !workspace) return B200CAM_E_NULL;
+    if (workspace_bytes < b200cam_sensor_workspace_bytes(N, B, 0)) return B200CAM_E_WORKSPACE;
+    if (!aligned16(conv) || !aligned16(sensor) || !aligned16(otf) || !aligned16(workspace) || !aligned16(psf) || !aligned16(spectrum))
+        return B200CAM_E_ALIGN;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    bf16* out = reinterpret_cast<bf16*>(sensor);
+    DISPATCH_N(N, (sensor_finish_impl<NN_>(psf, conv, img_max, tie_count, tie_pos, reinterpret_cast<float2*>(otf),
+                                           reinterpret_cast<const float2*>(spectrum), SensorWs(workspace, NN_, B, false),
+                                           B, otf_ready, s, epi, out)));
+}
+
+int b200cam_sensor_bwd_bf16(const unsigned short* grad_sensor, const float* img, const float* img_max, const int* tie_count,
+                            const int* tie_pos, const float* psf, const float* otf, const float* spectrum, float* grad_psf,
+                            float* grad_img, void* workspace, size_t workspace_bytes, int B, int N, void* stream) {
+    if (!b200cam_supported(N) || B < 1) return B200CAM_E_BAD_SIZE;
+    if (!grad_sensor || !img || !img_max || !tie_count || !tie_pos || !psf || !otf || !grad_psf || !workspace) return B200CAM_E_NULL;
+    if (workspace_bytes < b200cam_sensor_workspace_bytes(N, B, grad_img != nullptr)) return B200CAM_E_WORKSPACE;
+    if (!aligned16(grad_sensor) || !aligned16(img) || !aligned16(otf) || !aligned16(workspace) || !aligned16(grad_psf) ||
+        (spectrum && !aligned16(spectrum)) || (grad_img && !aligned16(grad_img)))
+        return B200CAM_E_ALIGN;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const bf16* g = reinterpret_cast<const bf16*>(grad_sensor);
+    DISPATCH_N(N, (sensor_bwd_impl<NN_, bf16>(g, img, nullptr, img_max, tie_count, tie_pos, psf, reinterpret_cast<const float2*>(otf),
+                                              reinterpret_cast<const float2*>(spectrum), grad_psf, grad_img, workspace, B, s)));
 }
 
 }  // extern "C"

@@ -12,6 +12,7 @@
 #include <cstring>
 
 #if defined(__CUDACC__)
+#include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #define B200_HD __host__ __device__ __forceinline__
 #define B200_D __device__ __forceinline__
@@ -58,6 +59,66 @@ B200_HD T ld_ro(const T* p) {
     return __ldg(p);
 #else
     return *p;
+#endif
+}
+
+// ---- bf16 sensor images / gradients ---------------------------------------------------------
+// A bfloat16 value as its bit pattern (it crosses the C ABI as unsigned short: C has no bf16 type).  Widening to fp32 is
+// exact (the 16 bits become the high half of the float); narrowing rounds to nearest-even, as torch's .to(torch.bfloat16).
+struct bf16 {
+    unsigned short bits;
+};
+B200_HD float to_float(float v) { return v; }
+B200_HD float to_float(bf16 v) {
+    const uint32_t u = static_cast<uint32_t>(v.bits) << 16;
+#if defined(__CUDA_ARCH__)
+    return __uint_as_float(u);
+#else
+    float f;
+    std::memcpy(&f, &u, 4);
+    return f;
+#endif
+}
+// element loads through the read-only path (fp32, or bf16 widened in registers)
+B200_HD float load_elem(const float* p) { return ld_ro(p); }
+B200_HD float load_elem(const bf16* p) { return to_float(bf16{ld_ro(reinterpret_cast<const unsigned short*>(p))}); }
+// fp32 -> bf16, round to nearest-even.  Device: __float2bfloat16_rn (the conversion torch's CUDA cast uses).  Host (emulator):
+// the same bit rule - add 0x7fff plus the lowest kept bit, truncate - which gives the identical result for every finite
+// value and for the infinities; NaN becomes the canonical quiet NaN of its sign.
+B200_HD unsigned short bf16_bits_rn(float v) {
+#if defined(__CUDA_ARCH__)
+    return __bfloat16_as_ushort(__float2bfloat16_rn(v));
+#else
+    uint32_t u;
+    std::memcpy(&u, &v, 4);
+    if ((u & 0x7fffffffu) > 0x7f800000u) return static_cast<unsigned short>(((u >> 16) & 0x8000u) | 0x7fc0u);
+    return static_cast<unsigned short>((u + 0x7fffu + ((u >> 16) & 1u)) >> 16);
+#endif
+}
+// four outputs of an element-wise pass: fp32 as one float4 store, bf16 as one 8-byte store
+B200_HD void store4(float* base, long long i4, float a, float b, float c, float d) {
+    reinterpret_cast<float4*>(base)[i4] = make_float4(a, b, c, d);
+}
+B200_HD void store4(bf16* base, long long i4, float a, float b, float c, float d) {
+    const uint32_t lo = static_cast<uint32_t>(bf16_bits_rn(a)) | (static_cast<uint32_t>(bf16_bits_rn(b)) << 16);
+    const uint32_t hi = static_cast<uint32_t>(bf16_bits_rn(c)) | (static_cast<uint32_t>(bf16_bits_rn(d)) << 16);
+#if defined(__CUDACC__)
+    reinterpret_cast<uint2*>(base)[i4] = make_uint2(lo, hi);
+#else
+    uint32_t* p = reinterpret_cast<uint32_t*>(base) + 2 * i4;
+    p[0] = lo;
+    p[1] = hi;
+#endif
+}
+// four consecutive gradient values (16-byte fp32 / 8-byte bf16 load)
+B200_HD float4 load4(const float* base, long long i4) { return ld_ro(reinterpret_cast<const float4*>(base) + i4); }
+B200_HD float4 load4(const bf16* base, long long i4) {
+#if defined(__CUDA_ARCH__)
+    const uint2 w = __ldg(reinterpret_cast<const uint2*>(base) + i4);
+    return make_float4(__uint_as_float(w.x << 16), __uint_as_float(w.x & 0xffff0000u), __uint_as_float(w.y << 16),
+                       __uint_as_float(w.y & 0xffff0000u));
+#else
+    return make_float4(to_float(base[4 * i4]), to_float(base[4 * i4 + 1]), to_float(base[4 * i4 + 2]), to_float(base[4 * i4 + 3]));
 #endif
 }
 

@@ -38,13 +38,16 @@ struct Tile {
 //      init_max/init_count (tile 0 of channel 0) reset the per-image max / tie counters for the
 //      kernels that follow in the stream.
 // ---------------------------------------------------------------------------------------------
-struct RowsR2CParams {
-    const float* x;          // [planes][N][N]
+// `In`: element type of x - fp32, or bf16 (an upstream gradient handed over in bf16; widened exactly in registers)
+template <class In>
+struct RowsR2CParamsT {
+    const In* x;             // [planes][N][N]
     float2* st;              // [planes][NC][N]
     const float2* tw;
     float* init_max;         // nullable, [planes/3]
     int* init_count;         // nullable, [planes/3]
 };
+using RowsR2CParams = RowsR2CParamsT<float>;
 
 // Shared memory of the row passes: one block of PA float2 per row pair, used first as the exchange array E of the
 // two-pass FFT and then, IN PLACE, as the natural-order line F of the same pair (only the 16/32 lanes of the pair touch
@@ -68,8 +71,8 @@ struct RowState {
     float2 v[Plan<N>::R2];
 };
 
-template <int N, class Exec>
-B200_HD void rows_r2c_body(Exec& ex, const RowsR2CParams& p, float2* smem) {
+template <int N, class Exec, class In>
+B200_HD void rows_r2c_body(Exec& ex, const RowsR2CParamsT<In>& p, float2* smem) {
     using P = Plan<N>;
     using T = Tile<N>;
     using S = RowsR2CSmem<N>;
@@ -80,11 +83,11 @@ B200_HD void rows_r2c_body(Exec& ex, const RowsR2CParams& p, float2* smem) {
     ex.warp_phase([&](int tid) {
         const int j = tid / P::LANES, a = tid % P::LANES;
         if (a < P::R2) {
-            const float* r0 = p.x + (static_cast<size_t>(plane) * N + y0 + 2 * j) * N;
-            const float* r1 = r0 + N;
+            const In* r0 = p.x + (static_cast<size_t>(plane) * N + y0 + 2 * j) * N;
+            const In* r1 = r0 + N;
             float2 v[P::R1];
 #pragma unroll
-            for (int i = 0; i < P::R1; ++i) v[i] = make_float2(ld_ro(r0 + P::R2 * i + a), ld_ro(r1 + P::R2 * i + a));
+            for (int i = 0; i < P::R1; ++i) v[i] = make_float2(load_elem(r0 + P::R2 * i + a), load_elem(r1 + P::R2 * i + a));
             P::stepA(v, a, smem + j * S::PA, p.tw);
         }
         if (tid == 0 && tile == 0 && plane % 3 == 0) {
@@ -125,33 +128,37 @@ B200_HD void rows_r2c_body(Exec& ex, const RowsR2CParams& p, float2* smem) {
 //      was fetched by two different instructions), the loads are asynchronous, and - the kernel being persistent - the
 //      lane's twiddles stay in registers.  grid = any (the launch picks the resident CTAs per SM), block NP*LANES.
 // ---------------------------------------------------------------------------------------------
-template <int N>
+template <int N, class In = float>
 struct RowsStreamSmem {
     using R = RowsR2CSmem<N>;
     using T = Tile<N>;
     // Each image row is copied by its own bulk copy into a staging row of pitch N + 8 floats: the two row pairs that
     // share a warp then read from banks 16 apart (with contiguous rows, 2N floats = 0 mod 32 banks put them on the SAME
     // banks: ncu showed a quarter of this kernel's shared-memory wavefronts to be such conflicts).
-    static constexpr int ROW_PITCH = N + 8;                                   // floats; 4*ROW_PITCH is a multiple of 16 bytes
-    static constexpr int TILE_FLOATS = T::ROWS * ROW_PITCH;
-    static constexpr int TILE_BYTES = T::ROWS * N * 4;                        // bytes that arrive per tile
+    // bf16 rows (In = bf16): pitch N + 8 elements as well, i.e. 16 padding bytes.  Two lanes read the two halves of one
+    // 4-byte word (a broadcast, not a conflict), so a row pair's R2 lanes touch R2/2 consecutive banks, and the rows of the
+    // pairs that share a warp are 2 * (N + 8) / 2 = N + 8 words = 8 banks apart: the 2 (N = 128, 256) or 4 (N = 64) pairs of a
+    // warp read disjoint banks.  The pitch stays a multiple of 16 bytes, as the bulk copies need.
+    static constexpr int ROW_PITCH = N + 8;                                   // elements; ROW_PITCH * sizeof(In) is a multiple of 16 bytes
+    static constexpr int TILE_ELEMS = T::ROWS * ROW_PITCH;
+    static constexpr int TILE_BYTES = T::ROWS * N * static_cast<int>(sizeof(In));   // bytes that arrive per tile
     static constexpr int STAGE_OFF = (R::RED_OFF + 15) / 16 * 16;            // float2 units, 128-byte aligned
-    static constexpr int BAR_OFF = STAGE_OFF + TILE_FLOATS;                   // two tiles of floats = TILE_FLOATS float2
+    static constexpr int BAR_OFF = STAGE_OFF + (2 * TILE_ELEMS * static_cast<int>(sizeof(In)) + 7) / 8;   // two tiles, in float2 units
     static constexpr int FLOAT2S = BAR_OFF + 2;                               // two 8-byte mbarriers
     static constexpr int BYTES = FLOAT2S * 8;
     static constexpr int THREADS = R::THREADS;
     static_assert(T::ROWS <= R::THREADS, "one issuing thread per row");
 };
 
-template <int N, class Exec>
-B200_HD void rows_r2c_stream_body(Exec& ex, const RowsR2CParams& p, float2* smem, int total_tiles, int nctas) {
+template <int N, class Exec, class In>
+B200_HD void rows_r2c_stream_body(Exec& ex, const RowsR2CParamsT<In>& p, float2* smem, int total_tiles, int nctas) {
     using P = Plan<N>;
     using T = Tile<N>;
     using S = RowsR2CSmem<N>;
-    using Q = RowsStreamSmem<N>;
+    using Q = RowsStreamSmem<N, In>;
     constexpr int TILES = N / T::ROWS;
     constexpr bool RT = P::REG_TW;
-    float* stage = reinterpret_cast<float*>(smem + Q::STAGE_OFF);
+    In* stage = reinterpret_cast<In*>(smem + Q::STAGE_OFF);
     unsigned long long* bars = reinterpret_cast<unsigned long long*>(smem + Q::BAR_OFF);
     RowState<N> st[Exec::IS_HOST ? S::THREADS : 1];
     float2 wreg[RT ? P::R1 : 1];
@@ -160,8 +167,8 @@ B200_HD void rows_r2c_stream_body(Exec& ex, const RowsR2CParams& p, float2* smem
     auto issue = [&](int tid, int t, int buf) {
         if (tid == 0) ex.bulk_expect(bars + buf, Q::TILE_BYTES);
         if (tid < T::ROWS)
-            ex.bulk_load(stage + buf * Q::TILE_FLOATS + tid * Q::ROW_PITCH, p.x + (static_cast<size_t>(t) * T::ROWS + tid) * N, N * 4,
-                         bars + buf);
+            ex.bulk_load(stage + buf * Q::TILE_ELEMS + tid * Q::ROW_PITCH, p.x + (static_cast<size_t>(t) * T::ROWS + tid) * N,
+                         N * static_cast<unsigned>(sizeof(In)), bars + buf);
     };
 
     ex.phase([&](int tid) {
@@ -186,11 +193,11 @@ B200_HD void rows_r2c_stream_body(Exec& ex, const RowsR2CParams& p, float2* smem
             ex.bulk_wait(bars + buf, (it >> 1) & 1);
             const int j = tid / P::LANES, a = tid % P::LANES;
             if (a < P::R2) {
-                const float* r0 = stage + buf * Q::TILE_FLOATS + (2 * j) * Q::ROW_PITCH;
-                const float* r1 = r0 + Q::ROW_PITCH;
+                const In* r0 = stage + buf * Q::TILE_ELEMS + (2 * j) * Q::ROW_PITCH;
+                const In* r1 = r0 + Q::ROW_PITCH;
                 float2 v[P::R1];
 #pragma unroll
-                for (int i = 0; i < P::R1; ++i) v[i] = make_float2(r0[P::R2 * i + a], r1[P::R2 * i + a]);
+                for (int i = 0; i < P::R1; ++i) v[i] = make_float2(to_float(r0[P::R2 * i + a]), to_float(r1[P::R2 * i + a]));
                 if constexpr (RT) {
                     if constexpr (Exec::IS_HOST) P::load_tw(wreg, p.tw, a);
                     P::stepA(v, a, smem + j * S::PA, wreg);
@@ -837,8 +844,11 @@ struct NormaliseParams {
 // y = conv * (1/max) instead of a division per element; the arg-max element itself is written as exactly 1.
 // A CTA works on a slice of ONE image at a time (unit = image x slice): the maximum is loaded once per unit and no
 // per-element index division is left (the flat-index version spent ~120 instructions per float4, 11.6 M warp instructions).
-template <class Exec>
-B200_HD void normalise_body(Exec& ex, const NormaliseParams& p, int grid_x) {
+// Out = float: in place, p.y holds conv on entry and the sensor image on exit.  Out = bf16: p.y (the fp32 conv) is only
+// read and the sensor image goes to `out`, each value the fp32 result rounded to nearest-even as the very last step (after
+// the tie recording and the epilogue), i.e. exactly the fp32 image cast with torch.
+template <class Out = float, class Exec>
+B200_HD void normalise_body(Exec& ex, const NormaliseParams& p, int grid_x, Out* out = nullptr) {
     ex.phase([&](int tid) {
         constexpr int U = 4;
         const int B = static_cast<int>(p.n4 / p.per_image4);
@@ -872,7 +882,10 @@ B200_HD void normalise_body(Exec& ex, const NormaliseParams& p, int grid_x) {
                         }
                         e[q] = apply_epilogue(p.epi, e[q], (static_cast<size_t>(b) * p.per_image4 + i) * 4 + q);
                     }
-                    img4[i] = make_float4(e[0], e[1], e[2], e[3]);
+                    if constexpr (sizeof(Out) == sizeof(float))
+                        img4[i] = make_float4(e[0], e[1], e[2], e[3]);
+                    else
+                        store4(out, static_cast<long long>(b) * p.per_image4 + i, e[0], e[1], e[2], e[3]);
                 }
             }
         }

@@ -17,6 +17,8 @@
 // (kernels.cuh); n in {128, 256, 512, 1024}.
 #include <cuda_runtime.h>
 
+#include <type_traits>
+
 #include "../../include/b200cam.h"
 #include "kernels.cuh"
 
@@ -45,8 +47,9 @@ struct ImgLoadU8 {      // a uint8 image: a quarter of the bytes; = torch's u8.f
         return __fmul_rn(static_cast<float>(__ldg(x + (static_cast<size_t>(plane) * P + r) * P + c)), 1.0f / 255.0f);
     }
 };
-struct GradLoad {       // dL/dconv from dL/dy: adjoint of / max, |.|, crop and nearest resize (Utils.py:289-295, Lens.py:312)
-    const float* g;     // [planes][P][P] dL/dy
+template <class G>      // G: element type of dL/dy - fp32, or bf16 (widened exactly in registers)
+struct GradLoadT {      // dL/dconv from dL/dy: adjoint of / max, |.|, crop and nearest resize (Utils.py:289-295, Lens.py:312)
+    const G* g;         // [planes][P][P] dL/dy
     const float* raw;   // [planes][P][P] signed un-normalised sensor image of the forward
     const float* gmax;  // device scalar: batch maximum m (all ranks)
     const float* coef;  // device scalar: s / (m n), s = sum(g y), n = number of positions that attain m
@@ -57,7 +60,7 @@ struct GradLoad {       // dL/dconv from dL/dy: adjoint of / max, |.|, crop and 
         cf = __ldg(coef);
     }
     __device__ __forceinline__ float draw(size_t o) const {
-        const float rv = __ldg(raw + o), gv = __ldg(g + o);
+        const float rv = __ldg(raw + o), gv = load_elem(g + o);
         const float d = gv * inv_m - (fabsf(rv) == m ? cf : 0.f);
         return rv > 0.f ? d : (rv < 0.f ? -d : 0.f);
     }
@@ -77,10 +80,14 @@ struct GradLoad {       // dL/dconv from dL/dy: adjoint of / max, |.|, crop and 
         return v;
     }
 };
+using GradLoad = GradLoadT<float>;
 
 // ---- KA: zero-padded real rows -> transposed half spectrum, live rows only.  grid (P / ROWS, planes), block NP * LANES ------
-template <int N, class Load>
-__global__ void __launch_bounds__(RowsR2CSmem<N>::THREADS) k_lrows_r2c(Load load, float2* __restrict__ st, const float2* __restrict__ tw) {
+// MIN_CTAS > 0: held to that many resident CTAs per SM (__launch_bounds__ minimum; 0 emits no bound).  Used for the bf16
+// gradient loader at n = 512, which otherwise costs ptxas 4 registers more than the fp32 one (84 vs 80: 2 instead of 3 CTAs of
+// 256 threads per SM; measured 77 against 64 us per launch at B = 64, one B200).
+template <int N, class Load, int MIN_CTAS = 0>
+__global__ void __launch_bounds__(RowsR2CSmem<N>::THREADS, MIN_CTAS) k_lrows_r2c(Load load, float2* __restrict__ st, const float2* __restrict__ tw) {
     using P = Plan<N>;
     using T = Tile<N>;
     using S = RowsR2CSmem<N>;
@@ -325,9 +332,10 @@ __global__ void __launch_bounds__(ColsSmem<N>::THREADS, N <= 512 ? 2 : 1) k_lcol
 }
 
 // ---- element-wise: y = |raw| / m [-> read-out epilogue] ; partial sums of g * y and the number of positions that attain m -----
+// Out = bf16: the fp32 value rounded to nearest-even as the last step (= the fp32 sensor image cast with torch)
 constexpr int EWT = 256;
-template <bool EPI>
-__global__ void __launch_bounds__(EWT) k_lnormalise(const float4* __restrict__ raw, const float* __restrict__ gmax, float4* __restrict__ y, long long n4,
+template <bool EPI, class Out = float>
+__global__ void __launch_bounds__(EWT) k_lnormalise(const float4* __restrict__ raw, const float* __restrict__ gmax, Out* __restrict__ y, long long n4,
                                                     SensorEpilogue epi) {
     const float m = __ldg(gmax);
     for (long long i = blockIdx.x * static_cast<long long>(EWT) + threadIdx.x; i < n4; i += static_cast<long long>(gridDim.x) * EWT) {
@@ -338,11 +346,15 @@ __global__ void __launch_bounds__(EWT) k_lnormalise(const float4* __restrict__ r
             o = make_float4(apply_epilogue(epi, o.x, e), apply_epilogue(epi, o.y, e + 1), apply_epilogue(epi, o.z, e + 2),
                             apply_epilogue(epi, o.w, e + 3));
         }
-        y[i] = o;
+        if constexpr (sizeof(Out) == sizeof(float))
+            reinterpret_cast<float4*>(y)[i] = o;
+        else
+            store4(y, i, o.x, o.y, o.z, o.w);
     }
 }
 // part[block] = {sum g y, ties} in double / as a count; fixed order inside a block, blocks summed in order by k_ldot_final
-__global__ void __launch_bounds__(EWT) k_ldot(const float4* __restrict__ g, const float4* __restrict__ raw, const float* __restrict__ gmax, long long n4,
+template <class G = float>     // G: element type of dL/dy (fp32 / bf16)
+__global__ void __launch_bounds__(EWT) k_ldot(const G* __restrict__ g, const float4* __restrict__ raw, const float* __restrict__ gmax, long long n4,
                                               double* __restrict__ part) {
     __shared__ double rs[EWT / 32];
     __shared__ double rt[EWT / 32];
@@ -350,7 +362,7 @@ __global__ void __launch_bounds__(EWT) k_ldot(const float4* __restrict__ g, cons
     const float inv = 1.0f / m;
     double s = 0.0, t = 0.0;
     for (long long i = blockIdx.x * static_cast<long long>(EWT) + threadIdx.x; i < n4; i += static_cast<long long>(gridDim.x) * EWT) {
-        const float4 v = __ldg(raw + i), gg = __ldg(g + i);
+        const float4 v = __ldg(raw + i), gg = load4(g, i);
         const float ax = fabsf(v.x), ay = fabsf(v.y), az = fabsf(v.z), aw = fabsf(v.w);
         s += static_cast<double>(gg.x * (ax * inv)) + static_cast<double>(gg.y * (ay * inv)) + static_cast<double>(gg.z * (az * inv)) +
              static_cast<double>(gg.w * (aw * inv));
@@ -473,8 +485,8 @@ static int fwd_impl(Load load, const float* kern, float* raw, float* gmax, float
     return 0;
 }
 
-template <int N>
-static int bwd_impl(const float* g, const float* raw, const float* gmax, const float* coef, const float2* otf, const float2* spectrum,
+template <int N, class G = float>
+static int bwd_impl(const G* g, const float* raw, const float* gmax, const float* coef, const float2* otf, const float2* spectrum,
                     float* grad_kern, float* grad_img, void* wsp, int B, cudaStream_t s) {
     using T = Tile<N>;
     const float2* tw = lens_twiddle(N);
@@ -482,10 +494,11 @@ static int bwd_impl(const float* g, const float* raw, const float* gmax, const f
     Ws ws(wsp, N, B);
     const int planes = 3 * B, tiles = (N / 2) / T::ROWS;
     const int colgroups = (3 * T::NC + T::COLS - 1) / T::COLS, nch = lchunks(N, B);
-    LCK(optin(k_lrows_r2c<N, GradLoad>, RowsR2CSmem<N>::BYTES));
+    constexpr int MIN_CTAS = (N == 512 && !std::is_same<G, float>::value) ? 3 : 0;
+    auto rows = k_lrows_r2c<N, GradLoadT<G>, MIN_CTAS>;
+    LCK(optin(rows, RowsR2CSmem<N>::BYTES));
     LCK(optin(k_lcols_accum<N>, ColsSmem<N>::BYTES_CONV));
-    k_lrows_r2c<N, GradLoad><<<dim3(tiles, planes), RowsR2CSmem<N>::THREADS, RowsR2CSmem<N>::BYTES, s>>>(
-        GradLoad{g, raw, gmax, coef, 0.f, 0.f, 0.f}, ws.stg, tw);
+    rows<<<dim3(tiles, planes), RowsR2CSmem<N>::THREADS, RowsR2CSmem<N>::BYTES, s>>>(GradLoadT<G>{g, raw, gmax, coef, 0.f, 0.f, 0.f}, ws.stg, tw);
     LLAUNCH();
     k_lcols_accum<N><<<dim3(colgroups, nch), ColsSmem<N>::THREADS, ColsSmem<N>::BYTES_CONV, s>>>(spectrum, ws.stg, ws.partial, tw, B, nch);
     LLAUNCH();
@@ -531,6 +544,63 @@ static int lens_fwd(Load load, const void* img, const float* kernel, float* raw,
     }
 }
 
+// checks and launches of the element-wise / backward entry points; Out / G: fp32, or bf16 (the _bf16 entry points)
+template <class Out>
+static int lens_normalise(const float* raw, const float* gmax, Out* y, long long count, void* stream, int flags, const float* noise,
+                          float noise_scale, int quant_bits) {
+    SensorEpilogue epi;
+    if (const int rc = make_epilogue(flags, noise, noise_scale, quant_bits, &epi)) return rc;
+    if (!raw || !gmax || !y) return B200CAM_E_NULL;
+    if (count < 0 || count % 4 != 0) return B200CAM_E_BAD_SIZE;
+    if (!al16(raw) || !al16(y)) return B200CAM_E_ALIGN;
+    if (count == 0) return 0;
+    const auto r4 = reinterpret_cast<const float4*>(raw);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (flags)
+        k_lnormalise<true><<<ew_grid(count / 4), EWT, 0, s>>>(r4, gmax, y, count / 4, epi);
+    else
+        k_lnormalise<false><<<ew_grid(count / 4), EWT, 0, s>>>(r4, gmax, y, count / 4, epi);
+    LLAUNCH();
+    return 0;
+}
+
+template <class G>
+static int lens_dot(const G* grad_y, const float* raw, const float* gmax, float* dot_ties, void* workspace, size_t workspace_bytes, int B,
+                    int P, void* stream) {
+    if (!lens_n_ok(P) || B < 1) return B200CAM_E_BAD_SIZE;
+    if (!grad_y || !raw || !gmax || !dot_ties || !workspace) return B200CAM_E_NULL;
+    if (!al16(grad_y) || !al16(raw)) return B200CAM_E_ALIGN;
+    Ws ws(workspace, 2 * P, B);
+    if (workspace_bytes < ws.bytes) return B200CAM_E_WORKSPACE;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const long long n4 = static_cast<long long>(B) * 3 * P * P / 4;
+    const int grid = ew_grid(n4);
+    k_ldot<<<grid, EWT, 0, s>>>(grad_y, reinterpret_cast<const float4*>(raw), gmax, n4, ws.dpart);
+    LLAUNCH();
+    k_ldot_final<<<1, EWT, 0, s>>>(ws.dpart, grid, dot_ties);
+    LLAUNCH();
+    return 0;
+}
+
+template <class G>
+static int lens_bwd(const G* grad_y, const float* raw, const float* gmax, const float* coef, const float* otf, const float* spectrum,
+                    float* grad_kernel, float* grad_img, void* workspace, size_t workspace_bytes, int B, int P, void* stream) {
+    if (!lens_n_ok(P) || B < 1) return B200CAM_E_BAD_SIZE;
+    if (!grad_y || !raw || !gmax || !coef || !otf || !spectrum || !grad_kernel || !workspace) return B200CAM_E_NULL;
+    if (!al16(grad_y) || !al16(raw) || !al16(spectrum) || !al16(workspace)) return B200CAM_E_ALIGN;
+    const int N = 2 * P;
+    if (workspace_bytes < Ws(nullptr, N, B).bytes) return B200CAM_E_WORKSPACE;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const float2* o = reinterpret_cast<const float2*>(otf);
+    const float2* sp = reinterpret_cast<const float2*>(spectrum);
+    switch (N) {
+        case 128: return bwd_impl<128>(grad_y, raw, gmax, coef, o, sp, grad_kernel, grad_img, workspace, B, s);
+        case 256: return bwd_impl<256>(grad_y, raw, gmax, coef, o, sp, grad_kernel, grad_img, workspace, B, s);
+        case 512: return bwd_impl<512>(grad_y, raw, gmax, coef, o, sp, grad_kernel, grad_img, workspace, B, s);
+        default: return bwd_impl<1024>(grad_y, raw, gmax, coef, o, sp, grad_kernel, grad_img, workspace, B, s);
+    }
+}
+
 extern "C" {
 
 size_t b200cam_lens_sensor_workspace_bytes(int P, int B) {
@@ -554,56 +624,34 @@ int b200cam_lens_normalise(const float* raw, const float* gmax, float* y, long l
 
 int b200cam_lens_normalise_ex(const float* raw, const float* gmax, float* y, long long count, void* stream, int flags, const float* noise,
                               float noise_scale, int quant_bits) {
-    SensorEpilogue epi;
-    if (const int rc = make_epilogue(flags, noise, noise_scale, quant_bits, &epi)) return rc;
-    if (!raw || !gmax || !y) return B200CAM_E_NULL;
-    if (count < 0 || count % 4 != 0) return B200CAM_E_BAD_SIZE;
-    if (!al16(raw) || !al16(y)) return B200CAM_E_ALIGN;
-    if (count == 0) return 0;
-    const auto r4 = reinterpret_cast<const float4*>(raw);
-    const auto y4 = reinterpret_cast<float4*>(y);
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    if (flags)
-        k_lnormalise<true><<<ew_grid(count / 4), EWT, 0, s>>>(r4, gmax, y4, count / 4, epi);
-    else
-        k_lnormalise<false><<<ew_grid(count / 4), EWT, 0, s>>>(r4, gmax, y4, count / 4, epi);
-    LLAUNCH();
-    return 0;
+    return lens_normalise(raw, gmax, y, count, stream, flags, noise, noise_scale, quant_bits);
+}
+
+int b200cam_lens_normalise_bf16(const float* raw, const float* gmax, unsigned short* y, long long count, void* stream, int flags,
+                                const float* noise, float noise_scale, int quant_bits) {
+    return lens_normalise(raw, gmax, reinterpret_cast<bf16*>(y), count, stream, flags, noise, noise_scale, quant_bits);
 }
 
 int b200cam_lens_sensor_dot(const float* grad_y, const float* raw, const float* gmax, float* dot_ties, void* workspace, size_t workspace_bytes,
                             int B, int P, void* stream) {
-    if (!lens_n_ok(P) || B < 1) return B200CAM_E_BAD_SIZE;
-    if (!grad_y || !raw || !gmax || !dot_ties || !workspace) return B200CAM_E_NULL;
-    if (!al16(grad_y) || !al16(raw)) return B200CAM_E_ALIGN;
-    Ws ws(workspace, 2 * P, B);
-    if (workspace_bytes < ws.bytes) return B200CAM_E_WORKSPACE;
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    const long long n4 = static_cast<long long>(B) * 3 * P * P / 4;
-    const int grid = ew_grid(n4);
-    k_ldot<<<grid, EWT, 0, s>>>(reinterpret_cast<const float4*>(grad_y), reinterpret_cast<const float4*>(raw), gmax, n4, ws.dpart);
-    LLAUNCH();
-    k_ldot_final<<<1, EWT, 0, s>>>(ws.dpart, grid, dot_ties);
-    LLAUNCH();
-    return 0;
+    return lens_dot(grad_y, raw, gmax, dot_ties, workspace, workspace_bytes, B, P, stream);
+}
+
+int b200cam_lens_sensor_dot_bf16(const unsigned short* grad_y, const float* raw, const float* gmax, float* dot_ties, void* workspace,
+                                 size_t workspace_bytes, int B, int P, void* stream) {
+    return lens_dot(reinterpret_cast<const bf16*>(grad_y), raw, gmax, dot_ties, workspace, workspace_bytes, B, P, stream);
 }
 
 int b200cam_lens_sensor_bwd(const float* grad_y, const float* raw, const float* gmax, const float* coef, const float* otf, const float* spectrum,
                             float* grad_kernel, float* grad_img, void* workspace, size_t workspace_bytes, int B, int P, void* stream) {
-    if (!lens_n_ok(P) || B < 1) return B200CAM_E_BAD_SIZE;
-    if (!grad_y || !raw || !gmax || !coef || !otf || !spectrum || !grad_kernel || !workspace) return B200CAM_E_NULL;
-    if (!al16(grad_y) || !al16(raw) || !al16(spectrum) || !al16(workspace)) return B200CAM_E_ALIGN;
-    const int N = 2 * P;
-    if (workspace_bytes < Ws(nullptr, N, B).bytes) return B200CAM_E_WORKSPACE;
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    const float2* o = reinterpret_cast<const float2*>(otf);
-    const float2* sp = reinterpret_cast<const float2*>(spectrum);
-    switch (N) {
-        case 128: return bwd_impl<128>(grad_y, raw, gmax, coef, o, sp, grad_kernel, grad_img, workspace, B, s);
-        case 256: return bwd_impl<256>(grad_y, raw, gmax, coef, o, sp, grad_kernel, grad_img, workspace, B, s);
-        case 512: return bwd_impl<512>(grad_y, raw, gmax, coef, o, sp, grad_kernel, grad_img, workspace, B, s);
-        default: return bwd_impl<1024>(grad_y, raw, gmax, coef, o, sp, grad_kernel, grad_img, workspace, B, s);
-    }
+    return lens_bwd(grad_y, raw, gmax, coef, otf, spectrum, grad_kernel, grad_img, workspace, workspace_bytes, B, P, stream);
+}
+
+int b200cam_lens_sensor_bwd_bf16(const unsigned short* grad_y, const float* raw, const float* gmax, const float* coef, const float* otf,
+                                 const float* spectrum, float* grad_kernel, float* grad_img, void* workspace, size_t workspace_bytes, int B,
+                                 int P, void* stream) {
+    return lens_bwd(reinterpret_cast<const bf16*>(grad_y), raw, gmax, coef, otf, spectrum, grad_kernel, grad_img, workspace,
+                    workspace_bytes, B, P, stream);
 }
 
 }  // extern "C"

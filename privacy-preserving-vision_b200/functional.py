@@ -140,6 +140,9 @@ def nvtx(name):
 # 1: the caller's image row pass is ordered behind the first PSF kernel (see b200cam_psf_field); B200CAM_HOLD_ROWS=0 lets
 # both start together (A/B switch)
 _HOLD_ROWS = 0 if os.environ.get("B200CAM_HOLD_ROWS", "1") == "0" else 1
+# B200CAM_PLANE=1 (opt-in N = 256 plane kernels, read once per process by the library): b200cam_sensor_rows then writes the
+# plane layout, which the bf16 sensor path (default two-pass pipeline only) cannot read
+PLANE_KERNELS = os.environ.get("B200CAM_PLANE", "0")[:1] == "1"
 
 
 def _stream() -> ctypes.c_void_p:
@@ -285,6 +288,16 @@ def read_out(img: torch.Tensor, sigma: float, bits: int, noise: torch.Tensor | N
     return (noise, sigma if noise is not None else 0.0, bits)
 
 
+SENSOR_DTYPES = (torch.float32, torch.bfloat16)
+
+
+def check_sensor_dtype(dtype) -> torch.dtype:
+    """The ``sensor_dtype`` module attribute of both cameras: torch.float32 (default) or torch.bfloat16."""
+    if dtype not in SENSOR_DTYPES:
+        raise ValueError(f"sensor_dtype must be torch.float32 or torch.bfloat16, got {dtype!r}")
+    return dtype
+
+
 def _check_img(img: torch.Tensor, N: int) -> None:
     if img.dim() != 4 or img.shape[1] != 3 or img.shape[2] != N or img.shape[3] != N:
         raise ValueError(f"expected img of shape (B,3,{N},{N}), got {tuple(img.shape)}")
@@ -320,9 +333,13 @@ def sensor_rows(img: torch.Tensor, plan: DevicePlan):
 class SensorConv(torch.autograd.Function):
     @staticmethod
     @nvtx("b200cam.SensorConv.forward")
-    def forward(ctx, img: torch.Tensor, psf: torch.Tensor, plan: DevicePlan, rows: RowSpectra | None = None, epilogue=None):
+    def forward(ctx, img: torch.Tensor, psf: torch.Tensor, plan: DevicePlan, rows: RowSpectra | None = None, epilogue=None,
+                out_dtype: torch.dtype = torch.float32):
         """`epilogue`: None (the reference's read-out: nothing) or (noise, noise_scale, quant_bits) - the opt-in sensor
-        noise + quantisation of include/b200cam.h (B200CAM_SENSOR_NOISE / _QUANT); straight-through in backward."""
+        noise + quantisation of include/b200cam.h (B200CAM_SENSOR_NOISE / _QUANT); straight-through in backward.
+        `out_dtype` torch.bfloat16: the sensor image is written in bf16 (the fp32 result rounded to nearest-even, i.e.
+        exactly ``fp32_result.to(torch.bfloat16)``) and the bf16 upstream gradient is read by the kernels as it is; the
+        un-normalised fp32 image is a scratch buffer of the forward and is not kept."""
         N = plan.N
         flags, noise_t, noise_scale, quant_bits = 0, None, 0.0, 0
         if epilogue is not None:
@@ -338,7 +355,10 @@ class SensorConv(torch.autograd.Function):
         x = rows.x if rows is not None else _as_f32(img.detach(), plan.device)
         p = _as_f32(psf.detach(), plan.device).reshape(3, N, N)
         B = x.shape[0]
+        bf16 = out_dtype == torch.bfloat16
+        # bf16: `sensor` is the fp32 conv scratch (dropped after the forward), `out` the bf16 image handed downstream
         sensor = torch.empty_like(x)
+        out = torch.empty(x.shape, dtype=torch.bfloat16, device=x.device) if bf16 else sensor
         img_max = rows.img_max if rows is not None else torch.empty(B, dtype=torch.float32, device=plan.device)
         tie_count = rows.tie_count if rows is not None else torch.empty(B, dtype=torch.int32, device=plan.device)
         tie_pos = torch.empty(B, 8, dtype=torch.int32, device=plan.device)
@@ -355,24 +375,39 @@ class SensorConv(torch.autograd.Function):
                 otf = cached[1]
             plan.otf_cache = None
             with torch.cuda.device(plan.index):
-                _lib.check(plan.lib.b200cam_sensor_finish_ex(
-                    _lib.ptr(p), _lib.ptr(sensor), _lib.ptr(img_max), _lib.ptr(tie_count), _lib.ptr(tie_pos),
-                    _lib.ptr(otf), _lib.ptr(spectrum), otf_ready, _lib.ptr(ws), ws.numel(), B, N, _stream(),
-                    flags, _lib.ptr(noise_t), float(noise_scale), int(quant_bits)))
+                if bf16:
+                    _lib.check(plan.lib.b200cam_sensor_finish_bf16(
+                        _lib.ptr(p), _lib.ptr(sensor), _lib.ptr(out), _lib.ptr(img_max), _lib.ptr(tie_count), _lib.ptr(tie_pos),
+                        _lib.ptr(otf), _lib.ptr(spectrum), otf_ready, _lib.ptr(ws), ws.numel(), B, N, _stream(),
+                        flags, _lib.ptr(noise_t), float(noise_scale), int(quant_bits)))
+                else:
+                    _lib.check(plan.lib.b200cam_sensor_finish_ex(
+                        _lib.ptr(p), _lib.ptr(sensor), _lib.ptr(img_max), _lib.ptr(tie_count), _lib.ptr(tie_pos),
+                        _lib.ptr(otf), _lib.ptr(spectrum), otf_ready, _lib.ptr(ws), ws.numel(), B, N, _stream(),
+                        flags, _lib.ptr(noise_t), float(noise_scale), int(quant_bits)))
             if not any(ctx.needs_input_grad[:2]):
                 spectrum = None
         elif B > 0:
             ws = plan.sensor_workspace(B)
             with torch.cuda.device(plan.index):
-                _lib.check(plan.lib.b200cam_sensor_fwd_ex(
-                    _lib.ptr(x), _lib.ptr(p), _lib.ptr(sensor), _lib.ptr(img_max), _lib.ptr(tie_count),
-                    _lib.ptr(tie_pos), _lib.ptr(otf), _lib.ptr(spectrum), _lib.ptr(ws), ws.numel(), B, N, _stream(),
-                    flags, _lib.ptr(noise_t), float(noise_scale), int(quant_bits)))
+                if bf16:
+                    _lib.check(plan.lib.b200cam_sensor_fwd_bf16(
+                        _lib.ptr(x), _lib.ptr(p), _lib.ptr(sensor), _lib.ptr(out), _lib.ptr(img_max), _lib.ptr(tie_count),
+                        _lib.ptr(tie_pos), _lib.ptr(otf), _lib.ptr(spectrum), _lib.ptr(ws), ws.numel(), B, N, _stream(),
+                        flags, _lib.ptr(noise_t), float(noise_scale), int(quant_bits)))
+                else:
+                    _lib.check(plan.lib.b200cam_sensor_fwd_ex(
+                        _lib.ptr(x), _lib.ptr(p), _lib.ptr(sensor), _lib.ptr(img_max), _lib.ptr(tie_count),
+                        _lib.ptr(tie_pos), _lib.ptr(otf), _lib.ptr(spectrum), _lib.ptr(ws), ws.numel(), B, N, _stream(),
+                        flags, _lib.ptr(noise_t), float(noise_scale), int(quant_bits)))
+        elif bf16:
+            out = sensor.to(torch.bfloat16)           # empty batch: nothing for the kernels to do
         ctx.plan = plan
         ctx.psf_shape = psf.shape
         ctx.spectrum = spectrum
-        ctx.save_for_backward(x, p, sensor, img_max, tie_count, tie_pos, otf)
-        return sensor
+        # the bf16 node keeps no image-sized fp32 sensor tensor (no backward kernel reads it)
+        ctx.save_for_backward(x, p, None if bf16 else sensor, img_max, tie_count, tie_pos, otf)
+        return out
 
     @staticmethod
     @nvtx("b200cam.SensorConv.backward")
@@ -385,7 +420,17 @@ class SensorConv(torch.autograd.Function):
         # the kernels overwrite every element of grad_psf; only the empty batch needs explicit zeros
         grad_psf = (torch.empty if B > 0 else torch.zeros)(3, N, N, dtype=torch.float32, device=plan.device)
         grad_img = torch.empty_like(x) if want_img else None
-        if B > 0:
+        if B > 0 and g.dtype == torch.bfloat16:
+            if g.device != plan.device:
+                raise RuntimeError(f"b200cam: tensor on {g.device}, camera tables on {plan.device}")
+            gc = g.contiguous()
+            ws = plan.sensor_workspace(B)
+            with torch.cuda.device(plan.index):
+                _lib.check(plan.lib.b200cam_sensor_bwd_bf16(
+                    _lib.ptr(gc), _lib.ptr(x), _lib.ptr(img_max), _lib.ptr(tie_count), _lib.ptr(tie_pos), _lib.ptr(p),
+                    _lib.ptr(otf), _lib.ptr(ctx.spectrum), _lib.ptr(grad_psf), _lib.ptr(grad_img),
+                    _lib.ptr(ws), ws.numel(), B, N, _stream()))
+        elif B > 0:
             gc = _as_f32(g, plan.device)
             ws = plan.sensor_workspace(B)
             with torch.cuda.device(plan.index):
@@ -394,7 +439,7 @@ class SensorConv(torch.autograd.Function):
                     _lib.ptr(tie_pos), _lib.ptr(p), _lib.ptr(otf), _lib.ptr(ctx.spectrum), _lib.ptr(grad_psf),
                     _lib.ptr(grad_img),
                     _lib.ptr(ws), ws.numel(), B, N, _stream()))
-        return grad_img, grad_psf.reshape(ctx.psf_shape), None, None, None
+        return grad_img, grad_psf.reshape(ctx.psf_shape), None, None, None, None
 
 
 def psf_synth(h: torch.Tensor, plan: DevicePlan, stream: torch.cuda.Stream | None = None):
@@ -402,5 +447,5 @@ def psf_synth(h: torch.Tensor, plan: DevicePlan, stream: torch.cuda.Stream | Non
 
 
 def sensor_conv(img: torch.Tensor, psf: torch.Tensor, plan: DevicePlan, rows: RowSpectra | None = None,
-                epilogue=None) -> torch.Tensor:
-    return SensorConv.apply(img, psf, plan, rows, epilogue)
+                epilogue=None, out_dtype: torch.dtype = torch.float32) -> torch.Tensor:
+    return SensorConv.apply(img, psf, plan, rows, epilogue, out_dtype)

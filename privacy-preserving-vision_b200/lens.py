@@ -27,7 +27,11 @@ Read-out (no reference counterpart, same meaning as on the Face-DeId ``Camera``)
   y = round(clamp(y, 0, 1) * L) / L, L = 2^bits - 1, applied after the batch-global max by the normalise kernel
   (``b200cam_lens_normalise_ex``; the torch expression elsewhere), straight through in backward.  ``forward(..., noise=)``
   takes the standard-normal tensor; otherwise it is drawn with ``torch.randn`` after the lens tolerance field.  With
-  ``data_parallel`` each rank draws the noise of its own shard.
+  ``data_parallel`` each rank draws the noise of its own shard;
+* ``sensor_dtype`` (default torch.float32): torch.bfloat16 returns the sensor image in bf16 for a bf16 encoder - the normalise
+  kernel rounds the fp32 result to nearest-even (``b200cam_lens_normalise_bf16``) and the backward reads the bf16 gradient as it
+  is (``_dot_bf16`` / ``_bwd_bf16``); the other geometries cast with torch.  Bit for bit the fp32 module followed by
+  ``.to(torch.bfloat16)``.
 
 Not reproduced: comet.ml summaries (``attach_summaries``), the ``psf_lab`` image file path, ``upsample=True``
 (1792^2 convolution, not a power of two) - they raise ``NotImplementedError`` - and the side effect of caching the
@@ -184,11 +188,14 @@ class LensSensor(torch.autograd.Function):
     group the maximum is all-reduced (MAX) and, in the backward, sum(g*y) and the tie count (SUM): N ranks reproduce the
     one-GPU result, the arg-max term landing on the rank(s) that hold the maximum.
     ``img`` may be fp32 or uint8 (read by the row kernel as img / 255.0).  ``epilogue``: None or (noise, noise_scale,
-    quant_bits) of ``F.read_out``, applied by the normalise kernel after the maximum; straight through in backward."""
+    quant_bits) of ``F.read_out``, applied by the normalise kernel after the maximum; straight through in backward.
+    ``out_dtype`` torch.bfloat16: the normalise kernel writes y in bf16 (its fp32 value rounded to nearest-even) and the bf16
+    gradient is read by the dot and row kernels as it is - the fp32 backward on g.float(), bit for bit."""
 
     @staticmethod
     @F.nvtx("b200cam.LensSensor.forward")
-    def forward(ctx, img: torch.Tensor, kpad: torch.Tensor, plan: F.DevicePlan, group, epilogue=None):
+    def forward(ctx, img: torch.Tensor, kpad: torch.Tensor, plan: F.DevicePlan, group, epilogue=None,
+                out_dtype: torch.dtype = torch.float32):
         import torch.distributed as dist
         dev, n = plan.device, plan.N
         P = n // 2
@@ -212,7 +219,8 @@ class LensSensor(torch.autograd.Function):
             if quant_bits:
                 flags |= 2
         raw = torch.empty(x.shape, dtype=torch.float32, device=dev)
-        y = torch.empty_like(raw)
+        bf16 = out_dtype == torch.bfloat16
+        y = torch.empty(x.shape, dtype=out_dtype, device=dev)
         gmax = torch.zeros(1, dtype=torch.float32, device=dev)
         otf = torch.empty(plan.otf_floats, dtype=torch.float32, device=dev)
         spectrum = torch.empty(lib.b200cam_spectrum_bytes(n, B) // 4, dtype=torch.float32, device=dev)
@@ -222,8 +230,9 @@ class LensSensor(torch.autograd.Function):
                            ws.numel(), B, P, F._stream()))
             if group is not None and dist.is_initialized():
                 dist.all_reduce(gmax, op=dist.ReduceOp.MAX, group=group)
-            _lib.check(lib.b200cam_lens_normalise_ex(_lib.ptr(raw), _lib.ptr(gmax), _lib.ptr(y), raw.numel(), F._stream(), flags,
-                                                     _lib.ptr(noise), float(noise_scale), int(quant_bits)))
+            normalise = lib.b200cam_lens_normalise_bf16 if bf16 else lib.b200cam_lens_normalise_ex
+            _lib.check(normalise(_lib.ptr(raw), _lib.ptr(gmax), _lib.ptr(y), raw.numel(), F._stream(), flags,
+                                 _lib.ptr(noise), float(noise_scale), int(quant_bits)))
         ctx.plan, ctx.group, ctx.kshape = plan, group, kpad.shape
         ctx.spectrum = spectrum if any(ctx.needs_input_grad[:2]) else None
         ctx.save_for_backward(raw, gmax, otf)
@@ -238,21 +247,26 @@ class LensSensor(torch.autograd.Function):
         dev, n = plan.device, plan.N
         P, B = n // 2, raw.shape[0]
         lib = plan.lib
-        gy = F._as_f32(g, dev)
+        if g.dtype == torch.bfloat16:         # bf16 sensor image: the kernels widen the gradient themselves
+            if g.device != dev:
+                raise RuntimeError(f"b200cam: tensor on {g.device}, camera tables on {dev}")
+            gy, sdot, sbwd = g.contiguous(), lib.b200cam_lens_sensor_dot_bf16, lib.b200cam_lens_sensor_bwd_bf16
+        else:
+            gy, sdot, sbwd = F._as_f32(g, dev), lib.b200cam_lens_sensor_dot, lib.b200cam_lens_sensor_bwd
         dot = torch.empty(2, dtype=torch.float32, device=dev)
         grad_k = torch.empty(3, n, n, dtype=torch.float32, device=dev)
         grad_img = torch.empty_like(raw) if ctx.needs_input_grad[0] else None
         ws = torch.empty(lib.b200cam_lens_sensor_workspace_bytes(P, B), dtype=torch.uint8, device=dev)
         with torch.cuda.device(plan.index):
-            _lib.check(lib.b200cam_lens_sensor_dot(_lib.ptr(gy), _lib.ptr(raw), _lib.ptr(gmax), _lib.ptr(dot), _lib.ptr(ws), ws.numel(),
+            _lib.check(sdot(_lib.ptr(gy), _lib.ptr(raw), _lib.ptr(gmax), _lib.ptr(dot), _lib.ptr(ws), ws.numel(),
                                                    B, P, F._stream()))
             if ctx.group is not None and dist.is_initialized():
                 dist.all_reduce(dot, op=dist.ReduceOp.SUM, group=ctx.group)
             coef = (dot[0] / (gmax[0] * dot[1].clamp(min=1.0))).reshape(1)      # s / (m n); torch.max splits exact ties evenly
-            _lib.check(lib.b200cam_lens_sensor_bwd(_lib.ptr(gy), _lib.ptr(raw), _lib.ptr(gmax), _lib.ptr(coef), _lib.ptr(otf),
+            _lib.check(sbwd(_lib.ptr(gy), _lib.ptr(raw), _lib.ptr(gmax), _lib.ptr(coef), _lib.ptr(otf),
                                                    _lib.ptr(ctx.spectrum), _lib.ptr(grad_k), _lib.ptr(grad_img), _lib.ptr(ws),
                                                    ws.numel(), B, P, F._stream()))
-        return grad_img, grad_k.reshape(ctx.kshape), None, None, None
+        return grad_img, grad_k.reshape(ctx.kshape), None, None, None, None
 
 
 class LensPsf(torch.autograd.Function):
@@ -363,6 +377,10 @@ class OpticsZernike(nn.Module):
         # bits; 0 / 0 = the reference
         self.sensor_noise_sigma = 0.0
         self.sensor_quant_bits = 0
+        # dtype of the returned sensor image, as on Camera: torch.float32 (the reference) or torch.bfloat16 for a downstream
+        # encoder that runs in bf16 - exactly the fp32 image .to(torch.bfloat16), written by the normalise kernel; backward =
+        # the fp32 one on g.float().  PSF, coefficients, loss and dL/dimg keep their dtypes.  Set by the caller.
+        self.sensor_dtype = torch.float32
         self._const: dict = {}            # per-device constant tables (wavefront, aperture, transfer function)
         self._plans: dict = {}
         self._process_group = None
@@ -544,9 +562,10 @@ class OpticsZernike(nn.Module):
         x = TF.interpolate(x, size=2 * [up * target], mode="nearest")     # torchvision Resize(interpolation=0)
         return TF.avg_pool2d(x, up, stride=up).permute(0, 2, 3, 1)
 
-    def _sensor(self, img: torch.Tensor, psf: torch.Tensor, epilogue=None) -> torch.Tensor:
+    def _sensor(self, img: torch.Tensor, psf: torch.Tensor, epilogue=None, out_dtype: torch.dtype = torch.float32) -> torch.Tensor:
         """img_psf_conv (Utils.py:251-297): zero-pad to 2P, circular FFT convolution, abs, crop, nearest resize; then the batch-global
-        max of Lens.py:312 and the opt-in read-out ``epilogue`` (``F.read_out``).  ``img``: fp32, or uint8 read as img / 255.0."""
+        max of Lens.py:312 and the opt-in read-out ``epilogue`` (``F.read_out``).  ``img``: fp32, or uint8 read as img / 255.0.
+        ``out_dtype``: the fused kernels write bf16 themselves; the other geometries cast the fp32 result with torch."""
         P = img.shape[2]
         if img.dim() != 4 or img.shape[1] != 3 or img.shape[3] != P or psf.shape[1] != P:
             raise ValueError(f"expected images (B,3,{psf.shape[1]},{psf.shape[1]}), got {tuple(img.shape)}")
@@ -562,7 +581,7 @@ class OpticsZernike(nn.Module):
             # patch sizes whose padded transform is not a power of two (the constructor default 368 -> 736): the reference's
             # own expression on the GPU (torch.fft), so that every constructor-valid geometry runs
             y = GlobalMaxNormalise.apply(self._sensor_torch(img.to(torch.float32), psf, n, pt, pb), self._process_group)
-            return self._read_out_torch(y, epilogue)
+            return self._read_out_torch(y, epilogue).to(out_dtype)
         x = None if fused else TF.pad(img.to(torch.float32), [pt, pb, pt, pb])
         # psf2otf (Utils.py:127-158): pad so that the PSF centre lands on n/2, the kernel's "centred frame"
         if (n - P) % 2 != 0:
@@ -572,10 +591,10 @@ class OpticsZernike(nn.Module):
         k = TF.pad(psf[0].permute(2, 0, 1).to(torch.float32), [kt, kb, kt, kb])          # (3, n, n)
         plan = self._plan(img.device, n)
         if fused:      # padding, |.|, crop, resize, the batch-global max and the read-out inside the kernels (csrc/lens_conv.cu)
-            return LensSensor.apply(img, k, plan, self._process_group, epilogue)
+            return LensSensor.apply(img, k, plan, self._process_group, epilogue, out_dtype)
         # |.|, the [pt+1 : n-pb] crop to (P-1)^2 and the nearest resize back to P (out[i] = crop[max(i-1,0)]) in one pass
         out = CropAbsResize.apply(CircConv.apply(x, k, plan), P, pt + 1, plan)
-        return self._read_out_torch(GlobalMaxNormalise.apply(out, self._process_group), epilogue)
+        return self._read_out_torch(GlobalMaxNormalise.apply(out, self._process_group), epilogue).to(out_dtype)
 
     @staticmethod
     def _read_out_torch(y: torch.Tensor, epilogue) -> torch.Tensor:
@@ -614,7 +633,9 @@ class OpticsZernike(nn.Module):
         """The reference's forward (Lens.py:157-316).  ``input_img``: (B,3,P,P) fp32, or uint8 (what a decoder or the caption
         HDF5 store yields; read as input_img / 255.0 on the GPU, a quarter of the host-to-device bytes).  ``noise``: optional
         standard-normal tensor shaped like the batch for the opt-in sensor noise (``sensor_noise_sigma``); with sigma > 0 and
-        none given it is drawn with torch.randn AFTER the lens tolerance field, so a seeded run draws both in the same order."""
+        none given it is drawn with torch.randn AFTER the lens tolerance field, so a seeded run draws both in the same order.
+        The sensor image is returned in ``sensor_dtype``."""
+        out_dtype = F.check_sensor_dtype(self.sensor_dtype)
         if psf_lab is True:
             raise NotImplementedError("psf_lab loads '../dataset_paula_real/psf_lab.jpg' in the reference (Lens.py:222-236)")
         if self.upsample:
@@ -642,7 +663,7 @@ class OpticsZernike(nn.Module):
 
         epilogue = (F.read_out(input_img, self.sensor_noise_sigma, self.sensor_quant_bits, noise)
                     if torch.is_tensor(input_img) else None)
-        sensor = self._sensor(input_img, psf, epilogue)
+        sensor = self._sensor(input_img, psf, epilogue, out_dtype)
         np.random.uniform(low=0.001, high=0.02)                     # noise_sigma is drawn and discarded (Lens.py:295)
         return sensor, psf, coeffs, loss                            # (the batch-global max of Lens.py:312 is inside _sensor)
 

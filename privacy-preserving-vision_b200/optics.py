@@ -65,6 +65,10 @@ class Camera(nn.Module):
         # standard deviation on the normalised sensor image, then quantisation to this many bits; 0 / 0 = the reference
         self.sensor_noise_sigma = 0.0
         self.sensor_quant_bits = 0
+        # dtype of the returned sensor image: torch.float32 (the reference) or torch.bfloat16 for a downstream net that runs in
+        # bf16 (torch.autocast).  bf16 = the fp32 image rounded to nearest-even, written by the kernels; its bf16 gradient is read
+        # by them as it is (backward = the fp32 one on g.float()).  Set by the caller, never inferred from autocast.
+        self.sensor_dtype = torch.float32
         self.overlap_psf = True          # run the PSF-independent half of forward() beside the PSF synthesis
         self._plans: dict[torch.device, F.DevicePlan] = {}
         self._pending_centering = None
@@ -156,7 +160,8 @@ class Camera(nn.Module):
 
     def forward(self, img, noise=None):
         """`noise`: optional standard-normal tensor shaped like `img` for the opt-in sensor noise (drawn here with
-        torch.randn when `sensor_noise_sigma > 0` and none is given)."""
+        torch.randn when `sensor_noise_sigma > 0` and none is given).  The sensor image is returned in `sensor_dtype`."""
+        out_dtype = F.check_sensor_dtype(self.sensor_dtype)
         # uint8 images (what a decoder produces; the reference's loader turns them into fp32 in [0,1] with ToTensor on the
         # host, Face-DeId/core/data_loader.py:118-124) may be passed as they are: the division by 255 then happens on the
         # GPU and the host->device copy is a quarter of the fp32 one.
@@ -172,11 +177,13 @@ class Camera(nn.Module):
         if not overlap:
             psf = self.get_psf()
             self.centering_loss = self._pending_centering
-            return F.sensor_conv(img, psf, self._plan(psf.device), None, epi)
+            return F.sensor_conv(img, psf, self._plan(psf.device), None, epi, out_dtype)
         plan = self._plan(img.device)
         side = plan.side_stream()
         psf = self.get_psf(_stream=side)                       # enqueued on `side`, not joined yet
-        rows = F.sensor_rows(img, plan) if psf.device == img.device else None
+        # (the bf16 read-out runs the default pipeline only: not the plane layout that sensor_rows writes with B200CAM_PLANE=1)
+        split = psf.device == img.device and not (out_dtype == torch.bfloat16 and self.N == 256 and F.PLANE_KERNELS)
+        rows = F.sensor_rows(img, plan) if split else None
         cur = torch.cuda.current_stream(psf.device)
         if rows is not None and plan.otf_event is not None:
             # the spectral product only needs the OTF: the PSF itself and the two regularisers are written on a
@@ -191,14 +198,14 @@ class Camera(nn.Module):
             plan.finish_psf(aux)
             cur.wait_event(ev)
             self.centering_loss = self._pending_centering
-            y = F.sensor_conv(img, psf, self._plan(psf.device), rows, epi)
+            y = F.sensor_conv(img, psf, self._plan(psf.device), rows, epi, out_dtype)
             cur.wait_stream(aux)
             cur.wait_stream(side)
             return y
         plan.finish_psf(side)
         cur.wait_stream(side)
         self.centering_loss = self._pending_centering
-        return F.sensor_conv(img, psf, self._plan(psf.device), rows, epi)
+        return F.sensor_conv(img, psf, self._plan(psf.device), rows, epi, out_dtype)
 
     # ------------------------------------------------------------------ CUDA-graph helper (no reference counterpart)
     def graphed(self, sample_img: torch.Tensor, num_warmup_iters: int = 3):
@@ -216,8 +223,8 @@ class Camera(nn.Module):
 
         The two regularisers are RETURNED (the module attributes ``loss_rad`` / ``centering_loss`` set during capture are not
         connected to the replayed graph).  Capture before the module's first eager backward (PyTorch's rule for
-        ``make_graphed_callables``: gradient-accumulation nodes created on the default stream cannot join a capture).  Re-capture after changing N, the batch size, ``data_parallel`` or the epilogue
-        switches.  Parameter updates in place (optimiser steps, ``load_state_dict``) are picked up by the replays."""
+        ``make_graphed_callables``: gradient-accumulation nodes created on the default stream cannot join a capture).  Re-capture after changing N, the batch size, ``data_parallel``, the epilogue
+        switches or ``sensor_dtype`` (the graph keeps the dtype it was captured with).  Parameter updates in place (optimiser steps, ``load_state_dict``) are picked up by the replays."""
         if not (torch.is_tensor(sample_img) and sample_img.is_cuda):
             raise RuntimeError("b200cam runs on CUDA (sm_100a) only; capture needs a sample batch on the GPU")
 

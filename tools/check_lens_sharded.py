@@ -2,7 +2,8 @@
 (`OpticsZernike.data_parallel`: all-reduce MAX of the batch-global maximum, SUM of sum(g*y) and of the tie count) must
 reproduce the single-GPU result on the whole batch - sensor images and the gradient of the trainable coefficient
 (summed over ranks).  Lens.py:312 couples all images of a batch; T5 in SURVEY 8.
-usage: python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 tools/check_lens_sharded.py
+usage: python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 tools/check_lens_sharded.py [--bf16]
+--bf16: both cameras with sensor_dtype = torch.bfloat16 (bf16 sensor images, bf16 upstream gradient).
 """
 import sys
 from pathlib import Path
@@ -16,6 +17,7 @@ from b200cam.lens import OpticsZernike     # noqa: E402
 
 
 def main():
+    out_dtype = torch.bfloat16 if "--bf16" in sys.argv[1:] else torch.float32
     rank, world, local = parallel.init_from_env("nccl")
     dev = torch.device("cuda", local)
     wave, patch, terms, per = 128, 64, 10, 3
@@ -27,6 +29,7 @@ def main():
         with torch.no_grad():
             cam.zernike_coeffs_train.fill_(-0.45)
             cam.zernike_coeffs_no_train2[1] = 0.3
+        cam.sensor_dtype = out_dtype
         return cam
 
     g = torch.Generator().manual_seed(31)
@@ -36,23 +39,25 @@ def main():
 
     whole = build()
     y_all, _, _, _ = whole(img.to(dev))
-    (y_all * w.to(dev)).sum().backward()
+    (y_all * w.to(dev, out_dtype)).sum().backward()
     g_all = whole.zernike_coeffs_train.grad.clone()
 
     shard = build().data_parallel()
     sl = slice(rank * per, (rank + 1) * per)
     y, _, _, _ = shard(img[sl].to(dev))
-    (y * w[sl].to(dev)).sum().backward()
+    (y * w[sl].to(dev, out_dtype)).sum().backward()
     g_sum = shard.zernike_coeffs_train.grad.clone()
     dist.all_reduce(g_sum)
 
-    e_y = float((y - y_all[sl]).norm() / y_all[sl].norm())
+    assert y.dtype == out_dtype
+    y, y_ref = y.float(), y_all[sl].float()
+    e_y = float((y - y_ref).norm() / y_ref.norm())
     e_g = float((g_sum - g_all).abs().max() / g_all.abs().max())
     ok = e_y <= 1e-6 and e_g <= 1e-4
     flag = torch.tensor([1.0 if ok else 0.0], device=dev)
     dist.all_reduce(flag, op=dist.ReduceOp.MIN)
     if rank == 0:
-        print(f"LENS_SHARDED world={world} sensor_rel={e_y:.2e} grad_rel={e_g:.2e} ok={bool(flag.item())}", flush=True)
+        print(f"LENS_SHARDED world={world} dtype={str(out_dtype).split('.')[-1]} sensor_rel={e_y:.2e} grad_rel={e_g:.2e} ok={bool(flag.item())}", flush=True)
     dist.destroy_process_group()
     sys.exit(0 if flag.item() == 1.0 else 1)
 
