@@ -232,6 +232,32 @@ int b200cam_sensor_bwd_bf16(const unsigned short* grad_sensor, const float* img,
                             const int* tie_pos, const float* psf, const float* otf, const float* spectrum, float* grad_psf,
                             float* grad_img, void* workspace, size_t workspace_bytes, int B, int N, void* stream);
 
+/* uint8 images (what a decoder yields, a quarter of the bytes of fp32): the same calls with img [B][3][N][N] as uint8, 16-byte
+ * aligned.  Each value is read as x * fp32(1/255) wherever the kernels read the image (the row transforms, the arg-max term of
+ * the backward), bit-identical to torch's img.float() / 255.0 on the GPU: every output - sensor image (fp32 or bf16), spectra,
+ * dL/dpsf, dL/dimg - is that of the fp32 call on the converted batch, bit for bit.  No fp32 copy of the batch is made.
+ *   b200cam_sensor_rows_u8       b200cam_sensor_rows; finish with b200cam_sensor_finish / _finish_ex / _finish_bf16 unchanged
+ *   b200cam_sensor_fwd_u8        b200cam_sensor_fwd_ex (epilogue arguments included)
+ *   b200cam_sensor_fwd_u8_bf16   b200cam_sensor_fwd_bf16
+ *   b200cam_sensor_bwd_u8        b200cam_sensor_bwd (the same img as the forward; spectrum NULL re-runs the row pass on it)
+ *   b200cam_sensor_bwd_u8_bf16   b200cam_sensor_bwd_bf16
+ * Workspace sizes are those of the fp32 calls.  These always run the default two-pass pipeline (the opt-in B200CAM_PLANE=1
+ * kernels read fp32 images only; B200CAM_ONE_PASS=1 still applies).  With B200CAM_PLANE=1 at N = 256 b200cam_sensor_finish
+ * expects the plane layout, so b200cam_sensor_rows_u8 returns B200CAM_E_BAD_SIZE there (use b200cam_sensor_fwd_u8). */
+int b200cam_sensor_rows_u8(const unsigned char* img, float* spectrum, float* img_max, int* tie_count, int B, int N, void* stream);
+int b200cam_sensor_fwd_u8(const unsigned char* img, const float* psf, float* sensor, float* img_max, int* tie_count, int* tie_pos,
+                          float* otf, float* spectrum, void* workspace, size_t workspace_bytes, int B, int N, void* stream, int flags,
+                          const float* noise, float noise_scale, int quant_bits);
+int b200cam_sensor_fwd_u8_bf16(const unsigned char* img, const float* psf, float* conv, unsigned short* sensor, float* img_max,
+                               int* tie_count, int* tie_pos, float* otf, float* spectrum, void* workspace, size_t workspace_bytes,
+                               int B, int N, void* stream, int flags, const float* noise, float noise_scale, int quant_bits);
+int b200cam_sensor_bwd_u8(const float* grad_sensor, const unsigned char* img, const float* sensor, const float* img_max,
+                          const int* tie_count, const int* tie_pos, const float* psf, const float* otf, const float* spectrum,
+                          float* grad_psf, float* grad_img, void* workspace, size_t workspace_bytes, int B, int N, void* stream);
+int b200cam_sensor_bwd_u8_bf16(const unsigned short* grad_sensor, const unsigned char* img, const float* img_max, const int* tie_count,
+                               const int* tie_pos, const float* psf, const float* otf, const float* spectrum, float* grad_psf,
+                               float* grad_img, void* workspace, size_t workspace_bytes, int B, int N, void* stream);
+
 /* Plain circular convolution of a batch with one centred kernel per channel, and its adjoints.  Replaces the FFT
  * part of img_psf_conv (Image_Caption/Camera/Utils.py:251-297): the caller zero-pads image and PSF to N (a power of
  * two, Utils.py:266-277 and psf2otf :127-158), then

@@ -109,6 +109,18 @@ _SIGNATURES = {
     "b200cam_lens_sensor_dot_bf16": (ctypes.c_int, [_f, _f, _f, _f, _f, ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_void_p]),
     "b200cam_lens_sensor_bwd_bf16": (ctypes.c_int, [_f, _f, _f, _f, _f, _f, _f, _f, _f, ctypes.c_size_t, ctypes.c_int, ctypes.c_int,
                                                     ctypes.c_void_p]),
+    # uint8 images in (unsigned char*: passed as plain device pointers)
+    "b200cam_sensor_rows_u8": (ctypes.c_int, [_f, _f, _f, _f, ctypes.c_int, ctypes.c_int, ctypes.c_void_p]),
+    "b200cam_sensor_fwd_u8": (ctypes.c_int, [_f, _f, _f, _f, _f, _f, _f, _f,
+                                             _f, ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_void_p,
+                                             ctypes.c_int, _f, ctypes.c_float, ctypes.c_int]),
+    "b200cam_sensor_fwd_u8_bf16": (ctypes.c_int, [_f, _f, _f, _f, _f, _f, _f, _f, _f,
+                                                  _f, ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_void_p,
+                                                  ctypes.c_int, _f, ctypes.c_float, ctypes.c_int]),
+    "b200cam_sensor_bwd_u8": (ctypes.c_int, [_f, _f, _f, _f, _f, _f, _f, _f, _f, _f, _f,
+                                             _f, ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_void_p]),
+    "b200cam_sensor_bwd_u8_bf16": (ctypes.c_int, [_f, _f, _f, _f, _f, _f, _f, _f, _f, _f,
+                                                  _f, ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_void_p]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 

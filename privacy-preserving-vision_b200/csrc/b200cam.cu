@@ -95,7 +95,8 @@ __global__ void __launch_bounds__(ReduceInvSmem<N>::THREADS) k_cols_reduce_inv(C
     DeviceExec ex;
     cols_reduce_inv_body<N>(ex, p, SMEM2);
 }
-__global__ void __launch_bounds__(EW_THREADS) k_tie_term(TieTermParams p) {
+template <class Img = float>
+__global__ void __launch_bounds__(EW_THREADS) k_tie_term(TieTermParamsT<Img> p) {
     pdl_gate();
     __shared__ float s_coef[TIE_PASS * MAX_TIES];
     __shared__ int s_meta[3 * TIE_PASS * MAX_TIES];
@@ -574,6 +575,7 @@ struct DeviceState {
     cudaEvent_t chain_ev = nullptr;                      // orders a caller stream behind the first PSF-chain kernel
     int r2c_fit[11] = {0}, c2r_fit[11] = {0};            // resident CTAs per SM of the persistent row kernels
     int r2c16_fit[11] = {0};                             // ... and of the bf16-input forward row kernel (upstream gradient)
+    int r2c8_fit[11] = {0};                              // ... and of the uint8-input forward row kernel (uint8 images)
     float* scratch = nullptr;                            // SCRATCH_FLOATS floats: slice partials of the Zernike adjoint
     int prow_fit = 0, pconv_g3 = 0, pacc_g3 = 0;         // plane kernels (N = 256): resident CTAs per SM / co-resident cluster triples
     unsigned* err_host = nullptr; unsigned* err_dev = nullptr;   // device error word (mapped pinned host memory)
@@ -628,6 +630,8 @@ static cudaError_t init_kernels() {
     if ((e = optin(k_rows_r2c_persist<N>, RowsStreamSmem<N>::BYTES))) return e;
     if ((e = optin(k_rows_r2c<N, bf16>, RowsR2CSmem<N>::BYTES))) return e;
     if ((e = optin(k_rows_r2c_persist<N, bf16>, RowsStreamSmem<N, bf16>::BYTES))) return e;
+    if ((e = optin(k_rows_r2c<N, u8>, RowsR2CSmem<N>::BYTES))) return e;
+    if ((e = optin(k_rows_r2c_persist<N, u8>, RowsStreamSmem<N, u8>::BYTES))) return e;
     if ((e = optin(k_rows_c2r_persist<N, false>, RowsC2RStreamSmem<N>::BYTES))) return e;
     if ((e = optin(k_rows_c2r_persist<N, true>, RowsC2RStreamSmem<N>::BYTES))) return e;
     if ((e = optin(k_cols_conv<N>, ColsSmem<N>::BYTES_CONV))) return e;
@@ -663,11 +667,13 @@ static cudaError_t coop_grid_size(int dev, int sms, int* out) {
 
 // resident CTAs (one wave) of the persistent column kernels on this device
 template <int N>
-static cudaError_t row_fits(int* r2c, int* r2c16, int* c2r) {
+static cudaError_t row_fits(int* r2c, int* r2c16, int* r2c8, int* c2r) {
     cudaError_t e;
     if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(r2c, k_rows_r2c_persist<N>, RowsStreamSmem<N>::THREADS, RowsStreamSmem<N>::BYTES))) return e;
     if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(r2c16, k_rows_r2c_persist<N, bf16>, RowsStreamSmem<N, bf16>::THREADS,
                                                            RowsStreamSmem<N, bf16>::BYTES))) return e;
+    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(r2c8, k_rows_r2c_persist<N, u8>, RowsStreamSmem<N, u8>::THREADS,
+                                                           RowsStreamSmem<N, u8>::BYTES))) return e;
     return cudaOccupancyMaxActiveBlocksPerMultiprocessor(c2r, k_rows_c2r_persist<N, false>, RowsC2RStreamSmem<N>::THREADS, RowsC2RStreamSmem<N>::BYTES);
 }
 template <int N>
@@ -740,10 +746,12 @@ static int persistent_grid(int fit, int want_per_sm, int total_tiles) {
     const long long cap = static_cast<long long>(sms) * per_sm;
     return static_cast<int>(total_tiles < cap ? total_tiles : cap);
 }
-static int rows_fit(int N, bool inverse, bool bf16_input = false) {
+// in_bytes: element size of the forward row kernel's input (4 fp32, 2 bf16, 1 uint8)
+static int rows_fit(int N, bool inverse, int in_bytes = 4) {
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= MAX_DEV) return 1;
-    if (bf16_input) return g_state[dev].r2c16_fit[log2i(N)];
+    if (!inverse && in_bytes == 2) return g_state[dev].r2c16_fit[log2i(N)];
+    if (!inverse && in_bytes == 1) return g_state[dev].r2c8_fit[log2i(N)];
     return inverse ? g_state[dev].c2r_fit[log2i(N)] : g_state[dev].r2c_fit[log2i(N)];
 }
 
@@ -1043,15 +1051,16 @@ static int otf_cols_impl(const float2* rows, float2* otf, const float2* tw, floa
 // first half of the generic forward: row transforms of the images (independent of the PSF, so a caller may run it on a
 // second stream while b200cam_psf_fwd is still busy); also resets the per-image max / tie counters
 // allow_plane = false: always the standard spectrum layout (the bf16 sensor path runs the default two-pass pipeline only)
-template <int N>
-static int sensor_rows_impl(const float* img, float2* srow, float* img_max, int* tie_count, int B, cudaStream_t s,
+// Img = u8: uint8 images, converted in the row kernel; always the standard layout (the plane kernels read fp32 only)
+template <int N, class Img = float>
+static int sensor_rows_impl(const Img* img, float2* srow, float* img_max, int* tie_count, int B, cudaStream_t s,
                             bool allow_plane = true) {
     using T = Tile<N>;
     const float2* tw = twiddle(N);
     if (tw == nullptr) return B200CAM_E_NOT_INIT;
     // B200CAM_ROWS_PER_SM resident CTAs per SM (default 3 of the 4 that fit): see k_rows_r2c_persist
     static const int per_sm = [] { const char* e = getenv("B200CAM_ROWS_PER_SM"); const int v = e ? atoi(e) : 3; return v > 0 ? v : 3; }();
-    if constexpr (N == 256) {
+    if constexpr (N == 256 && std::is_same<Img, float>::value) {
         if (allow_plane && plane_selected()) {
             // plane layout "A"; the words behind it (the buffer is sized for 129 columns, A uses 128) hold the per-image
             // {max key, arrivals} pairs of k_pconv: reset here, early, beside the PSF chain
@@ -1068,9 +1077,9 @@ static int sensor_rows_impl(const float* img, float2* srow, float* img_max, int*
         }
     }
     const int total = (N / T::ROWS) * 3 * B;
-    const int grid = persistent_grid(rows_fit(N, false), per_sm, total);
-    launch_k(k_rows_r2c_persist<N>, grid, RowsStreamSmem<N>::THREADS, RowsStreamSmem<N>::BYTES, s, 
-        RowsR2CParams{img, srow, tw, img_max, tie_count}, total);
+    const int grid = persistent_grid(rows_fit(N, false, static_cast<int>(sizeof(Img))), per_sm, total);
+    launch_k(k_rows_r2c_persist<N, Img>, grid, RowsStreamSmem<N, Img>::THREADS, RowsStreamSmem<N, Img>::BYTES, s,
+        RowsR2CParamsT<Img>{img, srow, tw, img_max, tie_count}, total);
     LAUNCH_CHECK();
     return 0;
 }
@@ -1078,10 +1087,13 @@ static int sensor_rows_impl(const float* img, float2* srow, float* img_max, int*
 // second half: OTF of the PSF, column convolution, inverse rows + per-image max, normalise
 // out16 != nullptr: bf16 sensor image.  `sensor` is then the fp32 conv scratch, and the default two-pass pipeline runs
 // whatever B200CAM_PLANE / B200CAM_ONE_PASS say (those opt-in kernels write fp32 only).
+// allow_plane = false: `srow` is in the standard layout whatever B200CAM_PLANE says (the uint8 row pass writes no other), so
+// the plane kernels are not used for this call; the one-pass kernel still is (it reads the standard layout).
 template <int N>
 static int sensor_finish_impl(const float* psf, float* sensor, float* img_max, int* tie_count, int* tie_pos, float2* otf,
                               const float2* srow, const SensorWs& ws, int B, int otf_ready, cudaStream_t s,
-                              SensorEpilogue epi = SensorEpilogue{nullptr, 0.f, 0.f}, bf16* out16 = nullptr) {
+                              SensorEpilogue epi = SensorEpilogue{nullptr, 0.f, 0.f}, bf16* out16 = nullptr,
+                              bool allow_plane = true) {
     using T = Tile<N>;
     const float2* tw = twiddle(N);
     if (tw == nullptr) return B200CAM_E_NOT_INIT;
@@ -1091,7 +1103,7 @@ static int sensor_finish_impl(const float* psf, float* sensor, float* img_max, i
     }
     const int planes = 3 * B;
     if constexpr (N == 256) {
-        if (out16 == nullptr && plane_selected() && epi.noise == nullptr && epi.levels <= 0.f) {   // (the opt-in plane kernels have no read-out epilogue)
+        if (allow_plane && out16 == nullptr && plane_selected() && epi.noise == nullptr && epi.levels <= 0.f) {   // (the opt-in plane kernels have no read-out epilogue)
             const DeviceState* st = cur_state();
             if (st == nullptr || st->pconv_g3 < 1) return B200CAM_E_NOT_INIT;
             const int G3 = B < st->pconv_g3 ? B : st->pconv_g3;
@@ -1270,21 +1282,24 @@ static int conv_bwd_impl(const float* g, const float* img, const float2* otf, co
     return 0;
 }
 
-template <int N>
-static int sensor_fwd_impl(const float* img, const float* psf, float* sensor, float* img_max, int* tie_count,
+template <int N, class Img = float>
+static int sensor_fwd_impl(const Img* img, const float* psf, float* sensor, float* img_max, int* tie_count,
                            int* tie_pos, float2* otf, float2* spectrum, void* ws_ptr, int B, cudaStream_t s,
                            SensorEpilogue epi = SensorEpilogue{nullptr, 0.f, 0.f}, bf16* out16 = nullptr) {
     SensorWs ws(ws_ptr, N, B, false);
     float2* srow = spectrum != nullptr ? spectrum : ws.stx;      // row spectra: kept for the backward when asked
-    int rc = sensor_rows_impl<N>(img, srow, img_max, tie_count, B, s, out16 == nullptr);
+    constexpr bool FP32_IMG = std::is_same<Img, float>::value;  // (uint8 images: standard layout, no plane kernels)
+    int rc = sensor_rows_impl<N, Img>(img, srow, img_max, tie_count, B, s, out16 == nullptr);
     if (rc) return rc;
-    return sensor_finish_impl<N>(psf, sensor, img_max, tie_count, tie_pos, otf, srow, ws, B, 0, s, epi, out16);
+    return sensor_finish_impl<N>(psf, sensor, img_max, tie_count, tie_pos, otf, srow, ws, B, 0, s, epi, out16, FP32_IMG);
 }
 
 // In = bf16: the upstream gradient arrives in bf16 and is widened in the row kernels; everything after them is the fp32
 // pipeline (the plane kernels are fp32 only: the bf16 path always runs the generic one)
-template <int N, class In = float>
-static int sensor_bwd_impl(const In* g, const float* img, const float* sensor, const float* img_max,
+// Img = u8: the images are uint8 (converted in registers wherever they are read: the row pass that rebuilds the spectra when
+// the forward kept none, and the arg-max gather); likewise the generic pipeline only
+template <int N, class In = float, class Img = float>
+static int sensor_bwd_impl(const In* g, const Img* img, const float* sensor, const float* img_max,
                            const int* tie_count, const int* tie_pos, const float* psf, const float2* otf,
                            const float2* spectrum, float* grad_psf, float* grad_img, void* ws_ptr, int B,
                            cudaStream_t s) {
@@ -1294,7 +1309,7 @@ static int sensor_bwd_impl(const In* g, const float* img, const float* sensor, c
     SensorWs ws(ws_ptr, N, B, true);
     const int planes = 3 * B, tiles = N / T::ROWS;
     const dim3 rgrid(tiles, planes);
-    if constexpr (N == 256 && std::is_same<In, float>::value) {
+    if constexpr (N == 256 && std::is_same<In, float>::value && std::is_same<Img, float>::value) {
         if (plane_selected()) {
             const DeviceState* st = cur_state();
             if (st == nullptr || st->pacc_g3 < 1 || st->pconv_g3 < 1) return B200CAM_E_NOT_INIT;
@@ -1322,7 +1337,7 @@ static int sensor_bwd_impl(const In* g, const float* img, const float* sensor, c
                 RowsC2RParams{ws.stp, grad_psf, tw, nullptr, 1.0f});
             LAUNCH_CHECK();
             const int per_ch = N * N / 2 / EW_THREADS < 592 ? N * N / 2 / EW_THREADS : 592;
-            launch_k(Pdl{}, k_tie_term, dim3(per_ch, 3), EW_THREADS, 0, s, TieTermParams{grad_psf, img, tie_count, tie_pos, ws.coef, B, N});
+            launch_k(Pdl{}, k_tie_term<>, dim3(per_ch, 3), EW_THREADS, 0, s, TieTermParams{grad_psf, img, tie_count, tie_pos, ws.coef, B, N});
             LAUNCH_CHECK();
             if (grad_img != nullptr) {           // optional output (no reference caller asks for it): generic kernels on g
                 launch_k(k_rows_r2c<N>, rgrid, RowsR2CSmem<N>::THREADS, RowsR2CSmem<N>::BYTES, s, RowsR2CParams{g, ws.stg, tw, nullptr, nullptr});
@@ -1345,8 +1360,8 @@ static int sensor_bwd_impl(const In* g, const float* img, const float* sensor, c
     }
     const float2* srow = spectrum;
     if (srow == nullptr) {                       // forward did not keep the row spectra: recompute them
-        launch_k(k_rows_r2c<N>, rgrid, RowsR2CSmem<N>::THREADS, RowsR2CSmem<N>::BYTES, s, 
-            RowsR2CParams{img, ws.stx, tw, nullptr, nullptr});
+        launch_k(k_rows_r2c<N, Img>, rgrid, RowsR2CSmem<N>::THREADS, RowsR2CSmem<N>::BYTES, s,
+            RowsR2CParamsT<Img>{img, ws.stx, tw, nullptr, nullptr});
         LAUNCH_CHECK();
         srow = ws.stx;
     }
@@ -1357,7 +1372,7 @@ static int sensor_bwd_impl(const In* g, const float* img, const float* sensor, c
         static const int per_sm = [] { const char* e = getenv("B200CAM_GROWS_PER_SM"); return e ? atoi(e) : 3; }();
         if (per_sm > 0) {
             const int total = tiles * planes;
-            const int grid = persistent_grid(rows_fit(N, false, !std::is_same<In, float>::value), per_sm, total);
+            const int grid = persistent_grid(rows_fit(N, false, static_cast<int>(sizeof(In))), per_sm, total);
             launch_k(k_rows_r2c_persist<N, In>, grid, RowsStreamSmem<N, In>::THREADS, RowsStreamSmem<N, In>::BYTES, s,
                 RowsR2CParamsT<In>{g, ws.stg, tw, nullptr, nullptr}, total);
         } else {
@@ -1384,14 +1399,14 @@ static int sensor_bwd_impl(const In* g, const float* img, const float* sensor, c
     launch_k(Pdl{}, k_cols_reduce_inv<N>, 3 * T::NC + (side_job ? B : 0), ReduceInvSmem<N>::THREADS, ReduceInvSmem<N>::BYTES, s, 
         ColsReduceInvParams{ws.partial, ws.stp, tw, nchunks, 1.0f / (static_cast<float>(N) * N),
                             side_job ? ws.dot_lanes : nullptr, img_max, tie_count, ws.coef, B, spectral ? nullptr : img, tie_pos,
-                            spectral ? srow : nullptr, dot_warps, dot_count});
+                            spectral ? srow : nullptr, dot_warps, dot_count, static_cast<int>(sizeof(Img))});
     LAUNCH_CHECK();
-    launch_k(Pdl{}, k_rows_c2r<N>, dim3(tiles, 3), RowsR2CSmem<N>::THREADS, RowsR2CSmem<N>::BYTES, s, 
+    launch_k(Pdl{}, k_rows_c2r<N>, dim3(tiles, 3), RowsR2CSmem<N>::THREADS, RowsR2CSmem<N>::BYTES, s,
         RowsC2RParams{ws.stp, grad_psf, tw, nullptr, 1.0f});
     LAUNCH_CHECK();
     if (!spectral) {   // arg-max term of the amax backward (spatial form), ties of channel c handled by the CTAs of row c
         const int per_ch = N * N / 2 / EW_THREADS < 592 ? N * N / 2 / EW_THREADS : 592;   // two adjacent pixels per thread
-        launch_k(Pdl{}, k_tie_term, dim3(per_ch, 3), EW_THREADS, 0, s, TieTermParams{grad_psf, img, tie_count, tie_pos, ws.coef, B, N});
+        launch_k(Pdl{}, k_tie_term<Img>, dim3(per_ch, 3), EW_THREADS, 0, s, TieTermParamsT<Img>{grad_psf, img, tie_count, tie_pos, ws.coef, B, N});
         LAUNCH_CHECK();
     }
     if (grad_img != nullptr) {
@@ -1573,13 +1588,14 @@ int b200cam_init(int N) {
     if (e == cudaSuccess) {
         int* rf = &g_state[dev].r2c_fit[l];
         int* rf16 = &g_state[dev].r2c16_fit[l];
+        int* rf8 = &g_state[dev].r2c8_fit[l];
         int* cf = &g_state[dev].c2r_fit[l];
         switch (N) {
-            case 64: e = row_fits<64>(rf, rf16, cf); break;
-            case 128: e = row_fits<128>(rf, rf16, cf); break;
-            case 256: e = row_fits<256>(rf, rf16, cf); break;
-            case 512: e = row_fits<512>(rf, rf16, cf); break;
-            case 1024: e = row_fits<1024>(rf, rf16, cf); break;
+            case 64: e = row_fits<64>(rf, rf16, rf8, cf); break;
+            case 128: e = row_fits<128>(rf, rf16, rf8, cf); break;
+            case 256: e = row_fits<256>(rf, rf16, rf8, cf); break;
+            case 512: e = row_fits<512>(rf, rf16, rf8, cf); break;
+            case 1024: e = row_fits<1024>(rf, rf16, rf8, cf); break;
         }
     }
     if (e != cudaSuccess) {
@@ -1977,6 +1993,88 @@ int b200cam_sensor_bwd_bf16(const unsigned short* grad_sensor, const float* img,
     const bf16* g = reinterpret_cast<const bf16*>(grad_sensor);
     DISPATCH_N(N, (sensor_bwd_impl<NN_, bf16>(g, img, nullptr, img_max, tie_count, tie_pos, psf, reinterpret_cast<const float2*>(otf),
                                               reinterpret_cast<const float2*>(spectrum), grad_psf, grad_img, workspace, B, s)));
+}
+
+// ---- uint8 images ------------------------------------------------------------------------------------------
+// The same calls with the images as uint8 bytes (what a decoder yields), converted in the kernels as byte * fp32(1/255), i.e.
+// exactly torch's u8.float() / 255.0 on the GPU: every output is that of the fp32 call on the converted batch, bit for bit.
+// They always run the default two-pass pipeline (the opt-in plane kernels read fp32 images only).
+int b200cam_sensor_rows_u8(const unsigned char* img, float* spectrum, float* img_max, int* tie_count, int B, int N, void* stream) {
+    if (!b200cam_supported(N) || B < 1) return B200CAM_E_BAD_SIZE;
+    if (N == 256 && plane_selected()) return B200CAM_E_BAD_SIZE;     // b200cam_sensor_finish would expect the plane layout
+    if (!img || !spectrum || !img_max || !tie_count) return B200CAM_E_NULL;
+    if (!aligned16(img) || !aligned16(spectrum)) return B200CAM_E_ALIGN;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const u8* x = reinterpret_cast<const u8*>(img);
+    DISPATCH_N(N, (sensor_rows_impl<NN_, u8>(x, reinterpret_cast<float2*>(spectrum), img_max, tie_count, B, s)));
+}
+
+int b200cam_sensor_fwd_u8(const unsigned char* img, const float* psf, float* sensor, float* img_max, int* tie_count, int* tie_pos,
+                          float* otf, float* spectrum, void* workspace, size_t workspace_bytes, int B, int N, void* stream, int flags,
+                          const float* noise, float noise_scale, int quant_bits) {
+    SensorEpilogue epi;
+    if (const int rc = make_epilogue(flags, noise, noise_scale, quant_bits, &epi)) return rc;
+    if (!b200cam_supported(N) || B < 1) return B200CAM_E_BAD_SIZE;
+    if (!img || !psf || !sensor || !img_max || !tie_count || !tie_pos || !otf || !workspace) return B200CAM_E_NULL;
+    if (workspace_bytes < b200cam_sensor_workspace_bytes(N, B, 0)) return B200CAM_E_WORKSPACE;
+    if (!aligned16(img) || !aligned16(sensor) || !aligned16(otf) || !aligned16(workspace) || !aligned16(psf) ||
+        (spectrum != nullptr && !aligned16(spectrum)))
+        return B200CAM_E_ALIGN;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const u8* x = reinterpret_cast<const u8*>(img);
+    DISPATCH_N(N, (sensor_fwd_impl<NN_, u8>(x, psf, sensor, img_max, tie_count, tie_pos, reinterpret_cast<float2*>(otf),
+                                            reinterpret_cast<float2*>(spectrum), workspace, B, s, epi)));
+}
+
+int b200cam_sensor_fwd_u8_bf16(const unsigned char* img, const float* psf, float* conv, unsigned short* sensor, float* img_max,
+                               int* tie_count, int* tie_pos, float* otf, float* spectrum, void* workspace, size_t workspace_bytes,
+                               int B, int N, void* stream, int flags, const float* noise, float noise_scale, int quant_bits) {
+    SensorEpilogue epi;
+    if (const int rc = make_epilogue(flags, noise, noise_scale, quant_bits, &epi)) return rc;
+    if (!b200cam_supported(N) || B < 1) return B200CAM_E_BAD_SIZE;
+    if (!img || !psf || !conv || !sensor || !img_max || !tie_count || !tie_pos || !otf || !workspace) return B200CAM_E_NULL;
+    if (workspace_bytes < b200cam_sensor_workspace_bytes(N, B, 0)) return B200CAM_E_WORKSPACE;
+    if (!aligned16(img) || !aligned16(conv) || !aligned16(sensor) || !aligned16(otf) || !aligned16(workspace) || !aligned16(psf) ||
+        (spectrum != nullptr && !aligned16(spectrum)))
+        return B200CAM_E_ALIGN;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const u8* x = reinterpret_cast<const u8*>(img);
+    bf16* out = reinterpret_cast<bf16*>(sensor);
+    DISPATCH_N(N, (sensor_fwd_impl<NN_, u8>(x, psf, conv, img_max, tie_count, tie_pos, reinterpret_cast<float2*>(otf),
+                                            reinterpret_cast<float2*>(spectrum), workspace, B, s, epi, out)));
+}
+
+int b200cam_sensor_bwd_u8(const float* grad_sensor, const unsigned char* img, const float* sensor, const float* img_max,
+                          const int* tie_count, const int* tie_pos, const float* psf, const float* otf, const float* spectrum,
+                          float* grad_psf, float* grad_img, void* workspace, size_t workspace_bytes, int B, int N, void* stream) {
+    if (!b200cam_supported(N) || B < 1) return B200CAM_E_BAD_SIZE;
+    if (!grad_sensor || !img || !sensor || !img_max || !tie_count || !tie_pos || !psf || !otf || !grad_psf || !workspace)
+        return B200CAM_E_NULL;
+    if (workspace_bytes < b200cam_sensor_workspace_bytes(N, B, grad_img != nullptr)) return B200CAM_E_WORKSPACE;
+    if (!aligned16(grad_sensor) || !aligned16(img) || !aligned16(sensor) || !aligned16(otf) || !aligned16(workspace) ||
+        !aligned16(grad_psf) || (spectrum && !aligned16(spectrum)) || (grad_img && !aligned16(grad_img)))
+        return B200CAM_E_ALIGN;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const u8* x = reinterpret_cast<const u8*>(img);
+    DISPATCH_N(N, (sensor_bwd_impl<NN_, float, u8>(grad_sensor, x, sensor, img_max, tie_count, tie_pos, psf,
+                                                   reinterpret_cast<const float2*>(otf), reinterpret_cast<const float2*>(spectrum),
+                                                   grad_psf, grad_img, workspace, B, s)));
+}
+
+int b200cam_sensor_bwd_u8_bf16(const unsigned short* grad_sensor, const unsigned char* img, const float* img_max, const int* tie_count,
+                               const int* tie_pos, const float* psf, const float* otf, const float* spectrum, float* grad_psf,
+                               float* grad_img, void* workspace, size_t workspace_bytes, int B, int N, void* stream) {
+    if (!b200cam_supported(N) || B < 1) return B200CAM_E_BAD_SIZE;
+    if (!grad_sensor || !img || !img_max || !tie_count || !tie_pos || !psf || !otf || !grad_psf || !workspace) return B200CAM_E_NULL;
+    if (workspace_bytes < b200cam_sensor_workspace_bytes(N, B, grad_img != nullptr)) return B200CAM_E_WORKSPACE;
+    if (!aligned16(grad_sensor) || !aligned16(img) || !aligned16(otf) || !aligned16(workspace) || !aligned16(grad_psf) ||
+        (spectrum && !aligned16(spectrum)) || (grad_img && !aligned16(grad_img)))
+        return B200CAM_E_ALIGN;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const bf16* g = reinterpret_cast<const bf16*>(grad_sensor);
+    const u8* x = reinterpret_cast<const u8*>(img);
+    DISPATCH_N(N, (sensor_bwd_impl<NN_, bf16, u8>(g, x, nullptr, img_max, tie_count, tie_pos, psf, reinterpret_cast<const float2*>(otf),
+                                                  reinterpret_cast<const float2*>(spectrum), grad_psf, grad_img, workspace, B, s)));
 }
 
 }  // extern "C"

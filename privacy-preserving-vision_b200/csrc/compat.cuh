@@ -79,9 +79,25 @@ B200_HD float to_float(bf16 v) {
     return f;
 #endif
 }
-// element loads through the read-only path (fp32, or bf16 widened in registers)
+// ---- uint8 images ----------------------------------------------------------------------------
+// A uint8 image byte, as a decoder yields it.  Its value is byte * fp32(1/255): torch's u8.float() / 255.0 on the GPU
+// multiplies by the fp32 reciprocal of the CPU scalar, so this is bit for bit the image the caller would otherwise convert
+// (ImgLoadU8 of lens_conv.cu is the same rule).  A tag type of its own, so that no generic unsigned char conversion picks
+// it up by accident.
+struct u8 {
+    unsigned char bits;
+};
+B200_HD float to_float(u8 v) {
+#if defined(__CUDA_ARCH__)
+    return __fmul_rn(static_cast<float>(v.bits), 1.0f / 255.0f);
+#else
+    return static_cast<float>(v.bits) * (1.0f / 255.0f);
+#endif
+}
+// element loads through the read-only path (fp32, or bf16 / uint8 widened in registers)
 B200_HD float load_elem(const float* p) { return ld_ro(p); }
 B200_HD float load_elem(const bf16* p) { return to_float(bf16{ld_ro(reinterpret_cast<const unsigned short*>(p))}); }
+B200_HD float load_elem(const u8* p) { return to_float(u8{ld_ro(reinterpret_cast<const unsigned char*>(p))}); }
 // fp32 -> bf16, round to nearest-even.  Device: __float2bfloat16_rn (the conversion torch's CUDA cast uses).  Host (emulator):
 // the same bit rule - add 0x7fff plus the lowest kept bit, truncate - which gives the identical result for every finite
 // value and for the infinities; NaN becomes the canonical quiet NaN of its sign.

@@ -38,7 +38,8 @@ struct Tile {
 //      init_max/init_count (tile 0 of channel 0) reset the per-image max / tie counters for the
 //      kernels that follow in the stream.
 // ---------------------------------------------------------------------------------------------
-// `In`: element type of x - fp32, or bf16 (an upstream gradient handed over in bf16; widened exactly in registers)
+// `In`: element type of x - fp32, bf16 (an upstream gradient handed over in bf16; widened exactly in registers) or u8 (a uint8
+// image, converted in registers as byte * fp32(1/255))
 template <class In>
 struct RowsR2CParamsT {
     const In* x;             // [planes][N][N]
@@ -139,7 +140,11 @@ struct RowsStreamSmem {
     // 4-byte word (a broadcast, not a conflict), so a row pair's R2 lanes touch R2/2 consecutive banks, and the rows of the
     // pairs that share a warp are 2 * (N + 8) / 2 = N + 8 words = 8 banks apart: the 2 (N = 128, 256) or 4 (N = 64) pairs of a
     // warp read disjoint banks.  The pitch stays a multiple of 16 bytes, as the bulk copies need.
-    static constexpr int ROW_PITCH = N + 8;                                   // elements; ROW_PITCH * sizeof(In) is a multiple of 16 bytes
+    // uint8 rows (In = u8): pitch N + 16 bytes (N + 8 would not be a multiple of 16).  Four lanes read the four bytes of one word
+    // (a broadcast), so a row pair's R2 lanes touch R2/4 consecutive banks, and the rows of the pairs that share a warp are
+    // 2 * (N + 16) / 4 = N/2 + 8 words = 8 banks apart (N/2 = 0 mod 32 for N >= 64): the 2 pairs (N = 128, 256, R2/4 = 4 banks
+    // each) or 4 pairs (N = 64, 2 banks each) of a warp again read disjoint banks.
+    static constexpr int ROW_PITCH = N + (sizeof(In) == 1 ? 16 : 8);          // elements; ROW_PITCH * sizeof(In) is a multiple of 16 bytes
     static constexpr int TILE_ELEMS = T::ROWS * ROW_PITCH;
     static constexpr int TILE_BYTES = T::ROWS * N * static_cast<int>(sizeof(In));   // bytes that arrive per tile
     static constexpr int STAGE_OFF = (R::RED_OFF + 15) / 16 * 16;            // float2 units, 128-byte aligned
@@ -1069,7 +1074,7 @@ struct ColsReduceInvParams {
     // the side-job CTA of image b also pulls the planes that the arg-max term (K8) is about to gather from - x_b[c*] for every
     // recorded arg-max - into L2: K8 runs two small kernels later and would otherwise pay a DRAM miss per gather (the images
     // were last read a whole step ago)
-    const float* x = nullptr;        // nullable [B][3][N][N]
+    const void* x = nullptr;         // nullable [B][3][N][N] of x_elem-byte elements (fp32, or uint8: N^2 bytes per plane)
     const int* tie_pos = nullptr;    // [B][MAX_TIES]
     // Arg-max term of the amax backward folded into this pass (srow != nullptr; replaces K8 tie_term and its launch):
     //   gpsf[c][p] -= sum_t coef_t x_b[c][(p*_t - p + N/2) mod N]
@@ -1080,6 +1085,7 @@ struct ColsReduceInvParams {
     const float2* srow = nullptr;    // nullable [B*3][NC][N]
     const float* dot_warps = nullptr;   // [B][dot_count]
     int dot_count = 0;
+    int x_elem = 4;                  // bytes per element of x (4: fp32 images, 1: uint8 images)
 };
 constexpr int RINV_PASS = 64;        // images staged per pass of the tie list (<= RINV_PASS * MAX_TIES entries)
 
@@ -1116,8 +1122,8 @@ B200_HD void cols_reduce_inv_body(Exec& ex, const ColsReduceInvParams& p, float2
                 const int n = p.tie_count[b] < C2R_MAX_TIES ? p.tie_count[b] : C2R_MAX_TIES;
                 for (int k = 0; k < n; ++k) {
                     const int c = p.tie_pos[b * C2R_MAX_TIES + k] / (N * N);
-                    const char* plane = reinterpret_cast<const char*>(p.x + (static_cast<size_t>(b) * 3 + c) * N * N);
-                    for (int line = t; line < N * N * 4 / 128; line += N) prefetch_l2(plane + static_cast<size_t>(line) * 128);
+                    const char* plane = static_cast<const char*>(p.x) + (static_cast<size_t>(b) * 3 + c) * N * N * p.x_elem;
+                    for (int line = t; line < N * N * p.x_elem / 128; line += N) prefetch_l2(plane + static_cast<size_t>(line) * 128);
                 }
             });
         }
@@ -1303,15 +1309,19 @@ B200_HD void cols_reduce_inv_body(Exec& ex, const ColsReduceInvParams& p, float2
 //      gpsf[c][p] -= sum_b sum_{ties t of image b in channel c} (s_b/(n_b m_b)) * x_b[c][(p*_t - p + N/2) mod N]
 //      with s_b = sum(g_b * y_b) from the Parseval partials of K6, reduced by K7 (coef).
 //      grid-stride over 3*N*N outputs.
+//      `Img` = u8: the gather reads the uint8 image and converts each value in registers (to_float), so every gathered
+//      value - and with it the sum, in the same order - is that of the fp32 kernel on the converted image.
 // ---------------------------------------------------------------------------------------------
-struct TieTermParams {
+template <class Img>
+struct TieTermParamsT {
     float* gpsf;              // [3][N][N] in place
-    const float* x;           // [B][3][N][N]
+    const Img* x;             // [B][3][N][N]
     const int* tie_count;     // [B]
     const int* tie_pos;       // [B][MAX_TIES]
     const float* coef;        // [B]: s_b / (n_b m_b), written by K7
     int B, N;
 };
+using TieTermParams = TieTermParamsT<float>;
 
 constexpr int TIE_PASS = 256;   // images staged per pass (= block size of the kernel)
 
@@ -1319,8 +1329,8 @@ constexpr int TIE_PASS = 256;   // images staged per pass (= block size of the k
 // Staging is parallel (thread t <-> image b0+t) and the compaction offsets come from an ordered
 // scan, so the list - and therefore the floating-point subtraction order - is deterministic.
 // shared: s_coef[TIE_PASS*MAX_TIES], s_meta[3*TIE_PASS*MAX_TIES], s_cnt[TIE_PASS+1]
-template <class Exec>
-B200_HD void tie_term_body(Exec& ex, const TieTermParams& p, int grid_x, float* s_coef, int* s_meta, int* s_cnt) {
+template <class Exec, class Img>
+B200_HD void tie_term_body(Exec& ex, const TieTermParamsT<Img>& p, int grid_x, float* s_coef, int* s_meta, int* s_cnt) {
     const int N = p.N, NN = N * N, c = ex.by();
     for (int b0 = 0; b0 < p.B; b0 += TIE_PASS) {
         const int nb = (p.B - b0 < TIE_PASS) ? p.B - b0 : TIE_PASS;
@@ -1369,9 +1379,9 @@ B200_HD void tie_term_body(Exec& ex, const TieTermParams& p, int grid_x, float* 
                             const int ee = e + q < k ? e + q : k - 1;
                             const int sy = (s_meta[3 * ee + 1] - py + N / 2 + N) & (N - 1);
                             const int sx = (s_meta[3 * ee + 2] - px + N / 2 + N) & (N - 1);
-                            const float* row = p.x + (static_cast<size_t>(s_meta[3 * ee]) * 3 + c) * NN + sy * N;
-                            v0[q] = ld_ro(row + sx);
-                            v1[q] = ld_ro(row + ((sx - 1) & (N - 1)));
+                            const Img* row = p.x + (static_cast<size_t>(s_meta[3 * ee]) * 3 + c) * NN + sy * N;
+                            v0[q] = load_elem(row + sx);
+                            v1[q] = load_elem(row + ((sx - 1) & (N - 1)));
                         }
 #pragma unroll
                         for (int q = 0; q < 16; ++q) {

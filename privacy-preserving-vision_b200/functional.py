@@ -141,7 +141,7 @@ def nvtx(name):
 # both start together (A/B switch)
 _HOLD_ROWS = 0 if os.environ.get("B200CAM_HOLD_ROWS", "1") == "0" else 1
 # B200CAM_PLANE=1 (opt-in N = 256 plane kernels, read once per process by the library): b200cam_sensor_rows then writes the
-# plane layout, which the bf16 sensor path (default two-pass pipeline only) cannot read
+# plane layout, which the bf16 sensor path and the uint8 image path (default two-pass pipeline only) cannot read
 PLANE_KERNELS = os.environ.get("B200CAM_PLANE", "0")[:1] == "1"
 
 
@@ -155,6 +155,16 @@ def _as_f32(t: torch.Tensor, device: torch.device) -> torch.Tensor:
     if t.dtype != torch.float32:
         raise TypeError(f"b200cam computes in fp32, got {t.dtype}")
     return t.contiguous()
+
+
+def _as_img(t: torch.Tensor, device: torch.device) -> torch.Tensor:
+    """An image batch for the sensor kernels: fp32, or uint8 as it is (converted in the kernels as x * fp32(1/255), bit for
+    bit torch's ``x.float() / 255.0`` on the GPU)."""
+    if t.dtype == torch.uint8:
+        if t.device != device:
+            raise RuntimeError(f"b200cam: tensor on {t.device}, camera tables on {device}")
+        return t.contiguous()
+    return _as_f32(t, device)
 
 
 class PsfSynth(torch.autograd.Function):
@@ -314,19 +324,21 @@ class RowSpectra:
 def sensor_rows(img: torch.Tensor, plan: DevicePlan):
     """Enqueue the row transforms of ``img`` on the current stream (they need no PSF, so `Camera.forward` runs them
     while the PSF chain is busy on the plan's high-priority side stream).
-    Returns None when the split entry points do not apply (empty batch, fused N=256 kernels)."""
+    Returns None when the split entry points do not apply (empty batch, fused N=256 kernels).
+    ``img`` is fp32 or uint8; a uint8 batch is read by the row kernel as it is (not with ``B200CAM_PLANE=1`` at N = 256:
+    the finish call would then expect the plane layout, which only the fp32 row pass writes)."""
     N = plan.N
     _check_img(img, N)
     B = img.shape[0]
     if B == 0 or not plan.lib.b200cam_sensor_split_supported(N, B):
         return None
-    x = _as_f32(img.detach(), plan.device)
+    x = _as_img(img.detach(), plan.device)
     spectrum = torch.empty(plan.lib.b200cam_spectrum_bytes(N, B) // 4, dtype=torch.float32, device=plan.device)
     img_max = torch.empty(B, dtype=torch.float32, device=plan.device)
     tie_count = torch.empty(B, dtype=torch.int32, device=plan.device)
+    rows_fn = plan.lib.b200cam_sensor_rows_u8 if x.dtype == torch.uint8 else plan.lib.b200cam_sensor_rows
     with torch.cuda.device(plan.index):
-        _lib.check(plan.lib.b200cam_sensor_rows(_lib.ptr(x), _lib.ptr(spectrum), _lib.ptr(img_max), _lib.ptr(tie_count),
-                                                B, N, _stream()))
+        _lib.check(rows_fn(_lib.ptr(x), _lib.ptr(spectrum), _lib.ptr(img_max), _lib.ptr(tie_count), B, N, _stream()))
     return RowSpectra(x, spectrum, img_max, tie_count)
 
 
@@ -339,7 +351,9 @@ class SensorConv(torch.autograd.Function):
         noise + quantisation of include/b200cam.h (B200CAM_SENSOR_NOISE / _QUANT); straight-through in backward.
         `out_dtype` torch.bfloat16: the sensor image is written in bf16 (the fp32 result rounded to nearest-even, i.e.
         exactly ``fp32_result.to(torch.bfloat16)``) and the bf16 upstream gradient is read by the kernels as it is; the
-        un-normalised fp32 image is a scratch buffer of the forward and is not kept."""
+        un-normalised fp32 image is a scratch buffer of the forward and is not kept.
+        `img` fp32 or uint8: a uint8 batch is read by the kernels as it is (x * fp32(1/255) in registers, bit for bit the fp32
+        call on ``img.float() / 255.0``) and the node saves it as it is; uint8 is not differentiable, so no dL/dimg."""
         N = plan.N
         flags, noise_t, noise_scale, quant_bits = 0, None, 0.0, 0
         if epilogue is not None:
@@ -352,12 +366,13 @@ class SensorConv(torch.autograd.Function):
             if quant_bits:
                 flags |= 2
         _check_img(img, N)
-        x = rows.x if rows is not None else _as_f32(img.detach(), plan.device)
+        x = rows.x if rows is not None else _as_img(img.detach(), plan.device)
         p = _as_f32(psf.detach(), plan.device).reshape(3, N, N)
         B = x.shape[0]
         bf16 = out_dtype == torch.bfloat16
+        u8 = x.dtype == torch.uint8
         # bf16: `sensor` is the fp32 conv scratch (dropped after the forward), `out` the bf16 image handed downstream
-        sensor = torch.empty_like(x)
+        sensor = torch.empty(x.shape, dtype=torch.float32, device=x.device)
         out = torch.empty(x.shape, dtype=torch.bfloat16, device=x.device) if bf16 else sensor
         img_max = rows.img_max if rows is not None else torch.empty(B, dtype=torch.float32, device=plan.device)
         tie_count = rows.tie_count if rows is not None else torch.empty(B, dtype=torch.int32, device=plan.device)
@@ -391,12 +406,14 @@ class SensorConv(torch.autograd.Function):
             ws = plan.sensor_workspace(B)
             with torch.cuda.device(plan.index):
                 if bf16:
-                    _lib.check(plan.lib.b200cam_sensor_fwd_bf16(
+                    fwd = plan.lib.b200cam_sensor_fwd_u8_bf16 if u8 else plan.lib.b200cam_sensor_fwd_bf16
+                    _lib.check(fwd(
                         _lib.ptr(x), _lib.ptr(p), _lib.ptr(sensor), _lib.ptr(out), _lib.ptr(img_max), _lib.ptr(tie_count),
                         _lib.ptr(tie_pos), _lib.ptr(otf), _lib.ptr(spectrum), _lib.ptr(ws), ws.numel(), B, N, _stream(),
                         flags, _lib.ptr(noise_t), float(noise_scale), int(quant_bits)))
                 else:
-                    _lib.check(plan.lib.b200cam_sensor_fwd_ex(
+                    fwd = plan.lib.b200cam_sensor_fwd_u8 if u8 else plan.lib.b200cam_sensor_fwd_ex
+                    _lib.check(fwd(
                         _lib.ptr(x), _lib.ptr(p), _lib.ptr(sensor), _lib.ptr(img_max), _lib.ptr(tie_count),
                         _lib.ptr(tie_pos), _lib.ptr(otf), _lib.ptr(spectrum), _lib.ptr(ws), ws.numel(), B, N, _stream(),
                         flags, _lib.ptr(noise_t), float(noise_scale), int(quant_bits)))
@@ -405,7 +422,7 @@ class SensorConv(torch.autograd.Function):
         ctx.plan = plan
         ctx.psf_shape = psf.shape
         ctx.spectrum = spectrum
-        # the bf16 node keeps no image-sized fp32 sensor tensor (no backward kernel reads it)
+        # the bf16 node keeps no image-sized fp32 sensor tensor (no backward kernel reads it); a uint8 batch is kept as uint8
         ctx.save_for_backward(x, p, None if bf16 else sensor, img_max, tie_count, tie_pos, otf)
         return out
 
@@ -419,22 +436,25 @@ class SensorConv(torch.autograd.Function):
         want_img = ctx.needs_input_grad[0]
         # the kernels overwrite every element of grad_psf; only the empty batch needs explicit zeros
         grad_psf = (torch.empty if B > 0 else torch.zeros)(3, N, N, dtype=torch.float32, device=plan.device)
-        grad_img = torch.empty_like(x) if want_img else None
+        grad_img = torch.empty_like(x) if want_img else None      # (never for uint8 images: not differentiable)
+        u8 = x.dtype == torch.uint8
         if B > 0 and g.dtype == torch.bfloat16:
             if g.device != plan.device:
                 raise RuntimeError(f"b200cam: tensor on {g.device}, camera tables on {plan.device}")
             gc = g.contiguous()
             ws = plan.sensor_workspace(B)
+            bwd = plan.lib.b200cam_sensor_bwd_u8_bf16 if u8 else plan.lib.b200cam_sensor_bwd_bf16
             with torch.cuda.device(plan.index):
-                _lib.check(plan.lib.b200cam_sensor_bwd_bf16(
+                _lib.check(bwd(
                     _lib.ptr(gc), _lib.ptr(x), _lib.ptr(img_max), _lib.ptr(tie_count), _lib.ptr(tie_pos), _lib.ptr(p),
                     _lib.ptr(otf), _lib.ptr(ctx.spectrum), _lib.ptr(grad_psf), _lib.ptr(grad_img),
                     _lib.ptr(ws), ws.numel(), B, N, _stream()))
         elif B > 0:
             gc = _as_f32(g, plan.device)
             ws = plan.sensor_workspace(B)
+            bwd = plan.lib.b200cam_sensor_bwd_u8 if u8 else plan.lib.b200cam_sensor_bwd
             with torch.cuda.device(plan.index):
-                _lib.check(plan.lib.b200cam_sensor_bwd(
+                _lib.check(bwd(
                     _lib.ptr(gc), _lib.ptr(x), _lib.ptr(sensor), _lib.ptr(img_max), _lib.ptr(tie_count),
                     _lib.ptr(tie_pos), _lib.ptr(p), _lib.ptr(otf), _lib.ptr(ctx.spectrum), _lib.ptr(grad_psf),
                     _lib.ptr(grad_img),

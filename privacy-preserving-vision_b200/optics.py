@@ -163,9 +163,12 @@ class Camera(nn.Module):
         torch.randn when `sensor_noise_sigma > 0` and none is given).  The sensor image is returned in `sensor_dtype`."""
         out_dtype = F.check_sensor_dtype(self.sensor_dtype)
         # uint8 images (what a decoder produces; the reference's loader turns them into fp32 in [0,1] with ToTensor on the
-        # host, Face-DeId/core/data_loader.py:118-124) may be passed as they are: the division by 255 then happens on the
-        # GPU and the host->device copy is a quarter of the fp32 one.
-        if torch.is_tensor(img) and img.dtype == torch.uint8 and img.is_cuda:
+        # host, Face-DeId/core/data_loader.py:118-124) may be passed as they are: the sensor kernels read the bytes and convert
+        # them in registers as x * fp32(1/255), bit for bit torch's x.float() / 255.0 on the GPU - no fp32 copy of the batch is
+        # made or kept for the backward, and the host->device copy is a quarter of the fp32 one.  Only the opt-in plane kernels
+        # (B200CAM_PLANE=1 at N = 256) read fp32 images alone: there the batch is converted with that torch expression.
+        if (torch.is_tensor(img) and img.dtype == torch.uint8 and img.is_cuda and self.N == 256 and F.PLANE_KERNELS
+                and out_dtype == torch.float32):
             img = img.to(torch.float32).div_(255.0)
         # The PSF synthesis is a chain of small latency-bound kernels and the row transforms of the images do not
         # depend on it: put the chain on a high-priority side stream, run the row pass on the current stream meanwhile
@@ -181,7 +184,8 @@ class Camera(nn.Module):
         plan = self._plan(img.device)
         side = plan.side_stream()
         psf = self.get_psf(_stream=side)                       # enqueued on `side`, not joined yet
-        # (the bf16 read-out runs the default pipeline only: not the plane layout that sensor_rows writes with B200CAM_PLANE=1)
+        # (the bf16 read-out runs the default pipeline only: not the plane layout that sensor_rows writes with B200CAM_PLANE=1;
+        # a uint8 batch reaches this point at N = 256 with B200CAM_PLANE=1 only with bf16, see above)
         split = psf.device == img.device and not (out_dtype == torch.bfloat16 and self.N == 256 and F.PLANE_KERNELS)
         rows = F.sensor_rows(img, plan) if split else None
         cur = torch.cuda.current_stream(psf.device)
