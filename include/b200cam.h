@@ -185,12 +185,33 @@ int b200cam_sensor_finish(const float* psf, float* sensor, float* img_max, int* 
  * no live sensor noise and no quantiser (its gaussian_noise call is commented out: Image_Caption/Camera/Lens.py:295-301,
  * Utils.py:300-302; Face-DeId has none), so flags = 0 reproduces it.  With flags:
  *     y = conv / max;   NOISE: y += noise_scale * noise[b][c][y][x];   QUANT: y = round(clamp(y, 0, 1) * L) / L,  L = 2^quant_bits - 1
- * `noise` is a caller-supplied standard-normal tensor shaped like the images (draw it with the framework's seeded generator;
- * a fused Philox could not reproduce torch's stream).  b200cam_sensor_bwd treats the epilogue as the identity (straight
- * through).  Same arguments / reference lines as the calls without _ex.  The Image_Caption camera applies the same epilogue
- * through b200cam_lens_normalise_ex (below). */
+ * With NOISE, `noise` is a caller-supplied standard-normal tensor shaped like the images (drawn with the framework's seeded
+ * generator, e.g. torch.randn: no kernel reproduces that stream).  b200cam_sensor_bwd treats the epilogue as the identity
+ * (straight through).  Same arguments / reference lines as the calls without _ex.  The Image_Caption camera applies the same
+ * epilogue through b200cam_lens_normalise_ex (below).
+ *
+ * NOISE_PHILOX (instead of NOISE, not with it): the kernels draw the standard normals themselves, so no noise tensor is
+ * written and read back.  `noise` is then the DEVICE address (8-byte aligned) of a struct b200cam_noise_seed, read by the
+ * kernels when they run (a CUDA graph replay sees whatever key the block holds by then); noise_scale must be > 0.  The value
+ * added to element e of the call's [B][3][N][N] batch (flat index) is n(e) below, bit for bit what b200cam_sensor_noise writes
+ * for that e, added with the arithmetic of NOISE: the output equals the NOISE call on the materialised tensor.
+ *   Philox4x32-10 (Random123 / cuRAND constants), key = (lo32(key), hi32(key)), counter = (lo32(j), hi32(j), 0, 0) with
+ *   j = first4 + e / 4; its four words x_0..x_3 serve e % 4 = 0..3:
+ *     u_k = (2 (x_k >> 9) + 1) 2^-24        (exact in fp32, in [2^-24, 1 - 2^-24])
+ *     n_0 = r cospi(2 u_1), n_1 = r sinpi(2 u_1), r = sqrt(-2 log u_0);  n_2, n_3 the same from (u_2, u_3)   (Box-Muller)
+ *   so |n| <= sqrt(48 ln 2) = 5.77: the normal tail beyond that (probability ~1e-8) is cut off.  A value depends only on (key,
+ *   first4 + e / 4): a batch split into shards, each with first4 advanced by the float4s before it, gives the whole batch's
+ *   noise.  Not torch.randn's stream. */
 #define B200CAM_SENSOR_NOISE 1
 #define B200CAM_SENSOR_QUANT 2
+#define B200CAM_SENSOR_NOISE_PHILOX 4
+struct b200cam_noise_seed {
+    unsigned long long key;      /* Philox key */
+    unsigned long long first4;   /* counter of the call's first four elements */
+};
+/* The noise of NOISE_PHILOX materialised: out[e] = n(e) for e in [0, count), count % 4 == 0, out 16-byte aligned, seed_block
+ * as above (for tests, and for callers whose read-out does not run in these kernels). */
+int b200cam_sensor_noise(const void* seed_block, float* out, long long count, void* stream);
 int b200cam_sensor_fwd_ex(const float* img, const float* psf, float* sensor, float* img_max, int* tie_count, int* tie_pos,
                           float* otf, float* spectrum, void* workspace, size_t workspace_bytes, int B, int N, void* stream,
                           int flags, const float* noise, float noise_scale, int quant_bits);
@@ -322,8 +343,8 @@ int b200cam_lens_psf_bwd(const double* grad_psf_out, const double* grad_loss, co
  *                               torch's img.float() / 255.0 on the GPU; the padded image still never exists.  The backward is
  *                               the same (it reads the saved spectrum and raw, never the image).
  *   b200cam_lens_normalise_ex   y = |raw| / gmax followed by the opt-in read-out epilogue of b200cam_sensor_fwd_ex
- *                               (flags B200CAM_SENSOR_NOISE / _QUANT, noise [B][3][P][P] indexed like y; flags = 0 is
- *                               b200cam_lens_normalise).  b200cam_lens_sensor_dot / _bwd read raw, not y: straight through.
+ *                               (flags B200CAM_SENSOR_NOISE / _QUANT, noise [B][3][P][P] indexed like y, or _NOISE_PHILOX with
+ *                               e the flat index into y; flags = 0 is b200cam_lens_normalise).  b200cam_lens_sensor_dot / _bwd read raw, not y: straight through.
  * bf16 variants (a downstream network in bf16): same arguments and checks, y / grad_y as bf16 bit patterns.
  *   b200cam_lens_normalise_bf16   b200cam_lens_normalise_ex rounded to nearest-even as the last step (= its output cast with
  *                                 torch); b200cam_lens_sensor_dot_bf16 / _bwd_bf16 read grad_y in bf16, widened exactly, and

@@ -66,7 +66,9 @@ _SIGNATURES = {
     "b200cam_sensor_finish_ex": (ctypes.c_int, [_f, _f, _f, _f, _f, _f, _f, ctypes.c_int,
                                                 _f, ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_void_p,
                                                 ctypes.c_int, _f, ctypes.c_float, ctypes.c_int]),
-    "b200cam_sensor_split_supported": (ctypes.c_int, [ctypes.c_int, ctypes.c_int]),
+    # the Philox read-out's noise materialised (seed block: device address of {key, first4})
+    "b200cam_sensor_noise": (ctypes.c_int, [ctypes.c_void_p, _f, ctypes.c_longlong, ctypes.c_void_p]),
+    "b200cam_sensor_split_supported":(ctypes.c_int, [ctypes.c_int, ctypes.c_int]),
     "b200cam_sensor_rows": (ctypes.c_int, [_f, _f, _f, _f, ctypes.c_int, ctypes.c_int, ctypes.c_void_p]),
     "b200cam_psf_otf": (ctypes.c_int, [_f, _f, ctypes.c_int, ctypes.c_void_p]),
     "b200cam_sensor_finish": (ctypes.c_int, [_f, _f, _f, _f, _f, _f, _f, ctypes.c_int,

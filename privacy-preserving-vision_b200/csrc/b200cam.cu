@@ -82,6 +82,21 @@ __global__ void __launch_bounds__(EW_THREADS) k_normalise_bf16(NormaliseParams p
     DeviceExec ex;
     normalise_body<bf16>(ex, p, gridDim.x, out);
 }
+// the same two with the Philox read-out (p.epi.seed): the noise is drawn in the kernel, no tensor is read
+__global__ void __launch_bounds__(EW_THREADS) k_normalise_philox(NormaliseParams p) {
+    pdl_gate();
+    DeviceExec ex;
+    normalise_body<float, true>(ex, p, gridDim.x);
+}
+__global__ void __launch_bounds__(EW_THREADS) k_normalise_bf16_philox(NormaliseParams p, bf16* out) {
+    pdl_gate();
+    DeviceExec ex;
+    normalise_body<bf16, true>(ex, p, gridDim.x, out);
+}
+__global__ void __launch_bounds__(EW_THREADS) k_philox_noise(const b200cam_noise_seed* seed, float* out, long long n4) {
+    DeviceExec ex;
+    philox_noise_body(ex, seed, out, n4, gridDim.x);
+}
 template <int N>
 __global__ void __launch_bounds__(ColsSmem<N>::THREADS, N <= 256 ? 3 : 1) k_cols_accum(ColsAccumParams p) {
     pdl_gate();
@@ -1103,7 +1118,8 @@ static int sensor_finish_impl(const float* psf, float* sensor, float* img_max, i
     }
     const int planes = 3 * B;
     if constexpr (N == 256) {
-        if (allow_plane && out16 == nullptr && plane_selected() && epi.noise == nullptr && epi.levels <= 0.f) {   // (the opt-in plane kernels have no read-out epilogue)
+        if (allow_plane && out16 == nullptr && plane_selected() && epi.noise == nullptr && epi.seed == nullptr &&
+            epi.levels <= 0.f) {   // (the opt-in plane kernels have no read-out epilogue)
             const DeviceState* st = cur_state();
             if (st == nullptr || st->pconv_g3 < 1) return B200CAM_E_NOT_INIT;
             const int G3 = B < st->pconv_g3 ? B : st->pconv_g3;
@@ -1125,7 +1141,8 @@ static int sensor_finish_impl(const float* psf, float* sensor, float* img_max, i
     // previous tile's outputs (128 registers / thread at 4 CTAs per SM) that costs the time, not the waiting.
     static const int one_pass = [] { const char* e = getenv("B200CAM_ONE_PASS"); return e ? atoi(e) : 0; }();
     constexpr bool FUSABLE = (Plan<N>::R1 <= 16) && (Plan<N>::LANES == Plan<N>::R2);
-    const bool fused = FUSABLE && one_pass && per_sm > 0 && out16 == nullptr;
+    // (the one-pass kernel reads a noise tensor only: the Philox read-out runs in the normalise kernel)
+    const bool fused = FUSABLE && one_pass && per_sm > 0 && out16 == nullptr && epi.seed == nullptr;
     launch_k(k_cols_conv<N>, dim3(colgroups, nchunks), ColsSmem<N>::THREADS, ColsSmem<N>::BYTES_CONV, s, 
         ColsConvParams{srow, ws.st2, otf, tw, nullptr, B, nchunks, 0, 1.0f, fused ? ws.arrive : nullptr, fused ? 64 * B : 0});
     LAUNCH_CHECK();
@@ -1153,10 +1170,11 @@ static int sensor_finish_impl(const float* psf, float* sensor, float* img_max, i
     LAUNCH_CHECK();
     const long long n4 = static_cast<long long>(planes) * N * N / 4;
     const int grid = static_cast<int>(n4 / EW_THREADS < 148 * 8 ? (n4 + EW_THREADS - 1) / EW_THREADS : 148 * 8);
+    const NormaliseParams np{sensor, img_max, tie_count, tie_pos, n4, 3 * N * N / 4, epi};
     if (out16 != nullptr)
-        launch_k(k_normalise_bf16, grid, EW_THREADS, 0, s, NormaliseParams{sensor, img_max, tie_count, tie_pos, n4, 3 * N * N / 4, epi}, out16);
+        launch_k(epi.seed != nullptr ? k_normalise_bf16_philox : k_normalise_bf16, grid, EW_THREADS, 0, s, np, out16);
     else
-        launch_k(k_normalise, grid, EW_THREADS, 0, s, NormaliseParams{sensor, img_max, tie_count, tie_pos, n4, 3 * N * N / 4, epi});
+        launch_k(epi.seed != nullptr ? k_normalise_philox : k_normalise, grid, EW_THREADS, 0, s, np);
     LAUNCH_CHECK();
     return 0;
 }
@@ -1289,7 +1307,8 @@ static int sensor_fwd_impl(const Img* img, const float* psf, float* sensor, floa
     SensorWs ws(ws_ptr, N, B, false);
     float2* srow = spectrum != nullptr ? spectrum : ws.stx;      // row spectra: kept for the backward when asked
     constexpr bool FP32_IMG = std::is_same<Img, float>::value;  // (uint8 images: standard layout, no plane kernels)
-    int rc = sensor_rows_impl<N, Img>(img, srow, img_max, tie_count, B, s, out16 == nullptr);
+    // (bf16 and the Philox read-out run the default pipeline: the rows in the standard layout)
+    int rc = sensor_rows_impl<N, Img>(img, srow, img_max, tie_count, B, s, out16 == nullptr && epi.seed == nullptr);
     if (rc) return rc;
     return sensor_finish_impl<N>(psf, sensor, img_max, tie_count, tie_pos, otf, srow, ws, B, 0, s, epi, out16, FP32_IMG);
 }
@@ -1888,6 +1907,7 @@ int b200cam_sensor_finish_ex(const float* psf, float* sensor, float* img_max, in
     SensorEpilogue epi;
     if (const int rc = make_epilogue(flags, noise, noise_scale, quant_bits, &epi)) return rc;
     if (!b200cam_supported(N) || B < 1) return B200CAM_E_BAD_SIZE;
+    if (epi.seed != nullptr && N == 256 && plane_selected()) return B200CAM_E_BAD_SIZE;   // rows in the plane layout
     if (!psf || !sensor || !img_max || !tie_count || !tie_pos || !otf || !spectrum || !workspace) return B200CAM_E_NULL;
     if (workspace_bytes < b200cam_sensor_workspace_bytes(N, B, 0)) return B200CAM_E_WORKSPACE;
     if (!aligned16(sensor) || !aligned16(otf) || !aligned16(workspace) || !aligned16(psf) || !aligned16(spectrum))
@@ -1897,6 +1917,20 @@ int b200cam_sensor_finish_ex(const float* psf, float* sensor, float* img_max, in
     DISPATCH_N(N, (sensor_finish_impl<NN_>(psf, sensor, img_max, tie_count, tie_pos, reinterpret_cast<float2*>(otf),
                                            reinterpret_cast<const float2*>(spectrum), SensorWs(workspace, NN_, B, false),
                                            B, otf_ready, s, epi)));
+}
+
+// the noise of B200CAM_SENSOR_NOISE_PHILOX, materialised; the seed block is checked as make_epilogue checks it
+int b200cam_sensor_noise(const void* seed_block, float* out, long long count, void* stream) {
+    if (seed_block == nullptr || out == nullptr) return B200CAM_E_NULL;
+    if (count < 0 || count % 4 != 0) return B200CAM_E_BAD_SIZE;
+    if (reinterpret_cast<uintptr_t>(seed_block) % 8 != 0 || !aligned16(out)) return B200CAM_E_ALIGN;
+    if (count == 0) return 0;
+    const long long n4 = count / 4;
+    const int grid = static_cast<int>(n4 / EW_THREADS < 148 * 8 ? (n4 + EW_THREADS - 1) / EW_THREADS : 148 * 8);
+    launch_k(k_philox_noise, grid, EW_THREADS, 0, static_cast<cudaStream_t>(stream),
+             static_cast<const b200cam_noise_seed*>(seed_block), out, n4);
+    LAUNCH_CHECK();
+    return 0;
 }
 
 int b200cam_conv_fwd(const float* img, const float* kernel, float* out, float* otf, float* spectrum, void* workspace,

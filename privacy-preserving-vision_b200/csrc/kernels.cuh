@@ -462,29 +462,113 @@ constexpr int C2R_MAX_TIES = 8;     // = MAX_TIES (declared with the normalise k
 // Face-DeId `Camera`: applied where the sensor kernels write y (one-pass inverse rows, normalise kernel; b200cam.cu);
 // Image_Caption `OpticsZernike`: in the normalise kernel of lens_conv.cu, after the batch-global maximum.
 // `noise` is a caller-supplied N(0,1) tensor shaped like the image batch (drawn with torch's generator, so a run is
-// reproducible against the oracle); L = 2^bits - 1.  The backward is straight through (dL/dconv as if the epilogue
-// were the identity), the usual treatment of a quantiser.
+// reproducible against the oracle); L = 2^bits - 1.  Or `seed` (B200CAM_SENSOR_NOISE_PHILOX): the element-wise kernels draw
+// the normals with philox_normal4 below instead of reading a tensor - their own instantiations, which add them through
+// add_noise / quantise exactly as apply_epilogue adds a tensor's values.  The backward is straight through (dL/dconv as if
+// the epilogue were the identity), the usual treatment of a quantiser.
 struct SensorEpilogue {
     const float* noise;      // nullable
     float noise_scale;
     float levels;            // <= 0: no quantisation
+    const b200cam_noise_seed* seed;   // nullable; set: the Philox read-out (noise == nullptr then)
 };
-B200_HD float apply_epilogue(const SensorEpilogue& e, float y, size_t idx) {
-    if (e.noise != nullptr) y += e.noise_scale * ld_ro(e.noise + idx);
+B200_HD float add_noise(const SensorEpilogue& e, float y, float n) { return y + e.noise_scale * n; }
+B200_HD float quantise(const SensorEpilogue& e, float y) {
     if (e.levels > 0.f) {
         y = fminf(fmaxf(y, 0.f), 1.f);
         y = rintf(y * e.levels) / e.levels;
     }
     return y;
 }
+B200_HD float apply_epilogue(const SensorEpilogue& e, float y, size_t idx) {
+    if (e.noise != nullptr) y = add_noise(e, y, ld_ro(e.noise + idx));
+    return quantise(e, y);
+}
+
+// ---- the sensor noise of B200CAM_SENSOR_NOISE_PHILOX (include/b200cam.h): Philox4x32-10 + Box-Muller ------------------------
+// One counter j gives the standard normals of the four elements 4j'..4j'+3 of the call's batch, j = first4 + j'.  Every kernel
+// that draws them (the normalise kernels of both cameras, the materialiser) calls philox_normal4, so the fused read-out and the
+// materialised tensor agree bit for bit.
+struct Normal4 { float n[4]; };
+B200_HD uint32_t mulhi32(uint32_t a, uint32_t b) {
+#if defined(__CUDA_ARCH__)
+    return __umulhi(a, b);
+#else
+    return static_cast<uint32_t>((static_cast<uint64_t>(a) * b) >> 32);
+#endif
+}
+// Philox4x32-10 of Random123 (the cuRAND constants): 10 rounds, the key bumped between rounds
+B200_HD void philox4x32_10(uint32_t (&c)[4], uint32_t k0, uint32_t k1) {
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        if (r > 0) {
+            k0 += 0x9E3779B9u;
+            k1 += 0xBB67AE85u;
+        }
+        const uint32_t hi0 = mulhi32(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
+        const uint32_t hi1 = mulhi32(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
+        const uint32_t c1 = c[1], c3 = c[3];
+        c[0] = hi1 ^ c1 ^ k0;
+        c[1] = lo1;
+        c[2] = hi0 ^ c3 ^ k1;
+        c[3] = lo0;
+    }
+}
+// sin(pi x), cos(pi x).  Host (emulator): computed in double and rounded - host and device values are not compared.
+B200_HD void sincospi_f(float x, float* s, float* c) {
+#if defined(__CUDA_ARCH__)
+    sincospif(x, s, c);
+#else
+    const double a = M_PI * static_cast<double>(x);
+    *s = static_cast<float>(sin(a));
+    *c = static_cast<float>(cos(a));
+#endif
+}
+// (2 (x >> 9) + 1) 2^-24: a 24-bit odd integer times a power of two, exact; never 0 or 1
+B200_HD float philox_uniform(uint32_t x) { return static_cast<float>(2u * (x >> 9) + 1u) * 5.9604644775390625e-8f; }
+B200_HD void box_muller(float u0, float u1, float* n0, float* n1) {
+    const float r = sqrtf(-2.0f * logf(u0));
+    float s, c;
+    sincospi_f(2.0f * u1, &s, &c);
+#if defined(__CUDA_ARCH__)
+    *n0 = __fmul_rn(r, c);          // (no contraction into the caller's noise_scale * n + y)
+    *n1 = __fmul_rn(r, s);
+#else
+    *n0 = r * c;
+    *n1 = r * s;
+#endif
+}
+B200_HD Normal4 philox_normal4(unsigned long long key, unsigned long long j) {
+    uint32_t c[4] = {static_cast<uint32_t>(j), static_cast<uint32_t>(j >> 32), 0u, 0u};
+    philox4x32_10(c, static_cast<uint32_t>(key), static_cast<uint32_t>(key >> 32));
+    Normal4 o;
+    box_muller(philox_uniform(c[0]), philox_uniform(c[1]), &o.n[0], &o.n[1]);
+    box_muller(philox_uniform(c[2]), philox_uniform(c[3]), &o.n[2], &o.n[3]);
+    return o;
+}
+// the seed block as the kernels read it (device memory, so that a graph replay sees the key drawn in that replay)
+struct NoiseSeed { unsigned long long key, first4; };
+B200_HD NoiseSeed load_seed(const b200cam_noise_seed* s) {
+    const unsigned long long* w = reinterpret_cast<const unsigned long long*>(s);
+    return NoiseSeed{ld_ro(w), ld_ro(w + 1)};
+}
+
 // Validates the (flags, noise, noise_scale, quant_bits) arguments of the _ex entry points of both cameras (include/b200cam.h)
 // and builds the epilogue they select; host side, before anything is enqueued.
 inline int make_epilogue(int flags, const float* noise, float noise_scale, int quant_bits, SensorEpilogue* epi) {
-    *epi = SensorEpilogue{nullptr, 0.f, 0.f};
-    if (flags & ~(B200CAM_SENSOR_NOISE | B200CAM_SENSOR_QUANT)) return B200CAM_E_BAD_SIZE;
+    *epi = SensorEpilogue{nullptr, 0.f, 0.f, nullptr};
+    if (flags & ~(B200CAM_SENSOR_NOISE | B200CAM_SENSOR_QUANT | B200CAM_SENSOR_NOISE_PHILOX)) return B200CAM_E_BAD_SIZE;
+    if ((flags & B200CAM_SENSOR_NOISE) && (flags & B200CAM_SENSOR_NOISE_PHILOX)) return B200CAM_E_BAD_SIZE;
     if (flags & B200CAM_SENSOR_NOISE) {
         if (noise == nullptr) return B200CAM_E_NULL;
         epi->noise = noise;
+        epi->noise_scale = noise_scale;
+    }
+    if (flags & B200CAM_SENSOR_NOISE_PHILOX) {
+        if (!(noise_scale > 0.f)) return B200CAM_E_BAD_SIZE;      // a zero-amplitude draw: ask for no noise instead
+        if (noise == nullptr) return B200CAM_E_NULL;
+        if (reinterpret_cast<uintptr_t>(noise) % 8 != 0) return B200CAM_E_ALIGN;
+        epi->seed = reinterpret_cast<const b200cam_noise_seed*>(noise);
         epi->noise_scale = noise_scale;
     }
     if (flags & B200CAM_SENSOR_QUANT) {
@@ -852,10 +936,13 @@ struct NormaliseParams {
 // Out = float: in place, p.y holds conv on entry and the sensor image on exit.  Out = bf16: p.y (the fp32 conv) is only
 // read and the sensor image goes to `out`, each value the fp32 result rounded to nearest-even as the very last step (after
 // the tie recording and the epilogue), i.e. exactly the fp32 image cast with torch.
-template <class Out = float, class Exec>
+// PHILOX: the Philox read-out (p.epi.seed): one philox_normal4 per float4, counter first4 + the float4's index in the batch.
+template <class Out = float, bool PHILOX = false, class Exec>
 B200_HD void normalise_body(Exec& ex, const NormaliseParams& p, int grid_x, Out* out = nullptr) {
     ex.phase([&](int tid) {
         constexpr int U = 4;
+        NoiseSeed seed{0ull, 0ull};
+        if constexpr (PHILOX) seed = load_seed(p.epi.seed);
         const int B = static_cast<int>(p.n4 / p.per_image4);
         const int spi = grid_x / B > 1 ? grid_x / B : 1;               // slices per image
         const int nthr = ex.nthreads();
@@ -876,6 +963,8 @@ B200_HD void normalise_body(Exec& ex, const NormaliseParams& p, int grid_x, Out*
                     const int i = i0 + k * stride;
                     if (i >= p.per_image4) continue;
                     float e[4] = {v[k].x, v[k].y, v[k].z, v[k].w};
+                    Normal4 nz{};
+                    if constexpr (PHILOX) nz = philox_normal4(seed.key, seed.first4 + static_cast<unsigned long long>(b) * p.per_image4 + i);
 #pragma unroll
                     for (int q = 0; q < 4; ++q) {
                         if (e[q] == m) {
@@ -885,7 +974,10 @@ B200_HD void normalise_body(Exec& ex, const NormaliseParams& p, int grid_x, Out*
                         } else {
                             e[q] *= inv;
                         }
-                        e[q] = apply_epilogue(p.epi, e[q], (static_cast<size_t>(b) * p.per_image4 + i) * 4 + q);
+                        if constexpr (PHILOX)
+                            e[q] = quantise(p.epi, add_noise(p.epi, e[q], nz.n[q]));
+                        else
+                            e[q] = apply_epilogue(p.epi, e[q], (static_cast<size_t>(b) * p.per_image4 + i) * 4 + q);
                     }
                     if constexpr (sizeof(Out) == sizeof(float))
                         img4[i] = make_float4(e[0], e[1], e[2], e[3]);
@@ -893,6 +985,19 @@ B200_HD void normalise_body(Exec& ex, const NormaliseParams& p, int grid_x, Out*
                         store4(out, static_cast<long long>(b) * p.per_image4 + i, e[0], e[1], e[2], e[3]);
                 }
             }
+        }
+    });
+}
+
+// The noise of the Philox read-out materialised (b200cam_sensor_noise): out[e] = n(e), n4 float4s, 1-D grid-stride
+template <class Exec>
+B200_HD void philox_noise_body(Exec& ex, const b200cam_noise_seed* seed_block, float* out, long long n4, int grid_x) {
+    ex.phase([&](int tid) {
+        const NoiseSeed seed = load_seed(seed_block);
+        const long long stride = static_cast<long long>(grid_x) * ex.nthreads();
+        for (long long i = static_cast<long long>(ex.bx()) * ex.nthreads() + tid; i < n4; i += stride) {
+            const Normal4 nz = philox_normal4(seed.key, seed.first4 + static_cast<unsigned long long>(i));
+            store4(out, i, nz.n[0], nz.n[1], nz.n[2], nz.n[3]);
         }
     });
 }

@@ -334,14 +334,21 @@ __global__ void __launch_bounds__(ColsSmem<N>::THREADS, N <= 512 ? 2 : 1) k_lcol
 // ---- element-wise: y = |raw| / m [-> read-out epilogue] ; partial sums of g * y and the number of positions that attain m -----
 // Out = bf16: the fp32 value rounded to nearest-even as the last step (= the fp32 sensor image cast with torch)
 constexpr int EWT = 256;
-template <bool EPI, class Out = float>
+// PHILOX (with EPI): the Philox read-out (epi.seed), one philox_normal4 per float4 at counter first4 + i
+template <bool EPI, class Out = float, bool PHILOX = false>
 __global__ void __launch_bounds__(EWT) k_lnormalise(const float4* __restrict__ raw, const float* __restrict__ gmax, Out* __restrict__ y, long long n4,
                                                     SensorEpilogue epi) {
     const float m = __ldg(gmax);
+    NoiseSeed seed{0ull, 0ull};
+    if constexpr (PHILOX) seed = load_seed(epi.seed);
     for (long long i = blockIdx.x * static_cast<long long>(EWT) + threadIdx.x; i < n4; i += static_cast<long long>(gridDim.x) * EWT) {
         const float4 v = __ldg(raw + i);
         float4 o = make_float4(fabsf(v.x) / m, fabsf(v.y) / m, fabsf(v.z) / m, fabsf(v.w) / m);
-        if (EPI) {
+        if constexpr (PHILOX) {
+            const Normal4 nz = philox_normal4(seed.key, seed.first4 + static_cast<unsigned long long>(i));
+            o = make_float4(quantise(epi, add_noise(epi, o.x, nz.n[0])), quantise(epi, add_noise(epi, o.y, nz.n[1])),
+                            quantise(epi, add_noise(epi, o.z, nz.n[2])), quantise(epi, add_noise(epi, o.w, nz.n[3])));
+        } else if (EPI) {
             const size_t e = static_cast<size_t>(i) * 4;
             o = make_float4(apply_epilogue(epi, o.x, e), apply_epilogue(epi, o.y, e + 1), apply_epilogue(epi, o.z, e + 2),
                             apply_epilogue(epi, o.w, e + 3));
@@ -556,7 +563,9 @@ static int lens_normalise(const float* raw, const float* gmax, Out* y, long long
     if (count == 0) return 0;
     const auto r4 = reinterpret_cast<const float4*>(raw);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    if (flags)
+    if (epi.seed != nullptr)
+        k_lnormalise<true, Out, true><<<ew_grid(count / 4), EWT, 0, s>>>(r4, gmax, y, count / 4, epi);
+    else if (flags)
         k_lnormalise<true><<<ew_grid(count / 4), EWT, 0, s>>>(r4, gmax, y, count / 4, epi);
     else
         k_lnormalise<false><<<ew_grid(count / 4), EWT, 0, s>>>(r4, gmax, y, count / 4, epi);

@@ -286,16 +286,92 @@ def zernike_project(coef: torch.Tensor, volume: torch.Tensor, plan: DevicePlan) 
     return ZernikeProject.apply(coef, volume, plan)
 
 
-def read_out(img: torch.Tensor, sigma: float, bits: int, noise: torch.Tensor | None = None):
-    """The opt-in sensor read-out of both cameras (``sensor_noise_sigma`` / ``sensor_quant_bits``): (noise tensor, noise scale,
-    quantisation bits) for the kernels' epilogue, or None when it is off (the reference).  With ``sigma > 0`` and no ``noise``
-    given, the noise is drawn here with torch.randn shaped like ``img`` (torch's global generator: seed it to reproduce)."""
+NOISE_RNGS = ("torch", "philox")
+
+
+def check_noise_rng(rng) -> str:
+    """The ``sensor_noise_rng`` module attribute of both cameras: "torch" (default) or "philox"."""
+    if rng not in NOISE_RNGS:
+        raise ValueError(f"sensor_noise_rng must be 'torch' or 'philox', got {rng!r}")
+    return rng
+
+
+def read_out(img: torch.Tensor, sigma: float, bits: int, noise: torch.Tensor | None = None, rng: str = "torch",
+             first4: int = 0):
+    """The opt-in sensor read-out of both cameras (``sensor_noise_sigma`` / ``sensor_quant_bits``): (noise, noise scale,
+    quantisation bits) for the kernels' epilogue, or None when it is off (the reference).  A ``noise`` tensor given by the
+    caller is used as it is.  Otherwise, with ``sigma > 0``:
+    * ``rng="torch"``: the noise is drawn here with torch.randn shaped like ``img`` (torch's global generator: seed it to
+      reproduce);
+    * ``rng="philox"``: only a key is drawn here, with one torch.randint on the image's device (torch's generator, so seeded
+      runs repeat and a CUDA graph draws a new key on every replay), and "noise" is the (2,) int64 seed block {key, first4}
+      of include/b200cam.h (B200CAM_SENSOR_NOISE_PHILOX): the kernels draw the normals themselves.  ``first4`` is the counter
+      of the batch's first four elements (non-zero for a shard of a larger batch, see :func:`shard_first4`)."""
     sigma, bits = float(sigma), int(bits)
     if noise is None and sigma > 0.0:
-        noise = torch.randn(img.shape, dtype=torch.float32, device=img.device)
+        if rng == "philox":
+            key = torch.randint(2**63 - 1, (1,), dtype=torch.int64, device=img.device)
+            noise = torch.cat((key, torch.full((1,), int(first4), dtype=torch.int64, device=img.device)))
+        else:
+            noise = torch.randn(img.shape, dtype=torch.float32, device=img.device)
     if noise is None and bits == 0:
         return None
     return (noise, sigma if noise is not None else 0.0, bits)
+
+
+def noise_seed(epilogue) -> torch.Tensor | None:
+    """The Philox seed block of a :func:`read_out` result, None when the noise is a tensor or there is none."""
+    if epilogue is None or epilogue[0] is None or epilogue[0].dtype != torch.int64:
+        return None
+    return epilogue[0]
+
+
+def shard_first4(img: torch.Tensor, process_group) -> int:
+    """Philox counter of the first four elements of this rank's shard: rank * (elements per shard) / 4 for a batch sharded
+    in equal parts over ``process_group`` (``data_parallel``), 0 without one.  Ranks seeded alike then draw the noise of the
+    concatenated batch, as one GPU would."""
+    if process_group is None:
+        return 0
+    import torch.distributed as dist
+    if not dist.is_initialized():
+        return 0
+    return dist.get_rank(process_group) * (img.numel() // 4)
+
+
+def philox_normal(seed_block: torch.Tensor, shape) -> torch.Tensor:
+    """The standard normals the kernels draw for ``seed_block`` (the (2,) int64 {key, first4} of a Philox read-out), as an
+    fp32 tensor of ``shape`` (numel % 4 == 0) on its device: b200cam_sensor_noise, bit for bit the values the normalise kernels
+    add.  For tests, and for the geometries whose read-out runs as torch ops."""
+    if seed_block.dtype != torch.int64 or seed_block.numel() != 2 or not seed_block.is_cuda:
+        raise ValueError("seed_block must be a (2,) int64 CUDA tensor {key, first4}")
+    seed = seed_block.contiguous()
+    out = torch.empty(shape, dtype=torch.float32, device=seed.device)
+    lib = _lib.load_library()
+    with torch.cuda.device(seed.device):
+        _lib.check(lib.b200cam_sensor_noise(_lib.ptr(seed), _lib.ptr(out), out.numel(), _stream()))
+    return out
+
+
+def epilogue_flags(epilogue, shape, device: torch.device):
+    """(flags, noise, noise_scale, quant_bits) of the C ABI for a :func:`read_out` result: B200CAM_SENSOR_NOISE with an fp32
+    tensor shaped like the images, B200CAM_SENSOR_NOISE_PHILOX with a seed block, B200CAM_SENSOR_QUANT with bits."""
+    if epilogue is None:
+        return 0, None, 0.0, 0
+    noise, noise_scale, quant_bits = epilogue
+    flags = 0
+    if noise is not None and noise.dtype == torch.int64:
+        if noise.numel() != 2 or noise.device != device:
+            raise ValueError(f"a Philox seed block is a (2,) int64 tensor on {device}")
+        noise = noise.contiguous()
+        flags |= 4
+    elif noise is not None:
+        noise = _as_f32(noise.detach(), device)
+        if tuple(noise.shape) != tuple(shape):
+            raise ValueError(f"sensor noise must have the shape of the images {tuple(shape)}, got {tuple(noise.shape)}")
+        flags |= 1
+    if quant_bits:
+        flags |= 2
+    return flags, noise, noise_scale, quant_bits
 
 
 SENSOR_DTYPES = (torch.float32, torch.bfloat16)
@@ -347,24 +423,16 @@ class SensorConv(torch.autograd.Function):
     @nvtx("b200cam.SensorConv.forward")
     def forward(ctx, img: torch.Tensor, psf: torch.Tensor, plan: DevicePlan, rows: RowSpectra | None = None, epilogue=None,
                 out_dtype: torch.dtype = torch.float32):
-        """`epilogue`: None (the reference's read-out: nothing) or (noise, noise_scale, quant_bits) - the opt-in sensor
-        noise + quantisation of include/b200cam.h (B200CAM_SENSOR_NOISE / _QUANT); straight-through in backward.
+        """`epilogue`: None (the reference's read-out: nothing) or (noise, noise_scale, quant_bits) of `read_out` - the opt-in
+        sensor noise + quantisation of include/b200cam.h (B200CAM_SENSOR_NOISE, or _NOISE_PHILOX when `noise` is a seed block;
+        _QUANT); straight-through in backward.
         `out_dtype` torch.bfloat16: the sensor image is written in bf16 (the fp32 result rounded to nearest-even, i.e.
         exactly ``fp32_result.to(torch.bfloat16)``) and the bf16 upstream gradient is read by the kernels as it is; the
         un-normalised fp32 image is a scratch buffer of the forward and is not kept.
         `img` fp32 or uint8: a uint8 batch is read by the kernels as it is (x * fp32(1/255) in registers, bit for bit the fp32
         call on ``img.float() / 255.0``) and the node saves it as it is; uint8 is not differentiable, so no dL/dimg."""
         N = plan.N
-        flags, noise_t, noise_scale, quant_bits = 0, None, 0.0, 0
-        if epilogue is not None:
-            noise_t, noise_scale, quant_bits = epilogue
-            if noise_t is not None:
-                noise_t = _as_f32(noise_t.detach(), plan.device)
-                if noise_t.shape != img.shape:
-                    raise ValueError(f"sensor noise must have the shape of the images {tuple(img.shape)}, got {tuple(noise_t.shape)}")
-                flags |= 1
-            if quant_bits:
-                flags |= 2
+        flags, noise_t, noise_scale, quant_bits = epilogue_flags(epilogue, img.shape, plan.device)
         _check_img(img, N)
         x = rows.x if rows is not None else _as_img(img.detach(), plan.device)
         p = _as_f32(psf.detach(), plan.device).reshape(3, N, N)

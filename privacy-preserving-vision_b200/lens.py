@@ -27,7 +27,9 @@ Read-out (no reference counterpart, same meaning as on the Face-DeId ``Camera``)
   y = round(clamp(y, 0, 1) * L) / L, L = 2^bits - 1, applied after the batch-global max by the normalise kernel
   (``b200cam_lens_normalise_ex``; the torch expression elsewhere), straight through in backward.  ``forward(..., noise=)``
   takes the standard-normal tensor; otherwise it is drawn with ``torch.randn`` after the lens tolerance field.  With
-  ``data_parallel`` each rank draws the noise of its own shard;
+  ``data_parallel`` each rank draws the noise of its own shard.  ``sensor_noise_rng = "philox"``: a key is drawn there instead
+  and the normalise kernel draws the noise (``b200cam_lens_normalise_ex`` with ``B200CAM_SENSOR_NOISE_PHILOX``; the other
+  geometries use its materialised values, ``F.philox_normal``); sharded batches then get the one-GPU noise;
 * ``sensor_dtype`` (default torch.float32): torch.bfloat16 returns the sensor image in bf16 for a bf16 encoder - the normalise
   kernel rounds the fp32 result to nearest-even (``b200cam_lens_normalise_bf16``) and the backward reads the bf16 gradient as it
   is (``_dot_bf16`` / ``_bwd_bf16``); the other geometries cast with torch.  Bit for bit the fp32 module followed by
@@ -208,16 +210,7 @@ class LensSensor(torch.autograd.Function):
             x, fwd = F._as_f32(img.detach(), dev), lib.b200cam_lens_sensor_fwd
         k = F._as_f32(kpad.detach(), dev).reshape(3, n, n)
         B = x.shape[0]
-        flags, noise, noise_scale, quant_bits = 0, None, 0.0, 0
-        if epilogue is not None:
-            noise, noise_scale, quant_bits = epilogue
-            if noise is not None:
-                noise = F._as_f32(noise.detach(), dev)
-                if noise.shape != x.shape:
-                    raise ValueError(f"sensor noise must have the shape of the images {tuple(x.shape)}, got {tuple(noise.shape)}")
-                flags |= 1
-            if quant_bits:
-                flags |= 2
+        flags, noise, noise_scale, quant_bits = F.epilogue_flags(epilogue, x.shape, dev)
         raw = torch.empty(x.shape, dtype=torch.float32, device=dev)
         bf16 = out_dtype == torch.bfloat16
         y = torch.empty(x.shape, dtype=out_dtype, device=dev)
@@ -381,7 +374,11 @@ class OpticsZernike(nn.Module):
         # encoder that runs in bf16 - exactly the fp32 image .to(torch.bfloat16), written by the normalise kernel; backward =
         # the fp32 one on g.float().  PSF, coefficients, loss and dL/dimg keep their dtypes.  Set by the caller.
         self.sensor_dtype = torch.float32
-        self._const: dict = {}            # per-device constant tables (wavefront, aperture, transfer function)
+        # generator of the opt-in sensor noise, as on Camera: "torch" (torch.randn tensor) or "philox" (drawn in the normalise
+        # kernel from a key drawn with torch.randint; the key of the last forward is `sensor_noise_seed`)
+        self.sensor_noise_rng = "torch"
+        self.sensor_noise_seed = None
+        self._const: dict = {}           # per-device constant tables (wavefront, aperture, transfer function)
         self._plans: dict = {}
         self._process_group = None
 
@@ -599,11 +596,14 @@ class OpticsZernike(nn.Module):
     @staticmethod
     def _read_out_torch(y: torch.Tensor, epilogue) -> torch.Tensor:
         """The read-out epilogue of the kernels (kernels.cuh apply_epilogue) as torch ops, straight through in backward - for
-        the geometries the fused kernels do not cover."""
+        the geometries the fused kernels do not cover.  A Philox seed block is materialised with ``F.philox_normal``: the values the
+        fused normalise kernel would draw for it."""
         if epilogue is None:
             return y
         noise, sigma, bits = epilogue
         z = y
+        if noise is not None and noise.dtype == torch.int64:
+            noise = F.philox_normal(noise, y.shape)
         if noise is not None:
             if noise.shape != y.shape:
                 raise ValueError(f"sensor noise must have the shape of the images {tuple(y.shape)}, got {tuple(noise.shape)}")
@@ -634,8 +634,10 @@ class OpticsZernike(nn.Module):
         HDF5 store yields; read as input_img / 255.0 on the GPU, a quarter of the host-to-device bytes).  ``noise``: optional
         standard-normal tensor shaped like the batch for the opt-in sensor noise (``sensor_noise_sigma``); with sigma > 0 and
         none given it is drawn with torch.randn AFTER the lens tolerance field, so a seeded run draws both in the same order.
-        The sensor image is returned in ``sensor_dtype``."""
+        The sensor image is returned in ``sensor_dtype``.  With ``sensor_noise_rng = "philox"`` a key is drawn at that point
+        instead and the normalise kernel draws the noise (``sensor_noise_seed``)."""
         out_dtype = F.check_sensor_dtype(self.sensor_dtype)
+        rng = F.check_noise_rng(self.sensor_noise_rng)
         if psf_lab is True:
             raise NotImplementedError("psf_lab loads '../dataset_paula_real/psf_lab.jpg' in the reference (Lens.py:222-236)")
         if self.upsample:
@@ -661,8 +663,10 @@ class OpticsZernike(nn.Module):
             if prueba == "2" or prueba == "3":
                 psf = psf * self.mask_2
 
-        epilogue = (F.read_out(input_img, self.sensor_noise_sigma, self.sensor_quant_bits, noise)
+        epilogue = (F.read_out(input_img, self.sensor_noise_sigma, self.sensor_quant_bits, noise, rng,
+                               F.shard_first4(input_img, self._process_group))
                     if torch.is_tensor(input_img) else None)
+        self.sensor_noise_seed = F.noise_seed(epilogue)
         sensor = self._sensor(input_img, psf, epilogue, out_dtype)
         np.random.uniform(low=0.001, high=0.02)                     # noise_sigma is drawn and discarded (Lens.py:295)
         return sensor, psf, coeffs, loss                            # (the batch-global max of Lens.py:312 is inside _sensor)

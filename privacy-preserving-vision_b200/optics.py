@@ -69,7 +69,13 @@ class Camera(nn.Module):
         # bf16 (torch.autocast).  bf16 = the fp32 image rounded to nearest-even, written by the kernels; its bf16 gradient is read
         # by them as it is (backward = the fp32 one on g.float()).  Set by the caller, never inferred from autocast.
         self.sensor_dtype = torch.float32
-        self.overlap_psf = True          # run the PSF-independent half of forward() beside the PSF synthesis
+        # generator of the opt-in sensor noise: "torch" (the default: a torch.randn tensor shaped like the batch) or "philox" (the
+        # normalise kernel draws it from a key drawn with torch.randint - no noise tensor; include/b200cam.h
+        # B200CAM_SENSOR_NOISE_PHILOX).  The seed block {key, first4} of the last forward is `sensor_noise_seed` (None when the
+        # kernels drew nothing): F.philox_normal(seed, shape) re-creates that step's noise.
+        self.sensor_noise_rng = "torch"
+        self.sensor_noise_seed = None
+        self.overlap_psf = True         # run the PSF-independent half of forward() beside the PSF synthesis
         self._plans: dict[torch.device, F.DevicePlan] = {}
         self._pending_centering = None
         self._process_group = None
@@ -160,8 +166,10 @@ class Camera(nn.Module):
 
     def forward(self, img, noise=None):
         """`noise`: optional standard-normal tensor shaped like `img` for the opt-in sensor noise (drawn here with
-        torch.randn when `sensor_noise_sigma > 0` and none is given).  The sensor image is returned in `sensor_dtype`."""
+        torch.randn when `sensor_noise_sigma > 0` and none is given, or in the kernels with `sensor_noise_rng = "philox"`).  The
+        sensor image is returned in `sensor_dtype`."""
         out_dtype = F.check_sensor_dtype(self.sensor_dtype)
+        rng = F.check_noise_rng(self.sensor_noise_rng)
         # uint8 images (what a decoder produces; the reference's loader turns them into fp32 in [0,1] with ToTensor on the
         # host, Face-DeId/core/data_loader.py:118-124) may be passed as they are: the sensor kernels read the bytes and convert
         # them in registers as x * fp32(1/255), bit for bit torch's x.float() / 255.0 on the GPU - no fp32 copy of the batch is
@@ -176,7 +184,9 @@ class Camera(nn.Module):
         h_dev = self.Zer_train.device
         overlap = (self.overlap_psf and torch.is_tensor(img) and img.is_cuda and img.dim() == 4 and img.shape[0] > 0
                    and h_dev.type == "cuda")
-        epi = F.read_out(img, self.sensor_noise_sigma, self.sensor_quant_bits, noise) if torch.is_tensor(img) else None
+        epi = (F.read_out(img, self.sensor_noise_sigma, self.sensor_quant_bits, noise, rng, F.shard_first4(img, self._process_group))
+               if torch.is_tensor(img) else None)
+        self.sensor_noise_seed = F.noise_seed(epi)
         if not overlap:
             psf = self.get_psf()
             self.centering_loss = self._pending_centering
@@ -184,9 +194,10 @@ class Camera(nn.Module):
         plan = self._plan(img.device)
         side = plan.side_stream()
         psf = self.get_psf(_stream=side)                       # enqueued on `side`, not joined yet
-        # (the bf16 read-out runs the default pipeline only: not the plane layout that sensor_rows writes with B200CAM_PLANE=1;
-        # a uint8 batch reaches this point at N = 256 with B200CAM_PLANE=1 only with bf16, see above)
-        split = psf.device == img.device and not (out_dtype == torch.bfloat16 and self.N == 256 and F.PLANE_KERNELS)
+        # (the bf16 and Philox read-outs run the default pipeline only: not the plane layout that sensor_rows writes with
+        # B200CAM_PLANE=1; a uint8 batch reaches this point at N = 256 with B200CAM_PLANE=1 only with bf16, see above)
+        default_only = out_dtype == torch.bfloat16 or self.sensor_noise_seed is not None
+        split = psf.device == img.device and not (default_only and self.N == 256 and F.PLANE_KERNELS)
         rows = F.sensor_rows(img, plan) if split else None
         cur = torch.cuda.current_stream(psf.device)
         if rows is not None and plan.otf_event is not None:
